@@ -52,6 +52,9 @@ def parse_args():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: --windows per GPU (the driver's 1->8 run); strong: ONE batch of --windows windows dealt to the ranks "
                          "in cell-balanced bins (clb_balanced_partition, the rule of clb_popoa_batch_multi)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0's windows) to DIR/<name>.npy, float64: "
+                         "every window's score and the alignments of a fixed, seeded sample of windows")
     return ap.parse_args()
 
 
@@ -106,6 +109,27 @@ class ClockSampler:
         pw = [float(r[2]) for r in self.rows if len(r) > 2 and r[2].replace(".", "").isdigit()]
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None, "reasons": reasons,
                 "power_w_max": max(pw) if pw else None, "samples": len(sm)}
+
+
+DUMP_SAMPLE_WINDOWS = 64
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path, scores, alns):
+    """What a caller of the resident path receives, for comparing two builds output for output: scores.npy (one per
+    window), and for a seeded sample of windows (alignment_windows.npy, ascending) their alignments concatenated
+    (alignment_pairs.npy, node-id pairs, -1 = gap) with alignment_offsets.npy.  Every value is an integer below 2^53,
+    so float64 holds it exactly.  Sampled windows whose alignments would push the files past 64 MB are left out."""
+    rng = np.random.default_rng(SEED)
+    pick = np.sort(rng.choice(len(scores), min(DUMP_SAMPLE_WINDOWS, len(scores)), replace=False))
+    budget = (DUMP_MAX_BYTES - 8 * len(scores) - 16 * (len(pick) + 1)) // 16
+    keep = pick[np.cumsum([len(alns[w]) for w in pick]) <= budget]
+    off = np.zeros(len(keep) + 1, np.int64)
+    np.cumsum([len(alns[w]) for w in keep], out=off[1:])
+    pairs = np.concatenate([alns[w] for w in keep]) if len(keep) else np.zeros((0, 2), np.int32)
+    os.makedirs(path, exist_ok=True)
+    for name, a in (("scores", scores), ("alignment_windows", keep), ("alignment_offsets", off), ("alignment_pairs", pairs)):
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, np.float64))
 
 
 def dist_env():
@@ -456,6 +480,8 @@ def main():
         avail = psutil.virtual_memory().available / max(1, world)
         fit = int(avail * 0.6 / 0.8e6) * (world if args.scaling == "strong" else 1)
         if fit < args.windows:
+            if args.dump_outputs:  # dumped outputs are compared across runs: the inputs must not depend on the host's free RAM
+                raise SystemExit(f"bench.py: host RAM allows {fit} windows per rank, not {args.windows}; pass --windows {max(1000, fit)}")
             if rank == 0:
                 print(f"[bench] host RAM allows {fit} windows per rank, not {args.windows}: reducing", file=sys.stderr)
             args.windows = max(1000, fit)
@@ -511,6 +537,8 @@ def main():
     # results of the resident run (for the parity check of the CPU sample)
     scores, alns = db.download()
     scores = scores.copy()
+    if args.dump_outputs and rank == 0:  # before the e2e leg, which reuses db's alignment buffer
+        dump_outputs(args.dump_outputs, scores, alns)
     st = db.stats()  # now includes the D2H byte count
     db.close()
 

@@ -97,6 +97,13 @@ class CpuChecker:
             raise RuntimeError(f"{self.kind} pwfa checker failed with code {rc}")
         return int(score.value), aln[: ln.value].copy()
 
+    def run(self, batch: WindowBatch, params: AlignmentParameters, prune_limit=None):
+        """(scores, alignments) of every window: po_poa, or pwfa_po_poa on a batch in successor form when
+        ``prune_limit`` is given."""
+        res = [self.po_poa(batch, w, params) if prune_limit is None else self.pwfa_po_poa(batch, w, params, prune_limit)
+               for w in range(batch.n_windows)]
+        return [r[0] for r in res], [r[1] for r in res]
+
 
 def chain_oracle(problem: ChainProblem):
     """The C restatement of the reference's chaining DP (oracle/libcloracle.so :: clo_chain_dp) on the same flat

@@ -1,9 +1,12 @@
 """Loader for tests/golden/popoa_golden.npz (written by tests/golden/make_golden.py)."""
+import hashlib
+import json
 import os
 
 import numpy as np
 
-from centrolign_b200.batch import AlignmentParameters, GraphSide, WindowBatch
+from centrolign_b200.batch import (AlignmentParameters, GraphSide, WindowBatch, batch_from_graph_pairs, graph_from_edges,
+                                   successor_form, synth_windows)
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "popoa_golden.npz")
 
@@ -80,3 +83,39 @@ def load_chain_golden():
     z = np.load(CHAIN_GOLDEN)
     cases = sorted({k.split("/")[0] for k in z.files})
     return {c: problems_from_arrays(z, prefix=c + "/") for c in cases}
+
+
+LIVE_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "live_golden.json")
+
+
+def live_runs(name):
+    """Inputs on which tests compare with the unmodified reference: [(batch, params, prune_limit)].  prune_limit is None
+    for po_poa; for pwfa_po_poa the batch is in successor form."""
+    prod = AlignmentParameters()
+    if name == "po_poa_oracle":
+        batch = synth_windows(24, first_index=100, seed=3, len_min=30, len_max=900, alt_len=41, alt_period=300)
+        g = graph_from_edges("ACG", [(0, 1), (1, 2)], [0], [2])
+        e = graph_from_edges("", [], [], [])
+        return ([(batch, p, None) for p in (prod, prod.truncated(2), AlignmentParameters(1, 1, (1,), (1,)))]
+                + [(batch_from_graph_pairs([(g, e), (e, g), (e, e)]), prod, None)])
+    if name == "pwfa_oracle":
+        batch = synth_windows(10, first_index=500, seed=5, len_min=200, len_max=3000, alt_len=41, alt_period=300)
+        return [(sb, p, lim) for sb in (successor_form(batch), successor_form(batch, np.random.default_rng(1)))
+                for p, lim in ((prod, 50), (prod.truncated(1), 8))]
+    if name == "po_poa_gpu":
+        return [(synth_windows(10, first_index=200, seed=9, len_min=100, len_max=1200, alt_len=61, alt_period=400), prod, None)]
+    if name == "pwfa_gpu":
+        sb = successor_form(synth_windows(8, first_index=1200, seed=2, len_min=500, len_max=7000))
+        return [(sb, prod, 50), (sb, prod, 0)]
+    raise KeyError(name)
+
+
+def results_digest(scores, alns):
+    """[(score, sha256 of the alignment as little-endian int32 pairs)] per window: the form live_golden.json keeps."""
+    return [(int(s), hashlib.sha256(np.ascontiguousarray(a, "<i4").tobytes()).hexdigest()) for s, a in zip(scores, alns)]
+
+
+def load_live_golden(name):
+    """tests/golden/live_golden.json (tests/golden/make_live_golden.py): results_digest of every run of live_runs(name)."""
+    with open(LIVE_GOLDEN) as f:
+        return [[tuple(x) for x in run] for run in json.load(f)[name]]

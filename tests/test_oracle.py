@@ -2,16 +2,16 @@
 
 * the reference's own golden alignments (src/test/test_alignment.cpp:684-773),
 * fixtures produced by the unmodified reference (tests/golden/popoa_golden.npz),
-* live comparison with oracle/_ref/libclref.so whenever it is present (it is built from
-  /root/reference by oracle/Makefile and travels to the GPU box with the snapshot).
+* recorded results on further windows (tests/golden/live_golden.json), and a live comparison with
+  oracle/_ref/libclref.so on the same windows where it is built (oracle/Makefile, from the reference's sources).
 """
 import numpy as np
 import pytest
 
-from centrolign_b200.batch import (AlignmentParameters, batch_from_graph_pairs, graph_from_edges,
-                                   successor_form, synth_windows)
+from centrolign_b200.batch import AlignmentParameters, batch_from_graph_pairs, graph_from_edges, successor_form
 from checkers import CpuChecker  # test infrastructure: tests/checkers.py
-from golden_io import REFERENCE_UNIT_GOLDENS, TIEBREAK_PROBES, load_chain_golden, load_golden, load_pwfa_golden
+from golden_io import (REFERENCE_UNIT_GOLDENS, TIEBREAK_PROBES, live_runs, load_chain_golden, load_golden, load_live_golden,
+                       load_pwfa_golden, results_digest)
 
 
 @pytest.fixture(scope="module")
@@ -62,23 +62,22 @@ def test_empty_sides(oracle):
     assert s == 0 and len(a) == 0
 
 
-@pytest.mark.skipif(not CpuChecker.available("reference"), reason="oracle/_ref/libclref.so not built")
+def _check_live_runs(name, oracle):
+    """The oracle on golden_io.live_runs(name): equal to the results recorded in tests/golden/live_golden.json and, where
+    oracle/_ref/libclref.so is built, to the unmodified reference's."""
+    ref = CpuChecker("reference") if CpuChecker.available("reference") else None
+    for k, ((batch, p, lim), want) in enumerate(zip(live_runs(name), load_live_golden(name), strict=True)):
+        scores, alns = oracle.run(batch, p, lim)
+        assert results_digest(scores, alns) == want, f"{name} run {k}: differs from the recorded results"
+        if ref is not None:
+            rs, ra = ref.run(batch, p, lim)
+            for w in range(batch.n_windows):
+                assert scores[w] == rs[w] and np.array_equal(alns[w], ra[w]), f"{name} run {k} window {w} P={p.num_pw}"
+
+
 def test_live_against_reference(oracle):
-    ref = CpuChecker("reference")
-    batch = synth_windows(24, first_index=100, seed=3, len_min=30, len_max=900, alt_len=41, alt_period=300)
-    for w in range(batch.n_windows):
-        for p in (AlignmentParameters(), AlignmentParameters().truncated(2), AlignmentParameters(1, 1, (1,), (1,))):
-            so, ao = oracle.po_poa(batch, w, p)
-            sr, ar = ref.po_poa(batch, w, p)
-            assert so == sr and np.array_equal(ao, ar), f"window {w} P={p.num_pw}"
-    # empty sides agree with the reference too
-    g = graph_from_edges("ACG", [(0, 1), (1, 2)], [0], [2])
-    e = graph_from_edges("", [], [], [])
-    eb = batch_from_graph_pairs([(g, e), (e, g), (e, e)])
-    for w in range(3):
-        so, ao = oracle.po_poa(eb, w, AlignmentParameters())
-        sr, ar = ref.po_poa(eb, w, AlignmentParameters())
-        assert so == sr and np.array_equal(ao, ar)
+    """HOR-like windows up to 900 nodes with three parameter sets, and empty sides."""
+    _check_live_runs("po_poa_oracle", oracle)
 
 
 # ---- wavefront variant (oracle/pwfa_oracle.c) ------------------------------------------------------------
@@ -100,16 +99,9 @@ def test_pwfa_golden_fixture(oracle):
         assert np.array_equal(a, alns[k]), f"case {k}: alignment"
 
 
-@pytest.mark.skipif(not CpuChecker.available("reference"), reason="oracle/_ref/libclref.so not built")
 def test_pwfa_live_against_reference(oracle):
-    ref = CpuChecker("reference")
-    batch = synth_windows(10, first_index=500, seed=5, len_min=200, len_max=3000, alt_len=41, alt_period=300)
-    for sb in (successor_form(batch), successor_form(batch, np.random.default_rng(1))):
-        for w in range(batch.n_windows):
-            for p, lim in ((AlignmentParameters(), 50), (AlignmentParameters().truncated(1), 8)):
-                so, ao = oracle.pwfa_po_poa(sb, w, p, lim)
-                sr, ar = ref.pwfa_po_poa(sb, w, p, lim)
-                assert so == sr and np.array_equal(ao, ar), f"window {w} P={p.num_pw}"
+    """Windows up to 3000 nodes in two successor orders, two parameter sets and prune limits."""
+    _check_live_runs("pwfa_oracle", oracle)
 
 
 # ---- sparse anchor-chaining DP (oracle/chain_oracle.c) ---------------------------------------------------

@@ -1,6 +1,6 @@
 """GPU parity tests: the CUDA path, called through the C ABI, against the CPU oracle
-(oracle/po_poa_oracle.c), the committed reference fixtures, and -- when it travelled with the
-snapshot -- the unmodified reference itself (oracle/_ref/libclref.so).  Integer DP: bit-exact
+(oracle/po_poa_oracle.c), the committed reference fixtures, recorded results (tests/golden/live_golden.json)
+and, where it is built, the unmodified reference itself (oracle/_ref/libclref.so).  Integer DP: bit-exact
 scores and identical alignments are required."""
 import numpy as np
 import pytest
@@ -10,7 +10,7 @@ from centrolign_b200.batch import (AlignmentParameters, batch_from_graph_pairs, 
                                    sources_and_sinks, synth_windows)
 from centrolign_b200.popoa import DeviceBatch, po_poa_batch
 from checkers import CpuChecker  # test infrastructure: tests/checkers.py
-from golden_io import REFERENCE_UNIT_GOLDENS, TIEBREAK_PROBES, load_golden
+from golden_io import REFERENCE_UNIT_GOLDENS, TIEBREAK_PROBES, live_runs, load_golden, load_live_golden, results_digest
 
 pytestmark = pytest.mark.gpu
 
@@ -206,12 +206,14 @@ def test_tiled_fill_small_panels():
     assert res.returncode == 0 and "TILED-OK" in res.stdout, res.stdout[-3000:]
 
 
-@pytest.mark.skipif(not CpuChecker.available("reference"), reason="oracle/_ref/libclref.so did not travel")
 def test_live_against_unmodified_reference():
-    ref = CpuChecker("reference")
-    batch = synth_windows(10, first_index=200, seed=9, len_min=100, len_max=1200, alt_len=61, alt_period=400)
-    scores, alns = po_poa_batch(batch, PROD)
-    _compare(batch, PROD, scores, alns, ref, "reference")
+    """Equal to the results recorded in tests/golden/live_golden.json and, where oracle/_ref/libclref.so is built, to the
+    unmodified reference's."""
+    for (batch, p, _), want in zip(live_runs("po_poa_gpu"), load_live_golden("po_poa_gpu"), strict=True):
+        scores, alns = po_poa_batch(batch, p)
+        assert results_digest(scores, alns) == want, "differs from the recorded results"
+        if CpuChecker.available("reference"):
+            _compare(batch, p, scores, alns, CpuChecker("reference"), "reference")
 
 
 def test_staged_api_is_repeatable_and_matches_one_shot():

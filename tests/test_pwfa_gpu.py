@@ -1,6 +1,7 @@
 """GPU parity tests of the wavefront variant: ``clb_pwfa_batch`` (hand-written sm_100a kernel) against the
 CPU oracle (oracle/pwfa_oracle.c), the fixtures produced by the unmodified reference
-(tests/golden/pwfa_golden.npz) and, when it travelled, the reference itself.  The algorithm's output is
+(tests/golden/pwfa_golden.npz), recorded results (tests/golden/live_golden.json) and, where it is built,
+the reference itself.  The algorithm's output is
 defined by its dequeue order, so identical alignments and scores are required, not just equal scores."""
 import numpy as np
 import pytest
@@ -9,7 +10,7 @@ from centrolign_b200.batch import (AlignmentParameters, batch_from_graph_pairs, 
                                    graph_from_edges, select_windows, successor_form, synth_windows)
 from centrolign_b200.popoa import ClbError, PwfaStats, pwfa_po_poa_batch
 from checkers import CpuChecker  # test infrastructure: tests/checkers.py
-from golden_io import REFERENCE_UNIT_GOLDENS, load_pwfa_golden
+from golden_io import REFERENCE_UNIT_GOLDENS, live_runs, load_live_golden, load_pwfa_golden, results_digest
 
 pytestmark = pytest.mark.gpu
 
@@ -61,14 +62,14 @@ def test_hor_windows_vs_oracle(num_pw):
         _compare(sb, p, 50, scores, alns, port, f"P={num_pw}")
 
 
-@pytest.mark.skipif(not CpuChecker.available("reference"), reason="oracle/_ref/libclref.so did not travel")
 def test_live_against_unmodified_reference():
-    ref = CpuChecker("reference")
-    batch = synth_windows(8, first_index=1200, seed=2, len_min=500, len_max=7000)
-    sb = successor_form(batch)
-    for lim in (50, 0):
-        scores, alns = pwfa_po_poa_batch(sb, PROD, lim)
-        _compare(sb, PROD, lim, scores, alns, ref, f"reference prune={lim}")
+    """Equal to the results recorded in tests/golden/live_golden.json and, where oracle/_ref/libclref.so is built, to the
+    unmodified reference's."""
+    for (sb, p, lim), want in zip(live_runs("pwfa_gpu"), load_live_golden("pwfa_gpu"), strict=True):
+        scores, alns = pwfa_po_poa_batch(sb, p, lim)
+        assert results_digest(scores, alns) == want, f"prune={lim}: differs from the recorded results"
+        if CpuChecker.available("reference"):
+            _compare(sb, p, lim, scores, alns, CpuChecker("reference"), f"reference prune={lim}")
 
 
 def test_table_enlargement_gives_the_same_result(monkeypatch):
