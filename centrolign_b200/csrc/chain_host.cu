@@ -10,36 +10,23 @@
 //     the two outer spines a cross structure over the node's subtree ordered by offset, ties in the outer
 //     key order (stable sort on key 2 only, orthogonal_max_search_tree.hpp:175-239, max_search_tree.hpp:100-106).
 // There is no CPU fallback: without a CUDA device the call fails.
-#include <cuda_runtime.h>
-
-#include <algorithm>
-#include <atomic>
-#include <mutex>
 #include <chrono>
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <limits>
-#include <map>
 #include <numeric>
-#include <string>
-#include <thread>
-#include <type_traits>
-#include <vector>
 
-#include "centrolign_b200.h"
 #include "chain_device.cuh"
+#include "host_common.cuh"
 
 namespace clb {
 cudaError_t launch_chain(ChainArgs args, int grid, int cluster, int prepare_grid, cudaStream_t stream, cudaEvent_t after_prepare);
 cudaError_t launch_chain_small_batch(const ChainArgs* d_args, int n, int smem_bytes, bool any_global, cudaStream_t stream);
 int chain_max_grid(int device);
-int host_fail(int code, const std::string& msg);
 }  // namespace clb
 
-namespace {
+using clb::fail;
 
-using clb::host_fail;
+namespace {
 
 double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
@@ -125,30 +112,6 @@ void parallel_sort(std::vector<SortKey>& keys) {
     }
 }
 
-// A batch of small problems being collected by clb_chain_dp_batch: every problem whose arena fits shared memory is
-// laid out as usual, its copy segments are appended to ONE staging buffer, and its kernel arguments are recorded with
-// arena-relative pointers; flush() then needs one H2D copy, one launch (a CTA per problem) and one D2H copy for all.
-std::atomic<int64_t> g_batch_flushes(0), g_batch_problems(0);  // CLB_COUNT_CALLS: launches of the batched kernel / problems in them
-struct DeferredProblem {
-    clb::ChainArgs args;        // pointers relative to the problem's arena (offset from 0)
-    size_t arena_off = 0;       // of the problem's copy region in the combined buffer
-    size_t res_off = 0;         // of its results (match-count floats / words) in the compact result buffers
-    size_t zero_bytes = 0;      // size of the region behind the copy region that starts as zero
-    int64_t n_match = 0;
-    const clb_chain_problem* p = nullptr;
-    float* dp_out = nullptr;
-    int64_t* backptr_out = nullptr;
-    int64_t* chain_out = nullptr;
-    int64_t* chain_len = nullptr;
-    float* opt_score = nullptr;
-};
-struct BatchCtx {
-    std::vector<char> staging;  // concatenated copy regions (256-byte aligned)
-    std::vector<DeferredProblem> items;
-    size_t res_total = 0;
-    int max_smem = 0;
-};
-
 struct ArenaPlan {
     struct Seg {
         size_t off, bytes;
@@ -172,6 +135,66 @@ struct ArenaPlan {
     }
 };
 
+// A laid-out problem: the scalar kernel arguments, and where its arrays sit in the copy region (o_*) and in the zero
+// region (z_*) of its arena.
+struct ChainLayout {
+    clb::ChainArgs scalars{};  // every pointer null: bind() sets them
+    size_t copy_bytes = 0, zero_bytes = 0;
+    size_t arena_bytes() const { return copy_bytes + zero_bytes; }
+    size_t o_dp, o_bp, o_sins, o_ins, o_qoff, o_qm, o_w, o_qc1, o_qa1, o_qa2, o_qo, o_pg, o_gs, o_gb, o_gn, o_pb, o_gk, o_gm, o_os,
+        o_oo, o_om, o_ib, o_in, o_io, o_er;
+    size_t z_qrec, z_gford, z_gfbest, z_orord, z_bit, z_cbest, z_cbp, z_cnt, z_ranks;
+};
+
+// The kernel arguments of a laid-out problem whose copy region is at device address c and zero region at z.  The only
+// code that knows which array lives in which region.  arena_bytes covers both regions, copy_bytes the copy region.
+clb::ChainArgs bind(const ChainLayout& L, char* c, char* z) {
+    clb::ChainArgs a = L.scalars;
+    a.dp = (float*)(c + L.o_dp); a.backptr = (uint32_t*)(c + L.o_bp);
+    a.sins_off = (const int64_t*)(c + L.o_sins); a.ins = (const clb::InsRec*)(c + L.o_ins);
+    a.qry_off = (const int64_t*)(c + L.o_qoff); a.qry_match = (const uint32_t*)(c + L.o_qm);
+    a.weight = (const float*)(c + L.o_w); a.qry_chain1 = (const uint32_t*)(c + L.o_qc1);
+    a.qa1 = (const int32_t*)(c + L.o_qa1); a.qa2 = (const int32_t*)(c + L.o_qa2); a.qoff = (const uint32_t*)(c + L.o_qo);
+    a.pair_grp_off = (const int64_t*)(c + L.o_pg); a.grp_shift = (const int32_t*)(c + L.o_gs);
+    a.grp_base = (const uint32_t*)(c + L.o_gb); a.grp_n = (const uint32_t*)(c + L.o_gn); a.pair_base = (const uint32_t*)(c + L.o_pb);
+    a.gf_key = (const uint32_t*)(c + L.o_gk); a.gf_match = (const uint32_t*)(c + L.o_gm);
+    a.or_shift = (const int32_t*)(c + L.o_os); a.or_off = (const uint32_t*)(c + L.o_oo); a.or_match = (const uint32_t*)(c + L.o_om);
+    a.in_base = (const uint32_t*)(c + L.o_ib); a.in_n = (const uint32_t*)(c + L.o_in); a.in_off = (const uint32_t*)(c + L.o_io);
+    a.ent_rank = (const uint32_t*)(c + L.o_er);
+    a.qrec = (clb::QueryRec*)(z + L.z_qrec);
+    a.gf_ord = (uint32_t*)(z + L.z_gford); a.gf_best = (unsigned long long*)(z + L.z_gfbest);
+    a.or_ord = (uint32_t*)(z + L.z_orord); a.bit = (unsigned long long*)(z + L.z_bit);
+    a.rank_pool = a.rank_stride ? (uint32_t*)(z + L.z_ranks) : nullptr;
+    a.cand_best = (unsigned long long*)(z + L.z_cbest); a.cand_bp = (uint32_t*)(z + L.z_cbp); a.counters = (unsigned long long*)(z + L.z_cnt);
+    a.arena_base = c;
+    a.arena_bytes = (int64_t)L.arena_bytes();
+    a.copy_bytes = (int64_t)L.copy_bytes;
+    return a;
+}
+
+// A batch of small problems being collected by clb_chain_dp_batch: every problem whose arena fits shared memory is
+// laid out as usual, its copy segments are appended to ONE staging buffer, and its layout is recorded; flush() then needs
+// one H2D copy, one launch (a CTA per problem) and one D2H copy for all.
+std::atomic<int64_t> g_batch_flushes(0), g_batch_problems(0);  // CLB_COUNT_CALLS: launches of the batched kernel / problems in them
+struct DeferredProblem {
+    ChainLayout layout;
+    size_t arena_off = 0;       // of the problem's copy region in the combined buffer
+    size_t res_off = 0;         // of its results (match-count floats / words) in the compact result buffers
+    int64_t n_match = 0;
+    const clb_chain_problem* p = nullptr;
+    float* dp_out = nullptr;
+    int64_t* backptr_out = nullptr;
+    int64_t* chain_out = nullptr;
+    int64_t* chain_len = nullptr;
+    float* opt_score = nullptr;
+};
+struct BatchCtx {
+    std::vector<char> staging;  // concatenated copy regions (256-byte aligned)
+    std::vector<DeferredProblem> items;
+    size_t res_total = 0;
+    int max_smem = 0;
+};
+
 }  // namespace
 
 // the reference's traceback on the final DP values and back-pointers (anchorer.hpp:2483-2534)
@@ -193,7 +216,7 @@ static int chain_traceback(const clb_chain_problem* p, const float* h_dp, const 
     }
     int64_t len = 0;
     for (int64_t here = opt; here >= 0; here = h_bp[here] == 0xffffffffu ? -1 : (int64_t)h_bp[here]) {
-        if (len >= M) return host_fail(CLB_ECUDA, "internal: back-pointer cycle");
+        if (len >= M) return fail(CLB_ECUDA, "internal: back-pointer cycle");
         chain_out[len++] = here;
     }
     std::reverse(chain_out, chain_out + len);
@@ -239,11 +262,11 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
         calls += 1;
         matches += p->n_match;
     }
-    if (!p || !chain_out || !chain_len) return host_fail(CLB_EINVAL, "null problem or output");
-    if (p->num_pw < 0 || p->num_pw > CLB_MAX_PW) return host_fail(CLB_EINVAL, "num_pw outside 0..3");
-    if (p->n_match < 0 || p->n_step < 0 || p->n_chain1 < 0 || p->n_chain2 < 0) return host_fail(CLB_EINVAL, "negative sizes");
-    if (p->n_match > 0 && (p->n_chain1 < 1 || p->n_chain2 < 1)) return host_fail(CLB_EINVAL, "matches but no chains");
-    if (p->n_match >= (int64_t(1) << 31)) return host_fail(CLB_EINVAL, "more than 2^31 matches");
+    if (!p || !chain_out || !chain_len) return fail(CLB_EINVAL, "null problem or output");
+    if (p->num_pw < 0 || p->num_pw > CLB_MAX_PW) return fail(CLB_EINVAL, "num_pw outside 0..3");
+    if (p->n_match < 0 || p->n_step < 0 || p->n_chain1 < 0 || p->n_chain2 < 0) return fail(CLB_EINVAL, "negative sizes");
+    if (p->n_match > 0 && (p->n_chain1 < 1 || p->n_chain2 < 1)) return fail(CLB_EINVAL, "matches but no chains");
+    if (p->n_match >= (int64_t(1) << 31)) return fail(CLB_EINVAL, "more than 2^31 matches");
     if (const char* dump_dir = getenv("CLB_DUMP_DIR")) {  // debugging aid: every problem a caller sends, in the format of oracle/chain_shim.cpp
         static std::atomic<int> seq(0);
         if (p->n_match > 0 && p->ins_off && p->end_off && p->qry_off) {
@@ -277,30 +300,26 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
         }
     }
     const bool layout_only = getenv("CLB_CHAIN_LAYOUT_ONLY") != nullptr;  // host-layout timing without a device (no results)
-    int ndev = 0;
-    if (!layout_only) {
-        if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0)
-            return host_fail(CLB_ECUDA, "no CUDA device available (there is no CPU fallback)");
-        if (device < 0 || device >= ndev) return host_fail(CLB_EINVAL, "device index out of range");
-    }
+    if (!layout_only)
+        if (const int rc = clb::require_device(device)) return rc;
     *chain_len = 0;
     const float kLowest = std::numeric_limits<float>::lowest();
     if (opt_score) *opt_score = kLowest;
     const int64_t M = p->n_match, S = p->n_step;
     if (M == 0) return CLB_OK;
     if (!p->weight || !p->dp_init || !p->final_term || !p->end_off || !p->qry_off || !p->ins_off || !p->qa1 || !p->qa2 || !p->qoff)
-        return host_fail(CLB_EINVAL, "null problem arrays");
+        return fail(CLB_EINVAL, "null problem arrays");
     const int C1 = p->n_chain1, C2 = p->n_chain2, P = p->num_pw, T = 2 * P;
     const int64_t npair = (int64_t)C1 * C2;
     const int64_t E = p->ins_off[M];  // tree entries
-    if (E < 0 || E >= (int64_t(1) << 32) - 1) return host_fail(CLB_EINVAL, "entry count out of range");
+    if (E < 0 || E >= (int64_t(1) << 32) - 1) return fail(CLB_EINVAL, "entry count out of range");
     const int64_t n_end = p->end_off[S], n_qry = p->qry_off[S];
     for (int64_t k = 0; k < n_end; ++k)
-        if (p->end_match[k] >= (uint64_t)M) return host_fail(CLB_EINVAL, "end_match out of range");
+        if (p->end_match[k] >= (uint64_t)M) return fail(CLB_EINVAL, "end_match out of range");
     for (int64_t k = 0; k < n_qry; ++k)
-        if (p->qry_match[k] >= (uint64_t)M || p->qry_chain1[k] >= (uint32_t)C1) return host_fail(CLB_EINVAL, "query out of range");
+        if (p->qry_match[k] >= (uint64_t)M || p->qry_chain1[k] >= (uint32_t)C1) return fail(CLB_EINVAL, "query out of range");
     for (int64_t e = 0; e < E; ++e)
-        if (p->ins_p1[e] >= (uint32_t)C1 || p->ins_p2[e] >= (uint32_t)C2) return host_fail(CLB_EINVAL, "insert path out of range");
+        if (p->ins_p1[e] >= (uint32_t)C1 || p->ins_p2[e] >= (uint32_t)C2) return fail(CLB_EINVAL, "insert path out of range");
 
     // ------------------------------------------------------------------ layout ------------------------------------------------------------------
     std::vector<uint32_t> ent_match(E), ent_pair(E);
@@ -323,8 +342,8 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
         sins_off[s + 1] = (int64_t)sins_entry.size();
         max_q = std::max(max_q, p->qry_off[s + 1] - p->qry_off[s]);
     }
-    if ((int64_t)sins_entry.size() >= (int64_t(1) << 32) - 1) return host_fail(CLB_EINVAL, "more than 2^32 insertions");
-    if (max_q * C2 * (T + 1) >= (int64_t(1) << 32) - 1) return host_fail(CLB_EINVAL, "too many queries in one step");
+    if ((int64_t)sins_entry.size() >= (int64_t(1) << 32) - 1) return fail(CLB_EINVAL, "more than 2^32 insertions");
+    if (max_q * C2 * (T + 1) >= (int64_t(1) << 32) - 1) return fail(CLB_EINVAL, "too many queries in one step");
 
     std::vector<uint32_t> order(E);
     std::iota(order.begin(), order.end(), 0u);
@@ -410,7 +429,7 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
             for (uint32_t k = 0; k < n; ++k) ent_rank_off[order[ob + k] + 1] = nanc[heap_of_pos[k]];
         }
         for (int64_t e = 0; e < E; ++e) ent_rank_off[e + 1] += ent_rank_off[e];
-        if (ent_rank_off[E] != n_inner) return host_fail(CLB_ECUDA, "internal: inner list accounting mismatch");
+        if (ent_rank_off[E] != n_inner) return fail(CLB_ECUDA, "internal: inner list accounting mismatch");
         in_off.resize(n_inner);
         ent_rank.resize(n_inner);
         // pass 2: inner lists by merging children lists, one tree level at a time from the leaves up (the nodes of a
@@ -467,8 +486,8 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
         }
     }
     // insertion records in the reference's order, and the remaining per-entry tables in 32-bit form
-    if (n_inner >= (int64_t(1) << 32) - 1) return host_fail(CLB_EINVAL, "search structures exceed 2^32 inner slots");
-    if ((int64_t)sins_entry.size() >= (int64_t(1) << 31)) return host_fail(CLB_EINVAL, "more than 2^31 insertions");
+    if (n_inner >= (int64_t(1) << 32) - 1) return fail(CLB_EINVAL, "search structures exceed 2^32 inner slots");
+    if ((int64_t)sins_entry.size() >= (int64_t(1) << 31)) return fail(CLB_EINVAL, "more than 2^31 insertions");
     std::vector<clb::InsRec> ins(sins_entry.size());
     for (size_t i = 0; i < sins_entry.size(); ++i) {
         const uint32_t e = sins_entry[i];
@@ -489,7 +508,7 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
     if (layout_only) {
         fprintf(stderr, "[clb] chain layout only: %lld matches, %lld entries, %lld inner slots, %.1f ms\n", (long long)M, (long long)E,
                 (long long)n_inner, t_built - t_start);
-        return host_fail(CLB_ECUDA, "CLB_CHAIN_LAYOUT_ONLY: layout timed, nothing computed");
+        return fail(CLB_ECUDA, "CLB_CHAIN_LAYOUT_ONLY: layout timed, nothing computed");
     }
 
     // ------------------------------------------------------------------ device ------------------------------------------------------------------
@@ -501,18 +520,12 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
     std::lock_guard<std::mutex> arena_lock(g_arena_mu);
     DeviceArena& ar = g_arenas[device];
     bool keep = true;
-#define CHAIN_TRY(expr)                                                                                               \
-    do {                                                                                                              \
-        cudaError_t _e = (expr);                                                                                      \
-        if (_e != cudaSuccess) {                                                                                      \
-            rc = host_fail(_e == cudaErrorMemoryAllocation ? CLB_ENOMEM : CLB_ECUDA, std::string(#expr) + ": " + cudaGetErrorString(_e)); \
-            goto cleanup;                                                                                             \
-        }                                                                                                             \
-    } while (0)
     {
         ArenaPlan plan;
+        ChainLayout L{};
         std::vector<uint32_t> bp0(M, clb::kChainNone);
-        const size_t o_dp = plan.copy(p->dp_init, M * sizeof(float)), o_bp = plan.copy(bp0);
+        L.o_dp = plan.copy(p->dp_init, M * sizeof(float));
+        L.o_bp = plan.copy(bp0);
         // the device walks only the steps in which something happens (a caller may list every node of graph 1 as a step; the
         // builders of hostcpp/chain_b200.hpp list the nodes with events): the offsets are cumulative, so dropping an empty step
         // drops one equal entry of either list
@@ -525,22 +538,21 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
                 qry_live.push_back(p->qry_off[s + 1]);
             }
         const int64_t S_live = (int64_t)sins_live.size() - 1;
-        const size_t o_sins = plan.copy(sins_live), o_ins = plan.copy(ins);
-        const size_t o_qoff = plan.copy(qry_live), o_qm = plan.copy(p->qry_match, n_qry * sizeof(uint32_t));
-        const size_t o_w = plan.copy(p->weight, M * sizeof(float)), o_qc1 = plan.copy(p->qry_chain1, n_qry * sizeof(uint32_t));
-        const size_t o_qa1 = plan.copy(p->qa1, (size_t)M * C1 * sizeof(int32_t)), o_qa2 = plan.copy(p->qa2, (size_t)M * C2 * sizeof(int32_t));
-        const size_t o_qo = plan.copy(p->qoff, (size_t)M * C2 * sizeof(uint32_t));
-        const size_t o_pg = plan.copy(pair_grp_off), o_gs = plan.copy(grp_shift), o_gb = plan.copy(grp_base32), o_gn = plan.copy(grp_n);
-        const size_t o_pb = plan.copy(pair_base32), o_gk = plan.copy(gf_key), o_gm = plan.copy(gf_match);
-        const size_t o_os = plan.copy(or_shift), o_oo = plan.copy(or_off), o_om = plan.copy(or_match);
-        const size_t o_ib = plan.copy(in_base32), o_in = plan.copy(in_n), o_io = plan.copy(in_off), o_er = plan.copy(ent_rank);
-        const size_t z_qrec = plan.zero((size_t)n_qry * C2 * sizeof(clb::QueryRec));
-        const size_t z_gford = plan.zero((size_t)E * 4), z_gfbest = plan.zero((size_t)E * 8);
-        const size_t z_orord = plan.zero((size_t)T * E * 4), z_bit = plan.zero((size_t)T * n_inner * 8);
-        const size_t z_cbest = plan.zero((size_t)M * 16), z_cbp = plan.zero((size_t)(max_q * C2 * (T + 1)) * 4 * 2), z_cnt = plan.zero(8);
+        L.o_sins = plan.copy(sins_live); L.o_ins = plan.copy(ins);
+        L.o_qoff = plan.copy(qry_live); L.o_qm = plan.copy(p->qry_match, n_qry * sizeof(uint32_t));
+        L.o_w = plan.copy(p->weight, M * sizeof(float)); L.o_qc1 = plan.copy(p->qry_chain1, n_qry * sizeof(uint32_t));
+        L.o_qa1 = plan.copy(p->qa1, (size_t)M * C1 * sizeof(int32_t)); L.o_qa2 = plan.copy(p->qa2, (size_t)M * C2 * sizeof(int32_t));
+        L.o_qo = plan.copy(p->qoff, (size_t)M * C2 * sizeof(uint32_t));
+        L.o_pg = plan.copy(pair_grp_off); L.o_gs = plan.copy(grp_shift); L.o_gb = plan.copy(grp_base32); L.o_gn = plan.copy(grp_n);
+        L.o_pb = plan.copy(pair_base32); L.o_gk = plan.copy(gf_key); L.o_gm = plan.copy(gf_match);
+        L.o_os = plan.copy(or_shift); L.o_oo = plan.copy(or_off); L.o_om = plan.copy(or_match);
+        L.o_ib = plan.copy(in_base32); L.o_in = plan.copy(in_n); L.o_io = plan.copy(in_off); L.o_er = plan.copy(ent_rank);
+        L.z_qrec = plan.zero((size_t)n_qry * C2 * sizeof(clb::QueryRec));
+        L.z_gford = plan.zero((size_t)E * 4); L.z_gfbest = plan.zero((size_t)E * 8);
+        L.z_orord = plan.zero((size_t)T * E * 4); L.z_bit = plan.zero((size_t)T * n_inner * 8);
+        L.z_cbest = plan.zero((size_t)M * 16); L.z_cbp = plan.zero((size_t)(max_q * C2 * (T + 1)) * 4 * 2); L.z_cnt = plan.zero(8);
         // subtree-block ranks of every orthogonal walk (2 * (depth + 1) blocks at most), if memory allows
         int rank_stride = 0;
-        size_t z_ranks = 0;
         if (P > 0 && n_qry > 0 && !getenv("CLB_CHAIN_NO_RANKS")) {
             uint32_t max_n = 1;
             for (int64_t pr = 0; pr < npair; ++pr) max_n = std::max<uint32_t>(max_n, (uint32_t)(pair_base[pr + 1] - pair_base[pr]));
@@ -552,53 +564,33 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
                 cudaSetDevice(device);
                 fits = cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && bytes < free_b / 4 + (ar.cap > 0 ? ar.cap / 4 : 0);
             }
-            if (fits) z_ranks = plan.zero(bytes);
+            if (fits) L.z_ranks = plan.zero(bytes);
             else rank_stride = 0;
         }
+        L.copy_bytes = plan.copy_bytes;
+        L.zero_bytes = plan.zero_bytes;
+        clb::ChainArgs& b = L.scalars;
+        b.num_pw = P; b.n_chain1 = C1; b.n_chain2 = C2; b.scale = p->scale;
+        for (int k = 0; k < 3; ++k) {
+            b.gap_open[k] = p->gap_open[k];
+            b.gap_extend[k] = p->gap_extend[k];
+            b.scale_ext[k] = p->scale * p->gap_extend[k];  // anchorer.hpp:2330: local_scale * gap_extend[pw / 2] (* shift on the device)
+        }
+        b.n_match = M; b.n_step = S_live; b.n_entry = E; b.n_inner = n_inner; b.n_qry = n_qry; b.n_ins = (int64_t)ins.size();
+        b.cand_bp_stride = max_q * C2 * (T + 1);
+        b.rank_stride = rank_stride;
         const size_t total = plan.copy_bytes + plan.zero_bytes;
         if (ctx && total <= kChainBatchArena && !getenv("CLB_CHAIN_NO_SMALL")) {
-            // batched small problem: stage the copy region, record arena-relative arguments, finish in flush()
+            // batched small problem: stage the copy region and keep the layout; flush() binds it to the staged arena
             DeferredProblem d;
             d.arena_off = ctx->staging.size();
             ctx->staging.resize(d.arena_off + plan.copy_bytes);
             for (const auto& sg : plan.segs)
                 if (sg.bytes) memcpy(ctx->staging.data() + d.arena_off + sg.off, sg.src, sg.bytes);
-            char* const base = nullptr;           // arena-relative: flush() adds the device address of the problem's copy region
-            char* const zr0 = base + plan.copy_bytes;
-            clb::ChainArgs& b = d.args;
-            b = clb::ChainArgs{};
-            b.num_pw = P; b.n_chain1 = C1; b.n_chain2 = C2; b.scale = p->scale;
-            for (int k = 0; k < 3; ++k) {
-                b.gap_open[k] = p->gap_open[k];
-                b.gap_extend[k] = p->gap_extend[k];
-                b.scale_ext[k] = p->scale * p->gap_extend[k];
-            }
-            b.n_match = M; b.n_step = S_live; b.n_entry = E; b.n_inner = n_inner; b.n_qry = n_qry; b.n_ins = (int64_t)ins.size();
-            b.cand_bp_stride = max_q * C2 * (T + 1); b.sync_mode = 0;
-            b.dp = (float*)(base + o_dp); b.backptr = (uint32_t*)(base + o_bp);
-            b.sins_off = (const int64_t*)(base + o_sins); b.ins = (const clb::InsRec*)(base + o_ins);
-            b.qry_off = (const int64_t*)(base + o_qoff); b.qry_match = (const uint32_t*)(base + o_qm);
-            b.weight = (const float*)(base + o_w); b.qry_chain1 = (const uint32_t*)(base + o_qc1);
-            b.qa1 = (const int32_t*)(base + o_qa1); b.qa2 = (const int32_t*)(base + o_qa2); b.qoff = (const uint32_t*)(base + o_qo);
-            b.pair_grp_off = (const int64_t*)(base + o_pg); b.grp_shift = (const int32_t*)(base + o_gs);
-            b.grp_base = (const uint32_t*)(base + o_gb); b.grp_n = (const uint32_t*)(base + o_gn); b.pair_base = (const uint32_t*)(base + o_pb);
-            b.gf_key = (const uint32_t*)(base + o_gk); b.gf_match = (const uint32_t*)(base + o_gm);
-            b.or_shift = (const int32_t*)(base + o_os); b.or_off = (const uint32_t*)(base + o_oo); b.or_match = (const uint32_t*)(base + o_om);
-            b.in_base = (const uint32_t*)(base + o_ib); b.in_n = (const uint32_t*)(base + o_in); b.in_off = (const uint32_t*)(base + o_io);
-            b.ent_rank = (const uint32_t*)(base + o_er);
-            b.qrec = (clb::QueryRec*)(zr0 + z_qrec);
-            b.gf_ord = (uint32_t*)(zr0 + z_gford); b.gf_best = (unsigned long long*)(zr0 + z_gfbest);
-            b.or_ord = (uint32_t*)(zr0 + z_orord); b.bit = (unsigned long long*)(zr0 + z_bit);
-            b.rank_pool = rank_stride ? (uint32_t*)(zr0 + z_ranks) : nullptr;
-            b.rank_stride = rank_stride;
-            b.cand_best = (unsigned long long*)(zr0 + z_cbest); b.cand_bp = (uint32_t*)(zr0 + z_cbp); b.counters = (unsigned long long*)(zr0 + z_cnt);
-            b.arena_base = base;
-            b.arena_bytes = (int64_t)total;
-            b.copy_bytes = (int64_t)plan.copy_bytes;
+            d.layout = L;
             d.res_off = ctx->res_total;
             ctx->res_total += (size_t)M;
             if (total <= (size_t)clb::kChainSmallArena) ctx->max_smem = std::max(ctx->max_smem, (int)((total + 15) / 16 * 16));
-            d.zero_bytes = plan.zero_bytes;
             d.n_match = M; d.p = p; d.dp_out = dp_out; d.backptr_out = backptr_out; d.chain_out = chain_out; d.chain_len = chain_len;
             d.opt_score = opt_score;
             ctx->items.push_back(d);
@@ -614,19 +606,19 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
             return CLB_OK;
         }
         keep = total <= kArenaKeep;
-        CHAIN_TRY(cudaSetDevice(device));
+        CUDA_TRY_CLEANUP(cudaSetDevice(device));
         if (!ar.stream) {
-            CHAIN_TRY(cudaStreamCreateWithFlags(&ar.stream, cudaStreamNonBlocking));
-            CHAIN_TRY(cudaEventCreate(&ar.ev0));
-            CHAIN_TRY(cudaEventCreate(&ar.ev1));
-            CHAIN_TRY(cudaEventCreate(&ar.evp));
+            CUDA_TRY_CLEANUP(cudaStreamCreateWithFlags(&ar.stream, cudaStreamNonBlocking));
+            CUDA_TRY_CLEANUP(cudaEventCreate(&ar.ev0));
+            CUDA_TRY_CLEANUP(cudaEventCreate(&ar.ev1));
+            CUDA_TRY_CLEANUP(cudaEventCreate(&ar.evp));
         }
         if (ar.cap < total) {
             if (ar.d) cudaFree(ar.d);
             ar.d = nullptr;
             ar.cap = 0;
             const size_t want = keep ? std::max(total, std::min(kArenaKeep, 2 * total)) : total;
-            CHAIN_TRY(cudaMalloc((void**)&ar.d, want));
+            CUDA_TRY_CLEANUP(cudaMalloc((void**)&ar.d, want));
             ar.cap = want;
         }
         // A large problem is copied segment by segment straight from the caller's arrays: pinning a staging twin of tens to
@@ -638,7 +630,7 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
             ar.h = nullptr;
             ar.hcap = 0;
             const size_t want = std::max(plan.copy_bytes, std::min(kDirectCopyBytes, 2 * plan.copy_bytes));
-            CHAIN_TRY(cudaHostAlloc((void**)&ar.h, want, cudaHostAllocDefault));
+            CUDA_TRY_CLEANUP(cudaHostAlloc((void**)&ar.h, want, cudaHostAllocDefault));
             ar.hcap = want;
         }
         if (!direct)
@@ -647,37 +639,14 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
         const double t_staged = now_ms();
         if (direct) {
             for (const auto& sg : plan.segs)
-                if (sg.bytes) CHAIN_TRY(cudaMemcpyAsync(ar.d + sg.off, sg.src, sg.bytes, cudaMemcpyHostToDevice, ar.stream));
+                if (sg.bytes) CUDA_TRY_CLEANUP(cudaMemcpyAsync(ar.d + sg.off, sg.src, sg.bytes, cudaMemcpyHostToDevice, ar.stream));
         } else {
-            CHAIN_TRY(cudaMemcpyAsync(ar.d, ar.h, plan.copy_bytes, cudaMemcpyHostToDevice, ar.stream));
+            CUDA_TRY_CLEANUP(cudaMemcpyAsync(ar.d, ar.h, plan.copy_bytes, cudaMemcpyHostToDevice, ar.stream));
         }
         char* zr = ar.d + plan.copy_bytes;
-        CHAIN_TRY(cudaMemsetAsync(zr, 0, plan.zero_bytes, ar.stream));
-        a.num_pw = P; a.n_chain1 = C1; a.n_chain2 = C2; a.scale = p->scale;
-        for (int k = 0; k < 3; ++k) {
-            a.gap_open[k] = p->gap_open[k];
-            a.gap_extend[k] = p->gap_extend[k];
-            a.scale_ext[k] = p->scale * p->gap_extend[k];  // anchorer.hpp:2330: local_scale * gap_extend[pw / 2] (* shift on the device)
-        }
-        a.n_match = M; a.n_step = S_live; a.n_entry = E; a.n_inner = n_inner; a.n_qry = n_qry; a.n_ins = (int64_t)ins.size();
-        a.cand_bp_stride = max_q * C2 * (T + 1);
-        a.dp = (float*)(ar.d + o_dp); a.backptr = (uint32_t*)(ar.d + o_bp);
-        a.sins_off = (const int64_t*)(ar.d + o_sins); a.ins = (const clb::InsRec*)(ar.d + o_ins);
-        a.qry_off = (const int64_t*)(ar.d + o_qoff); a.qry_match = (const uint32_t*)(ar.d + o_qm);
-        a.weight = (const float*)(ar.d + o_w); a.qry_chain1 = (const uint32_t*)(ar.d + o_qc1);
-        a.qa1 = (const int32_t*)(ar.d + o_qa1); a.qa2 = (const int32_t*)(ar.d + o_qa2); a.qoff = (const uint32_t*)(ar.d + o_qo);
-        a.pair_grp_off = (const int64_t*)(ar.d + o_pg); a.grp_shift = (const int32_t*)(ar.d + o_gs);
-        a.grp_base = (const uint32_t*)(ar.d + o_gb); a.grp_n = (const uint32_t*)(ar.d + o_gn); a.pair_base = (const uint32_t*)(ar.d + o_pb);
-        a.gf_key = (const uint32_t*)(ar.d + o_gk); a.gf_match = (const uint32_t*)(ar.d + o_gm);
-        a.or_shift = (const int32_t*)(ar.d + o_os); a.or_off = (const uint32_t*)(ar.d + o_oo); a.or_match = (const uint32_t*)(ar.d + o_om);
-        a.in_base = (const uint32_t*)(ar.d + o_ib); a.in_n = (const uint32_t*)(ar.d + o_in); a.in_off = (const uint32_t*)(ar.d + o_io);
-        a.ent_rank = (const uint32_t*)(ar.d + o_er);
-        a.qrec = (clb::QueryRec*)(zr + z_qrec);
-        a.gf_ord = (uint32_t*)(zr + z_gford); a.gf_best = (unsigned long long*)(zr + z_gfbest);
-        a.or_ord = (uint32_t*)(zr + z_orord); a.bit = (unsigned long long*)(zr + z_bit);
-        a.rank_pool = rank_stride ? (uint32_t*)(zr + z_ranks) : nullptr;
-        a.rank_stride = rank_stride;
-        a.cand_best = (unsigned long long*)(zr + z_cbest); a.cand_bp = (uint32_t*)(zr + z_cbp); a.counters = (unsigned long long*)(zr + z_cnt);
+        CUDA_TRY_CLEANUP(cudaMemsetAsync(zr, 0, plan.zero_bytes, ar.stream));
+        a = bind(L, ar.d, zr);
+        a.copy_bytes = (int64_t)total;  // the single-problem path copies the zeroed region too
         // How the phases of a step are separated.  A step has `warps_per_step` independent warp-sized work items on average:
         // a handful run in one CTA (__syncthreads), up to as many as the largest cluster has warps in ONE thread-block cluster
         // (hardware cluster barrier, the items of a step spread over its SMs), more in a cooperative grid over all SMs (grid.sync).
@@ -694,25 +663,21 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
         } else if (warps_per_step > 1.5 * warps_per_cta) {
             while (cluster < kChainClusterMax && cluster * warps_per_cta < warps_per_step) cluster *= 2;
         }
-        a.arena_base = ar.d;
-        a.arena_bytes = (int64_t)total;
-        a.copy_bytes = (int64_t)total;  // the single-problem path copies the zeroed region too
-        a.out_dp = nullptr; a.out_backptr = nullptr;
         if (total <= (size_t)clb::kChainSmallArena && !getenv("CLB_CHAIN_NO_SMALL") && !getenv("CLB_CHAIN_GRID")) grid = 0;
         const int prepare_grid = (int)std::max<int64_t>(1, std::min<int64_t>((n_qry * C2 + 7) / 8, 8 * (int64_t)max_grid));
-        CHAIN_TRY(cudaEventRecord(ar.ev0, ar.stream));
-        CHAIN_TRY(clb::launch_chain(a, grid, cluster, prepare_grid, ar.stream, ar.evp));
-        CHAIN_TRY(cudaEventRecord(ar.ev1, ar.stream));
-        CHAIN_TRY(cudaMemcpyAsync(h_dp.data(), a.dp, M * sizeof(float), cudaMemcpyDeviceToHost, ar.stream));
-        CHAIN_TRY(cudaMemcpyAsync(h_bp.data(), a.backptr, M * sizeof(uint32_t), cudaMemcpyDeviceToHost, ar.stream));
-        CHAIN_TRY(cudaStreamSynchronize(ar.stream));
+        CUDA_TRY_CLEANUP(cudaEventRecord(ar.ev0, ar.stream));
+        CUDA_TRY_CLEANUP(clb::launch_chain(a, grid, cluster, prepare_grid, ar.stream, ar.evp));
+        CUDA_TRY_CLEANUP(cudaEventRecord(ar.ev1, ar.stream));
+        CUDA_TRY_CLEANUP(cudaMemcpyAsync(h_dp.data(), a.dp, M * sizeof(float), cudaMemcpyDeviceToHost, ar.stream));
+        CUDA_TRY_CLEANUP(cudaMemcpyAsync(h_bp.data(), a.backptr, M * sizeof(uint32_t), cudaMemcpyDeviceToHost, ar.stream));
+        CUDA_TRY_CLEANUP(cudaStreamSynchronize(ar.stream));
         if (call_timer.on) {
             CallTimer::phase()[0] += (int64_t)((t_built - t_start) * 1e3);
             CallTimer::phase()[1] += (int64_t)((t_staged - t_built) * 1e3);
             CallTimer::phase()[2] += (int64_t)((now_ms() - t_staged) * 1e3);
         }
         float ms = 0.f;
-        CHAIN_TRY(cudaEventElapsedTime(&ms, ar.ev0, ar.ev1));
+        CUDA_TRY_CLEANUP(cudaEventElapsedTime(&ms, ar.ev0, ar.ev1));
         if (getenv("CLB_TIMING")) {
             float pms = 0.f;
             cudaEventElapsedTime(&pms, ar.ev0, ar.evp);
@@ -744,7 +709,6 @@ cleanup:
         ar.cap = ar.hcap = 0;
     }
     return rc;
-#undef CHAIN_TRY
 }
 
 // Device and pinned buffers of the batched path, per device, grown on demand and kept (g_batch_mu serialises the flushes of
@@ -800,38 +764,32 @@ int flush_contexts(int device, BatchCtx* const* ctxs, int64_t n_ctx, clb_chain_s
     int rc = CLB_OK;
     std::lock_guard<std::mutex> lk(g_batch_mu);
     BatchArena& ba = g_batch_arenas[device];
-#define BATCH_TRY(expr)                                                                                                \
-    do {                                                                                                               \
-        cudaError_t _e = (expr);                                                                                       \
-        if (_e != cudaSuccess)                                                                                         \
-            return host_fail(_e == cudaErrorMemoryAllocation ? CLB_ENOMEM : CLB_ECUDA, std::string(#expr) + ": " + cudaGetErrorString(_e)); \
-    } while (0)
     const double t_start = now_ms();
-    BATCH_TRY(cudaSetDevice(device));
+    CUDA_TRY(cudaSetDevice(device));
     if (!ba.stream) {
-        BATCH_TRY(cudaStreamCreateWithFlags(&ba.stream, cudaStreamNonBlocking));
-        BATCH_TRY(cudaEventCreate(&ba.e0));
-        BATCH_TRY(cudaEventCreate(&ba.e1));
+        CUDA_TRY(cudaStreamCreateWithFlags(&ba.stream, cudaStreamNonBlocking));
+        CUDA_TRY(cudaEventCreate(&ba.e0));
+        CUDA_TRY(cudaEventCreate(&ba.e1));
     }
     const size_t args_bytes = (size_t)nb * sizeof(clb::ChainArgs);
-    BATCH_TRY(grow_device(ba.d_arena, ba.arena_cap, stage_bytes));
-    BATCH_TRY(grow_device(ba.d_args, ba.args_cap, args_bytes));
+    CUDA_TRY(grow_device(ba.d_arena, ba.arena_cap, stage_bytes));
+    CUDA_TRY(grow_device(ba.d_args, ba.args_cap, args_bytes));
     if (res_total * 4 > ba.res_cap) {
         size_t cap_dp = ba.res_cap, cap_bp = ba.res_cap;
-        BATCH_TRY(grow_device(ba.d_dp, cap_dp, res_total * 4));
-        BATCH_TRY(grow_device(ba.d_bp, cap_bp, res_total * 4));
+        CUDA_TRY(grow_device(ba.d_dp, cap_dp, res_total * 4));
+        CUDA_TRY(grow_device(ba.d_bp, cap_bp, res_total * 4));
         ba.res_cap = std::min(cap_dp, cap_bp);
     }
-    BATCH_TRY(grow_pinned(ba.h_stage, ba.stage_cap, stage_bytes + args_bytes));
-    BATCH_TRY(grow_pinned(ba.h_res, ba.hres_cap, res_total * 8));
+    CUDA_TRY(grow_pinned(ba.h_stage, ba.stage_cap, stage_bytes + args_bytes));
+    CUDA_TRY(grow_pinned(ba.h_res, ba.hres_cap, res_total * 8));
     clb::ChainArgs* h_args = reinterpret_cast<clb::ChainArgs*>(ba.h_stage + stage_bytes);
     float* h_dp = reinterpret_cast<float*>(ba.h_res);
     uint32_t* h_bp = reinterpret_cast<uint32_t*>(ba.h_res + res_total * 4);
     size_t zero_total = 0;  // problems too large for shared memory keep their zero-initialised region in global memory
     for (int64_t c = 0; c < n_ctx; ++c)
         for (const DeferredProblem& d : ctxs[c]->items)
-            if (d.args.arena_bytes > (int64_t)clb::kChainSmallArena) zero_total += ArenaPlan::align(d.zero_bytes);
-    BATCH_TRY(grow_device(ba.d_zero, ba.zero_cap, zero_total));
+            if (d.layout.arena_bytes() > (size_t)clb::kChainSmallArena) zero_total += ArenaPlan::align(d.layout.zero_bytes);
+    CUDA_TRY(grow_device(ba.d_zero, ba.zero_cap, zero_total));
     {
         size_t seg = 0, res_base = 0, zero_off = 0;
         int64_t k = 0;
@@ -839,28 +797,12 @@ int flush_contexts(int device, BatchCtx* const* ctxs, int64_t n_ctx, clb_chain_s
             const BatchCtx& ctx = *ctxs[c];
             if (!ctx.staging.empty()) memcpy(ba.h_stage + seg, ctx.staging.data(), ctx.staging.size());
             for (const DeferredProblem& d : ctx.items) {
-                clb::ChainArgs a = d.args;
-                const bool in_smem = a.arena_bytes <= (int64_t)clb::kChainSmallArena;
-                // fields of the copy region move to the staged copy; fields of the zero region follow it (shared memory: the
-                // kernel lays both out behind each other) or move to this problem's part of the cleared buffer
-                const ptrdiff_t shift = (ba.d_arena + seg + d.arena_off) - (char*)nullptr;
-                const ptrdiff_t zshift = in_smem ? shift : (ba.d_zero + zero_off) - ((char*)nullptr + a.copy_bytes);
-#define CLB_SHIFT_BY(f, by) a.f = reinterpret_cast<decltype(a.f)>(reinterpret_cast<char*>(const_cast<void*>(static_cast<const void*>(a.f))) + (by))
-#define CLB_SHIFT(f) CLB_SHIFT_BY(f, shift)
-#define CLB_ZSHIFT(f) CLB_SHIFT_BY(f, zshift)
-                CLB_SHIFT(dp); CLB_SHIFT(backptr); CLB_SHIFT(sins_off); CLB_SHIFT(ins); CLB_SHIFT(qry_off); CLB_SHIFT(qry_match);
-                CLB_SHIFT(weight); CLB_SHIFT(qry_chain1); CLB_SHIFT(qa1); CLB_SHIFT(qa2); CLB_SHIFT(qoff);
-                CLB_SHIFT(pair_grp_off); CLB_SHIFT(grp_shift); CLB_SHIFT(grp_base); CLB_SHIFT(grp_n); CLB_SHIFT(pair_base);
-                CLB_SHIFT(gf_key); CLB_SHIFT(gf_match); CLB_SHIFT(or_shift); CLB_SHIFT(or_off);
-                CLB_SHIFT(or_match); CLB_SHIFT(in_base); CLB_SHIFT(in_n); CLB_SHIFT(in_off);
-                CLB_SHIFT(ent_rank); CLB_SHIFT(arena_base);
-                CLB_ZSHIFT(qrec); CLB_ZSHIFT(gf_ord); CLB_ZSHIFT(gf_best); CLB_ZSHIFT(or_ord); CLB_ZSHIFT(bit);
-                CLB_ZSHIFT(cand_best); CLB_ZSHIFT(cand_bp); CLB_ZSHIFT(counters);
-                if (a.rank_pool) CLB_ZSHIFT(rank_pool);
-#undef CLB_ZSHIFT
-#undef CLB_SHIFT
-#undef CLB_SHIFT_BY
-                if (!in_smem) zero_off += ArenaPlan::align(d.zero_bytes);
+                // the copy region is the staged copy; the zero region follows it (shared memory: the kernel lays both out
+                // behind each other) or is this problem's part of the cleared buffer
+                char* const copy = ba.d_arena + seg + d.arena_off;
+                const bool in_smem = d.layout.arena_bytes() <= (size_t)clb::kChainSmallArena;
+                clb::ChainArgs a = bind(d.layout, copy, in_smem ? copy + d.layout.copy_bytes : ba.d_zero + zero_off);
+                if (!in_smem) zero_off += ArenaPlan::align(d.layout.zero_bytes);
                 a.out_dp = ba.d_dp + res_base + d.res_off;
                 a.out_backptr = ba.d_bp + res_base + d.res_off;
                 h_args[k++] = a;
@@ -870,18 +812,17 @@ int flush_contexts(int device, BatchCtx* const* ctxs, int64_t n_ctx, clb_chain_s
         }
     }
     const double t_staged = now_ms();
-    BATCH_TRY(cudaMemcpyAsync(ba.d_arena, ba.h_stage, stage_bytes, cudaMemcpyHostToDevice, ba.stream));
-    BATCH_TRY(cudaMemcpyAsync(ba.d_args, h_args, args_bytes, cudaMemcpyHostToDevice, ba.stream));
-    if (zero_total) BATCH_TRY(cudaMemsetAsync(ba.d_zero, 0, zero_total, ba.stream));
-    BATCH_TRY(cudaEventRecord(ba.e0, ba.stream));
-    BATCH_TRY(clb::launch_chain_small_batch(ba.d_args, (int)nb, max_smem, zero_total > 0, ba.stream));
-    BATCH_TRY(cudaEventRecord(ba.e1, ba.stream));
-    BATCH_TRY(cudaMemcpyAsync(h_dp, ba.d_dp, res_total * 4, cudaMemcpyDeviceToHost, ba.stream));
-    BATCH_TRY(cudaMemcpyAsync(h_bp, ba.d_bp, res_total * 4, cudaMemcpyDeviceToHost, ba.stream));
-    BATCH_TRY(cudaStreamSynchronize(ba.stream));
+    CUDA_TRY(cudaMemcpyAsync(ba.d_arena, ba.h_stage, stage_bytes, cudaMemcpyHostToDevice, ba.stream));
+    CUDA_TRY(cudaMemcpyAsync(ba.d_args, h_args, args_bytes, cudaMemcpyHostToDevice, ba.stream));
+    if (zero_total) CUDA_TRY(cudaMemsetAsync(ba.d_zero, 0, zero_total, ba.stream));
+    CUDA_TRY(cudaEventRecord(ba.e0, ba.stream));
+    CUDA_TRY(clb::launch_chain_small_batch(ba.d_args, (int)nb, max_smem, zero_total > 0, ba.stream));
+    CUDA_TRY(cudaEventRecord(ba.e1, ba.stream));
+    CUDA_TRY(cudaMemcpyAsync(h_dp, ba.d_dp, res_total * 4, cudaMemcpyDeviceToHost, ba.stream));
+    CUDA_TRY(cudaMemcpyAsync(h_bp, ba.d_bp, res_total * 4, cudaMemcpyDeviceToHost, ba.stream));
+    CUDA_TRY(cudaStreamSynchronize(ba.stream));
     float ms = 0.f;
-    BATCH_TRY(cudaEventElapsedTime(&ms, ba.e0, ba.e1));
-#undef BATCH_TRY
+    CUDA_TRY(cudaEventElapsedTime(&ms, ba.e0, ba.e1));
     if (stats) {
         stats->kernel_ms += ms;
         stats->kernel_launches += 1;
@@ -917,11 +858,11 @@ extern "C" int clb_chain_dp_batch(int device, int64_t n_problems, const clb_chai
                                   clb_chain_stats* stats) {
     const double t_start = now_ms();
     if (stats) memset(stats, 0, sizeof(*stats));
-    if (n_problems < 0 || (n_problems > 0 && (!problems || !chain_out || !chain_len))) return host_fail(CLB_EINVAL, "clb_chain_dp_batch: null arguments");
+    if (n_problems < 0 || (n_problems > 0 && (!problems || !chain_out || !chain_len))) return fail(CLB_EINVAL, "clb_chain_dp_batch: null arguments");
     BatchCtx ctx;
     clb_chain_stats one{};
     for (int64_t k = 0; k < n_problems; ++k) {
-        if (!problems[k] || !chain_out[k]) return host_fail(CLB_EINVAL, "clb_chain_dp_batch: null problem or output");
+        if (!problems[k] || !chain_out[k]) return fail(CLB_EINVAL, "clb_chain_dp_batch: null problem or output");
         const int rc = chain_dp_impl(device, problems[k], dp_out ? dp_out[k] : nullptr, backptr_out ? backptr_out[k] : nullptr, chain_out[k],
                                      &chain_len[k], opt_score ? &opt_score[k] : nullptr, stats ? &one : nullptr, &ctx);
         if (rc != CLB_OK) return rc;
@@ -948,11 +889,11 @@ struct clb_chain_job {
 
 extern "C" int clb_chain_job_create(int device, const clb_chain_problem* problem, float* dp_out, int64_t* backptr_out, int64_t* chain_out,
                                     int64_t* chain_len, float* opt_score, clb_chain_job** job) {
-    if (!job) return host_fail(CLB_EINVAL, "clb_chain_job_create: null job pointer");
+    if (!job) return fail(CLB_EINVAL, "clb_chain_job_create: null job pointer");
     *job = nullptr;
-    if (!problem || !chain_out || !chain_len) return host_fail(CLB_EINVAL, "clb_chain_job_create: null arguments");
+    if (!problem || !chain_out || !chain_len) return fail(CLB_EINVAL, "clb_chain_job_create: null arguments");
     clb_chain_job* j = new (std::nothrow) clb_chain_job();
-    if (!j) return host_fail(CLB_ENOMEM, "clb_chain_job_create: out of host memory");
+    if (!j) return fail(CLB_ENOMEM, "clb_chain_job_create: out of host memory");
     j->device = device;
     // a problem too large for one SM's shared memory is solved here and now (ctx stays empty)
     const int rc = chain_dp_impl(device, problem, dp_out, backptr_out, chain_out, chain_len, opt_score, nullptr, &j->ctx);
@@ -969,12 +910,12 @@ extern "C" int clb_chain_job_create(int device, const clb_chain_problem* problem
 }
 
 extern "C" int clb_chain_jobs_run(int device, int64_t n_jobs, clb_chain_job* const* jobs) {
-    if (n_jobs < 0 || (n_jobs > 0 && !jobs)) return host_fail(CLB_EINVAL, "clb_chain_jobs_run: null arguments");
+    if (n_jobs < 0 || (n_jobs > 0 && !jobs)) return fail(CLB_EINVAL, "clb_chain_jobs_run: null arguments");
     std::vector<BatchCtx*> ctxs;
     ctxs.reserve((size_t)n_jobs);
     for (int64_t k = 0; k < n_jobs; ++k) {
-        if (!jobs[k]) return host_fail(CLB_EINVAL, "clb_chain_jobs_run: null job");
-        if (jobs[k]->device != device) return host_fail(CLB_EINVAL, "clb_chain_jobs_run: job was created for another device");
+        if (!jobs[k]) return fail(CLB_EINVAL, "clb_chain_jobs_run: null job");
+        if (jobs[k]->device != device) return fail(CLB_EINVAL, "clb_chain_jobs_run: job was created for another device");
         if (!jobs[k]->ctx.items.empty()) ctxs.push_back(&jobs[k]->ctx);
     }
     const int rc = flush_contexts(device, ctxs.data(), (int64_t)ctxs.size(), nullptr);

@@ -7,21 +7,11 @@
 // topological order is used), predecessor lists are rewritten in previous() order with the
 // boundary index 0 appended last for sources (alignment.hpp:1069-1084), and the rows / columns
 // the kernels must keep ("persisted") are chosen.  Flattening is multi-threaded over windows.
-#include <cuda_runtime.h>
-
 #include <algorithm>
-#include <atomic>
 #include <chrono>
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
-#include <map>
-#include <mutex>
-#include <string>
-#include <thread>
-#include <vector>
 
-#include "centrolign_b200.h"
+#include "host_common.cuh"
 #include "popoa_device.cuh"
 
 namespace clb {
@@ -31,141 +21,19 @@ int popoa_smem_bytes();
 void popoa_wait_profile(bool reset);  // -DCLB_PROFILE builds: where the warps of popoa_kernel wait
 double int32_probe(int use_dpx, int sm_count);
 int popoa_nsmid();
-void chain_release_cache();  // chain_host.cu
 }  // namespace clb
 
+using clb::fail;
+using clb::g_cache;
+using clb::Staged;
+
 namespace {
-
-thread_local std::string g_err;
-int fail(int code, const std::string& msg) {
-    g_err = msg;
-    return code;
-}
-#define CUDA_TRY(expr)                                                                              \
-    do {                                                                                            \
-        cudaError_t _e = (expr);                                                                    \
-        if (_e != cudaSuccess)                                                                      \
-            return fail(_e == cudaErrorMemoryAllocation ? CLB_ENOMEM : CLB_ECUDA,                   \
-                        std::string(#expr) + ": " + cudaGetErrorString(_e));                        \
-    } while (0)
-
-// Process-wide cache of pinned-host and device blocks.  cudaHostAlloc / cudaFreeHost of the
-// multi-GB staging buffers cost seconds per call; a Stitcher calls the batch entry point once per
-// guide-tree node, so blocks are kept and reused (best fit) until clb_release_cached_memory().
-class MemCache {
-public:
-    void* host_alloc(size_t bytes, size_t* cap) {
-        bytes = round_up(bytes);
-        {
-            std::lock_guard<std::mutex> lk(mu_);
-            auto it = host_.lower_bound(bytes);
-            if (it != host_.end() && it->first <= 2 * bytes + (size_t(1) << 20)) {
-                void* p = it->second;
-                *cap = it->first;
-                host_.erase(it);
-                return p;
-            }
-        }
-        void* p = nullptr;
-        if (cudaHostAlloc(&p, bytes, cudaHostAllocDefault) != cudaSuccess) {
-            cudaGetLastError();
-            trim();
-            if (cudaHostAlloc(&p, bytes, cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); return nullptr; }
-        }
-        *cap = bytes;
-        return p;
-    }
-    void host_release(void* p, size_t cap) {
-        std::lock_guard<std::mutex> lk(mu_);
-        host_.emplace(cap, p);
-    }
-    void* dev_alloc(int device, size_t bytes, size_t* cap, bool any_larger) {
-        bytes = round_up(bytes);
-        {
-            std::lock_guard<std::mutex> lk(mu_);
-            auto& m = dev_[device];
-            auto it = m.lower_bound(bytes);
-            if (it != m.end() && (any_larger || it->first <= 2 * bytes + (size_t(1) << 20))) {
-                void* p = it->second;
-                *cap = it->first;
-                m.erase(it);
-                return p;
-            }
-        }
-        void* p = nullptr;
-        if (cudaMalloc(&p, bytes) != cudaSuccess) {
-            cudaGetLastError();
-            trim();
-            if (cudaMalloc(&p, bytes) != cudaSuccess) { cudaGetLastError(); return nullptr; }
-        }
-        *cap = bytes;
-        return p;
-    }
-    void dev_release(int device, void* p, size_t cap) {
-        std::lock_guard<std::mutex> lk(mu_);
-        dev_[device].emplace(cap, p);
-    }
-    size_t dev_cached(int device) {
-        std::lock_guard<std::mutex> lk(mu_);
-        size_t t = 0;
-        for (auto& kv : dev_[device]) t += kv.first;
-        return t;
-    }
-    void trim() {
-        std::lock_guard<std::mutex> lk(mu_);
-        for (auto& kv : host_) cudaFreeHost(kv.second);
-        host_.clear();
-        int cur = 0;
-        cudaGetDevice(&cur);
-        for (auto& d : dev_) {
-            cudaSetDevice(d.first);
-            for (auto& kv : d.second) cudaFree(kv.second);
-            d.second.clear();
-        }
-        cudaSetDevice(cur);
-    }
-
-private:
-    static size_t round_up(size_t b) { return (std::max<size_t>(b, 1) + 4095) & ~size_t(4095); }
-    std::mutex mu_;
-    std::multimap<size_t, void*> host_;
-    std::map<int, std::multimap<size_t, void*>> dev_;
-};
-MemCache g_cache;
-
-template <class T>
-struct Pinned {  // pinned host + device twin, both drawn from the cache
-    T* h = nullptr;
-    T* d = nullptr;
-    size_t n = 0, cap_h = 0, cap_d = 0;
-    int dev = 0;
-    int alloc_host(size_t count) {
-        n = count;
-        h = (T*)g_cache.host_alloc(count * sizeof(T), &cap_h);
-        return h ? CLB_OK : CLB_ENOMEM;
-    }
-    int alloc_dev(int device) {
-        dev = device;
-        d = (T*)g_cache.dev_alloc(device, n * sizeof(T), &cap_d, false);
-        return d ? CLB_OK : CLB_ENOMEM;
-    }
-    size_t bytes() const { return n * sizeof(T); }
-    void release() {
-        if (h) g_cache.host_release(h, cap_h);
-        if (d) g_cache.dev_release(dev, d, cap_d);
-        h = d = nullptr;
-    }
-};
-
+constexpr char kPopoaCalls[] = "[clb] ";  // CLB_COUNT_CALLS line of clb_popoa_batch / clb_popoa_batch_multi
 struct SideStage {
-    Pinned<uint32_t> info, depth, poff, pidx, sinks;
-    Pinned<int32_t> slot;
+    Staged<uint32_t> info, depth, poff, pidx, sinks;
+    Staged<int32_t> slot;
     std::vector<uint32_t> orig;  // matrix index -> caller node id (host only)
-    void release() {
-        info.release(); depth.release(); poff.release(); pidx.release(); sinks.release(); slot.release();
-    }
 };
-
 }  // namespace
 
 struct clb_batch {
@@ -173,11 +41,11 @@ struct clb_batch {
     int32_t nw = 0;
     clb_params params{};
     SideStage s[2];
-    Pinned<clb::WindowMeta> meta;
-    Pinned<int32_t> order;
-    Pinned<int64_t> score;
-    Pinned<int32_t> aln;
-    Pinned<uint32_t> aln_len;
+    Staged<clb::WindowMeta> meta;
+    Staged<int32_t> order;
+    Staged<int64_t> score;
+    Staged<int32_t> aln;
+    Staged<uint32_t> aln_len;
     int32_t* d_queue = nullptr;
     char* d_workspace = nullptr;
     size_t workspace_cap = 0;
@@ -262,24 +130,10 @@ uint32_t topological_ranks(uint32_t n, const uint32_t* po, const uint32_t* pr, u
 // Flatten one side of one window.  Returns CLB_OK / CLB_EINVAL / CLB_ECYCLE.
 int flatten_side(const clb_graph_batch& g, int64_t w, int side, SideStage& st, clb::WindowMeta& m, FlattenScratch& sc,
                  int64_t& int_ops_deg /* sum of in-degrees incl. boundary edges */) {
-    const int64_t n0 = g.node_off[w];
-    const uint32_t n = (uint32_t)(g.node_off[w + 1] - n0);
-    const uint32_t* po = g.pred_off + n0 + w;
-    const uint32_t* pr = g.pred + g.edge_off[w];
-    const uint32_t E = (uint32_t)(g.edge_off[w + 1] - g.edge_off[w]);
-    const uint32_t nsrc = (uint32_t)(g.src_off[w + 1] - g.src_off[w]);
-    const uint32_t nsnk = (uint32_t)(g.snk_off[w + 1] - g.snk_off[w]);
-    const uint32_t* src = g.src + g.src_off[w];
-    const uint32_t* snk = g.snk + g.snk_off[w];
-    if (po[0] != 0 || po[n] != E) return CLB_EINVAL;
-    for (uint32_t v = 0; v < n; ++v)
-        if (po[v + 1] < po[v]) return CLB_EINVAL;
-    for (uint32_t k = 0; k < E; ++k)
-        if (pr[k] >= n) return CLB_EINVAL;
-    for (uint32_t k = 0; k < nsrc; ++k)
-        if (src[k] >= n) return CLB_EINVAL;
-    for (uint32_t k = 0; k < nsnk; ++k)
-        if (snk[k] >= n) return CLB_EINVAL;
+    clb::GraphWindow gw;
+    if (clb::graph_window(g, w, gw) != CLB_OK) return CLB_EINVAL;
+    const uint32_t n = gw.n, E = gw.n_edge, nsrc = gw.n_src, nsnk = gw.n_snk;
+    const uint32_t *po = gw.off, *pr = gw.ids, *src = gw.src, *snk = gw.snk;
 
     const int64_t nb = (side == 0 ? m.node1 : m.node2);
     const int64_t pb = (side == 0 ? m.poff1 : m.poff2);
@@ -322,7 +176,7 @@ int flatten_side(const clb_graph_batch& g, int64_t w, int side, SideStage& st, c
         }
         depth[i] = dmin;
         poff[i + 1] = fill;
-        uint32_t word = (uint32_t)g.label[n0 + v];
+        uint32_t word = (uint32_t)gw.label[v];
         if (fill - first == 1 && pidx[first] == i - 1) {  // regular: also for i == 1 with the boundary as its only predecessor
             word |= clb::kInfoRegular;
             info[i] &= ~(clb::kInfoFar | clb::kInfoNearMask);
@@ -354,43 +208,13 @@ int flatten_side(const clb_graph_batch& g, int64_t w, int side, SideStage& st, c
     return CLB_OK;
 }
 
-int check_side(const clb_graph_batch* g, int64_t n_windows = -1) {
-    if (!g || !g->node_off || !g->edge_off || !g->pred_off || !g->src_off || !g->snk_off) return CLB_EINVAL;
-    if (n_windows > 0) {  // the payload arrays may only be null when they are empty
-        if (g->node_off[n_windows] > 0 && !g->label) return CLB_EINVAL;
-        if (g->edge_off[n_windows] > 0 && !g->pred) return CLB_EINVAL;
-        if (g->src_off[n_windows] > 0 && !g->src) return CLB_EINVAL;
-        if (g->snk_off[n_windows] > 0 && !g->snk) return CLB_EINVAL;
-    }
-    return CLB_OK;
-}
-
 }  // namespace
 
-namespace clb {
-int host_fail(int code, const std::string& msg) { return fail(code, msg); }  // for the other host files of the library
-// the process-wide cache of pinned-host and device blocks, for the other host files
-void* cache_host_alloc(size_t bytes, size_t* cap) { return g_cache.host_alloc(bytes, cap); }
-void cache_host_release(void* p, size_t cap) { g_cache.host_release(p, cap); }
-void* cache_dev_alloc(int device, size_t bytes, size_t* cap, bool any_larger) { return g_cache.dev_alloc(device, bytes, cap, any_larger); }
-void cache_dev_release(int device, void* p, size_t cap) { g_cache.dev_release(device, p, cap); }
-}  // namespace clb
-
 extern "C" {
-
-const char* clb_last_error(void) { return g_err.c_str(); }
-
-int clb_device_count(void) {
-    int n = 0;
-    if (cudaGetDeviceCount(&n) != cudaSuccess) return 0;
-    return n;
-}
 
 void clb_batch_destroy(clb_batch* b) {
     if (!b) return;
     cudaSetDevice(b->device);
-    for (auto& s : b->s) s.release();
-    b->meta.release(); b->order.release(); b->score.release(); b->aln.release(); b->aln_len.release();
     if (b->d_queue) g_cache.dev_release(b->device, b->d_queue, 4096);
     if (b->d_workspace && !b->shared_workspace) g_cache.dev_release(b->device, b->d_workspace, b->workspace_cap);
     if (b->ev0) cudaEventDestroy(b->ev0);
@@ -406,11 +230,9 @@ static int create_internal(int device, int32_t n_windows, const clb_graph_batch*
     *out = nullptr;
     if (n_windows < 0 || !params || params->num_pw < 1 || params->num_pw > CLB_MAX_PW)
         return fail(CLB_EINVAL, "bad n_windows or num_pw (must be 1..3)");
-    if (n_windows > 0 && (check_side(g1, n_windows) || check_side(g2, n_windows))) return fail(CLB_EINVAL, "null graph arrays");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        return fail(CLB_ECUDA, "no CUDA device: the gap-fill path has no CPU fallback");
-    if (device < 0 || device >= ndev) return fail(CLB_EINVAL, "device out of range");
+    if (n_windows > 0 && (clb::check_graph_batch(g1, n_windows) || clb::check_graph_batch(g2, n_windows)))
+        return fail(CLB_EINVAL, "null graph arrays");
+    if (const int rc = clb::require_device(device)) return rc;
     CUDA_TRY(cudaSetDevice(device));
 
     clb_batch* b = new clb_batch();
@@ -473,49 +295,27 @@ static int create_internal(int device, int32_t n_windows, const clb_graph_batch*
 
     // multi-threaded flatten
     const double t_alloc_done = std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count();
-    std::atomic<int64_t> next(0);
-    std::atomic<int> status(CLB_OK);
-    std::atomic<int64_t> bad_window(-1);
-    std::vector<int64_t> ops_part;
-    unsigned nthreads = std::max(1u, std::min(32u, std::thread::hardware_concurrency()));
-    if (nw < 64) nthreads = 1;
-    ops_part.assign(nthreads, 0);
+    const unsigned nthreads = clb::pool_threads(nw, 64);
+    std::vector<FlattenScratch> scratch(nthreads);
+    std::vector<int64_t> ops_part(nthreads, 0);
     std::vector<double> cells_part(nthreads, 0.0);
-    auto worker = [&](unsigned tix) {
-        FlattenScratch sc;
-        for (;;) {
-            const int64_t w0 = next.fetch_add(16);
-            if (w0 >= nw || status.load() != CLB_OK) break;
-            for (int64_t w = w0; w < std::min<int64_t>(nw, w0 + 16); ++w) {
-                clb::WindowMeta& m = b->meta.h[w];
-                int64_t deg1 = 0, deg2 = 0;
-                int r = flatten_side(*g1, src(w), 0, b->s[0], m, sc, deg1);
-                if (r == CLB_OK) r = flatten_side(*g2, src(w), 1, b->s[1], m, sc, deg2);
-                if (r != CLB_OK) {
-                    status.store(r);
-                    bad_window.store(src(w));
-                    return;
-                }
-                // SURVEY 8(d): per cell a*b + 1 + 4P(a+b) + 2P add/max; summed over the window this factorises:
-                //   sum_ij a_i*b_j = deg1*deg2,  sum_ij (a_i+b_j) = deg1*n2 + deg2*n1   (interior cells only)
-                const int64_t P = b->params.num_pw;
-                ops_part[tix] += deg1 * deg2 + (int64_t)m.n1 * m.n2 * (1 + 2 * P) + 4 * P * (deg1 * (int64_t)m.n2 + deg2 * (int64_t)m.n1);
-                cells_part[tix] += ((double)m.n1 + 1.0) * ((double)m.n2 + 1.0);
-            }
-        }
-    };
-    if (nthreads == 1) {
-        worker(0);
-    } else {
-        std::vector<std::thread> pool;
-        for (unsigned t = 0; t < nthreads; ++t) pool.emplace_back(worker, t);
-        for (auto& t : pool) t.join();
-    }
-    if (status.load() != CLB_OK) {
-        const int r = status.load();
-        const int64_t bw = bad_window.load();
+    int64_t bad = -1;
+    rc = clb::for_each_window(nw, 16, 64, [&](unsigned t, int64_t w) -> int {
+        clb::WindowMeta& m = b->meta.h[w];
+        int64_t deg1 = 0, deg2 = 0;
+        int r = flatten_side(*g1, src(w), 0, b->s[0], m, scratch[t], deg1);
+        if (r == CLB_OK) r = flatten_side(*g2, src(w), 1, b->s[1], m, scratch[t], deg2);
+        if (r != CLB_OK) return r;
+        // SURVEY 8(d): per cell a*b + 1 + 4P(a+b) + 2P add/max; summed over the window this factorises:
+        //   sum_ij a_i*b_j = deg1*deg2,  sum_ij (a_i+b_j) = deg1*n2 + deg2*n1   (interior cells only)
+        const int64_t P = b->params.num_pw;
+        ops_part[t] += deg1 * deg2 + (int64_t)m.n1 * m.n2 * (1 + 2 * P) + 4 * P * (deg1 * (int64_t)m.n2 + deg2 * (int64_t)m.n1);
+        cells_part[t] += ((double)m.n1 + 1.0) * ((double)m.n2 + 1.0);
+        return CLB_OK;
+    }, &bad);
+    if (rc != CLB_OK) {
         clb_batch_destroy(b);
-        return fail(r, std::string(r == CLB_ECYCLE ? "cyclic graph" : "malformed graph") + " in window " + std::to_string(bw));
+        return fail(rc, std::string(rc == CLB_ECYCLE ? "cyclic graph" : "malformed graph") + " in window " + std::to_string(src(bad)));
     }
     if (getenv("CLB_TIMING"))
         fprintf(stderr, "[clb] create: flatten %.3f s on %u threads\n",
@@ -723,7 +523,7 @@ int clb_batch_download(clb_batch* b, int64_t* score_out, const int64_t* aln_off,
     b->stats.d2h_bytes = (int64_t)(b->score.bytes() + b->aln_len.bytes() + b->aln.bytes());
     // translate topological ranks back to the caller's node ids; pairs were written backwards
     // from the end of each window's region, so they are already in forward order
-    auto translate = [&](int64_t w) {
+    clb::for_each_window(nw, 64, 64, [&](unsigned, int64_t w) -> int {
         const clb::WindowMeta& m = b->meta.h[w];
         const uint32_t len = b->aln_len.h[w];
         const int64_t cap = b->out_off[w + 1] - b->out_off[w];
@@ -738,24 +538,8 @@ int clb_batch_download(clb_batch* b, int64_t* score_out, const int64_t* aln_off,
         }
         aln_len[dst_w(w)] = len;
         score_out[dst_w(w)] = b->score.h[w];
-    };
-    unsigned nthreads = std::max(1u, std::min(32u, std::thread::hardware_concurrency()));
-    if (nw < 64) nthreads = 1;
-    if (nthreads == 1) {
-        for (int64_t w = 0; w < nw; ++w) translate(w);
-    } else {
-        std::atomic<int64_t> next(0);
-        std::vector<std::thread> pool;
-        for (unsigned t = 0; t < nthreads; ++t)
-            pool.emplace_back([&] {
-                for (;;) {
-                    const int64_t w0 = next.fetch_add(64);
-                    if (w0 >= nw) break;
-                    for (int64_t w = w0; w < std::min<int64_t>(nw, w0 + 64); ++w) translate(w);
-                }
-            });
-        for (auto& t : pool) t.join();
-    }
+        return CLB_OK;
+    });
     return CLB_OK;
 }
 
@@ -765,23 +549,11 @@ int clb_batch_get_stats(const clb_batch* b, clb_batch_stats* out) {
     return CLB_OK;
 }
 
-// evidence for integration tests that the GPU path really ran (CLB_COUNT_CALLS): calls and windows, printed at exit
-static void count_popoa_call(int64_t n_windows) {
-    if (!getenv("CLB_COUNT_CALLS")) return;
-    static std::atomic<int64_t> calls(0), windows(0);
-    static std::once_flag once;
-    std::call_once(once, [] {
-        atexit([] { fprintf(stderr, "[clb] calls %lld windows %lld\n", (long long)calls.load(), (long long)windows.load()); });
-    });
-    calls += 1;
-    windows += n_windows;
-}
-
 int clb_popoa_batch(int device, int32_t n_windows, const clb_graph_batch* g1, const clb_graph_batch* g2,
                     const clb_params* params, int64_t* score_out, const int64_t* aln_off, int32_t* aln_pairs,
                     uint32_t* aln_len) {
     const bool timing = getenv("CLB_TIMING") != nullptr;
-    count_popoa_call(n_windows);
+    clb::count_call<kPopoaCalls>(n_windows);
     if (const char* dump_dir = getenv("CLB_DUMP_DIR")) {  // debugging aid: every batch a caller sends, for tools/check_dump.py
         static std::atomic<int> seq(0);
         if (n_windows > 0 && g1 && g2 && params) {
@@ -829,7 +601,7 @@ int clb_popoa_batch(int device, int32_t n_windows, const clb_graph_batch* g1, co
         return rc;
     };
     if (!chunked) return one_batch();
-    if (check_side(g1) || check_side(g2) || !params) return fail(CLB_EINVAL, "null graph arrays");
+    if (clb::check_graph_batch(g1) || clb::check_graph_batch(g2) || !params) return fail(CLB_EINVAL, "null graph arrays");
     // windows by matrix size, largest first
     std::vector<int32_t> ord(n_windows);
     for (int32_t w = 0; w < n_windows; ++w) ord[w] = w;
@@ -930,8 +702,8 @@ int clb_popoa_batch_multi(int n_devices, const int* devices, int32_t n_windows, 
         if (part_out) for (int32_t w = 0; w < n_windows; ++w) part_out[w] = 0;
         return clb_popoa_batch(devices[0], n_windows, g1, g2, params, score_out, aln_off, aln_pairs, aln_len);
     }
-    if (n_windows < 0 || check_side(g1) || check_side(g2) || !params) return fail(CLB_EINVAL, "null graph arrays");
-    count_popoa_call(n_windows);
+    if (n_windows < 0 || clb::check_graph_batch(g1) || clb::check_graph_batch(g2) || !params) return fail(CLB_EINVAL, "null graph arrays");
+    clb::count_call<kPopoaCalls>(n_windows);
     std::vector<int64_t> cells(n_windows);
     for (int32_t w = 0; w < n_windows; ++w)
         cells[w] = (g1->node_off[w + 1] - g1->node_off[w] + 1) * (g2->node_off[w + 1] - g2->node_off[w] + 1);
@@ -955,7 +727,7 @@ int clb_popoa_batch_multi(int n_devices, const int* devices, int32_t n_windows, 
             if (r == CLB_OK) r = clb_batch_download(b, score_out, aln_off, aln_pairs, aln_len);
             clb_batch_destroy(b);
             rcs[k] = r;
-            if (r != CLB_OK) errs[k] = g_err;  // thread-local: hand it to the caller's thread
+            if (r != CLB_OK) errs[k] = clb_last_error();  // thread-local: hand it to the caller's thread
         });
     for (auto& t : pool) t.join();
     for (int k = 0; k < n_devices; ++k)
@@ -977,47 +749,6 @@ int clb_topological_ranks(uint32_t n_nodes, const uint32_t* pred_off, const uint
     if (topological_ranks(n_nodes, pred_off, pred, E, sc, orig.data()) != n_nodes) return fail(CLB_ECYCLE, "clb_topological_ranks: the graph has a cycle");
     for (uint32_t v = 0; v < n_nodes; ++v) rank_out[v] = sc.tpos[v];
     return CLB_OK;
-}
-
-// Context creation off the critical path: a process that knows it will use `device` calls this first thing; the CUDA
-// runtime serialises initialisation itself, so later calls of the library simply find the context there (or wait for it).
-namespace {
-std::mutex g_warm_mu;
-std::thread* g_warm_thread = nullptr;
-void join_warm_up() {
-    std::thread* t = nullptr;
-    {
-        std::lock_guard<std::mutex> lk(g_warm_mu);
-        t = g_warm_thread;
-        g_warm_thread = nullptr;
-    }
-    if (t) {
-        t->join();
-        delete t;
-    }
-}
-}  // namespace
-
-void clb_warm_up(int device) {
-    std::lock_guard<std::mutex> lk(g_warm_mu);
-    static bool started = false;
-    if (started) return;
-    started = true;
-    g_warm_thread = new (std::nothrow) std::thread([device] {
-        int n = 0;
-        if (cudaGetDeviceCount(&n) != cudaSuccess || device < 0 || device >= n) {
-            cudaGetLastError();
-            return;  // no device: the first real call reports it
-        }
-        if (cudaSetDevice(device) == cudaSuccess) cudaFree(nullptr);
-        cudaGetLastError();
-    });
-    if (g_warm_thread) atexit(join_warm_up);
-}
-
-void clb_release_cached_memory(void) {
-    g_cache.trim();
-    clb::chain_release_cache();
 }
 
 double clb_int32_peak_tops(int device, int use_dpx) {

@@ -8,47 +8,23 @@
 // (alignment.hpp:1992-1997), converts the parameters (to_wfa_params, alignment.hpp:1613-1654) and groups
 // the transition penalties into classes of equal value (see pwfa_kernels.cu).  The search and the
 // traceback run on the device; there is no CPU fallback.
-#include <cuda_runtime.h>
-
 #include <algorithm>
-#include <atomic>
-#include <chrono>
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
-#include <mutex>
 #include <numeric>
-#include <string>
-#include <thread>
-#include <vector>
 
-#include "centrolign_b200.h"
+#include "host_common.cuh"
 #include "pwfa_device.cuh"
 
 namespace clb {
 cudaError_t launch_pwfa(const PwfaArgs& args, int grid, cudaStream_t stream);
-int host_fail(int code, const std::string& msg);  // popoa_host.cu: sets clb_last_error()
-// popoa_host.cu: process-wide cache of pinned-host and device blocks (cudaHostAlloc / cudaMalloc of the staging and
-// workspace buffers cost more than the search itself on small batches)
-void* cache_host_alloc(size_t bytes, size_t* cap);
-void cache_host_release(void* p, size_t cap);
-void* cache_dev_alloc(int device, size_t bytes, size_t* cap, bool any_larger);
-void cache_dev_release(int device, void* p, size_t cap);
 }  // namespace clb
+
+using clb::fail;
+using clb::Staged;
 
 namespace {
 
-using clb::host_fail;
-
-#define PWFA_CUDA_TRY(expr)                                                                       \
-    do {                                                                                          \
-        cudaError_t _e = (expr);                                                                  \
-        if (_e != cudaSuccess) {                                                                  \
-            rc = host_fail(_e == cudaErrorMemoryAllocation ? CLB_ENOMEM : CLB_ECUDA,              \
-                           std::string(#expr) + ": " + cudaGetErrorString(_e));                   \
-            goto cleanup;                                                                         \
-        }                                                                                         \
-    } while (0)
+constexpr char kPwfaCalls[] = "[clb] pwfa ";  // CLB_COUNT_CALLS line of clb_pwfa_batch
 
 uint32_t gcd_u32(uint32_t a, uint32_t b) {
     while (b) {
@@ -65,32 +41,6 @@ int ceil_log2(uint64_t v) {
     return l;
 }
 
-// pinned host block + device twin, both drawn from the library's cache
-template <class T>
-struct Staged {
-    T* h = nullptr;
-    T* d = nullptr;
-    size_t n = 0, cap_h = 0, cap_d = 0;
-    int dev = 0;
-    bool alloc(int device, size_t count, bool host, bool any_larger = false) {
-        dev = device;
-        n = std::max<size_t>(count, 1);
-        if (host) {
-            h = (T*)clb::cache_host_alloc(n * sizeof(T), &cap_h);
-            if (!h) return false;
-        }
-        d = (T*)clb::cache_dev_alloc(device, n * sizeof(T), &cap_d, any_larger);
-        return d != nullptr;
-    }
-    size_t bytes() const { return n * sizeof(T); }
-    void release() {
-        if (h) clb::cache_host_release(h, cap_h);
-        if (d) clb::cache_dev_release(dev, d, cap_d);
-        h = d = nullptr;
-    }
-    ~Staged() { release(); }
-};
-
 struct SideOut {
     Staged<int4> info;
     Staged<uint32_t> next;
@@ -104,27 +54,16 @@ struct Scratch {
 };
 
 // one side of one window -> node records + successor array (sources appended for the virtual start)
-int flatten_side(const clb_graph_batch& g, int64_t w, int4* info, uint32_t* next_out, uint8_t* nlab, Scratch& sc) {
-    const int64_t n0 = g.node_off[w];
-    const uint32_t n = (uint32_t)(g.node_off[w + 1] - n0);
-    const uint32_t* no = g.pred_off + n0 + w;  // successor offsets (see clb_succ_graph_batch)
-    const uint32_t* nx = g.pred + g.edge_off[w];
-    const uint32_t E = (uint32_t)(g.edge_off[w + 1] - g.edge_off[w]);
-    const uint32_t nsrc = (uint32_t)(g.src_off[w + 1] - g.src_off[w]);
-    const uint32_t nsnk = (uint32_t)(g.snk_off[w + 1] - g.snk_off[w]);
-    const uint32_t* src = g.src + g.src_off[w];
-    const uint32_t* snk = g.snk + g.snk_off[w];
-    const uint8_t* label = g.label + n0;
-    if (no[0] != 0 || no[n] != E) return CLB_EINVAL;
+int flatten_side(const clb_succ_graph_batch& g, int64_t w, int4* info, uint32_t* next_out, uint8_t* nlab, Scratch& sc) {
+    clb::GraphWindow gw;
+    if (clb::graph_window(g, w, gw) != CLB_OK) return CLB_EINVAL;
+    const uint32_t n = gw.n, E = gw.n_edge, nsrc = gw.n_src, nsnk = gw.n_snk;
+    const uint32_t *no = gw.off, *nx = gw.ids, *src = gw.src, *snk = gw.snk;  // successor lists (see clb_succ_graph_batch)
+    const uint8_t* label = gw.label;
+    // the node records keep out-degrees and the source count in the 22 bits above kPwfaDegShift
     for (uint32_t v = 0; v < n; ++v)
-        if (no[v + 1] < no[v] || no[v + 1] - no[v] >= (1u << 22)) return CLB_EINVAL;
+        if (no[v + 1] - no[v] >= (1u << 22)) return CLB_EINVAL;
     if (nsrc >= (1u << 22)) return CLB_EINVAL;
-    for (uint32_t k = 0; k < E; ++k)
-        if (nx[k] >= n) return CLB_EINVAL;
-    for (uint32_t k = 0; k < nsrc; ++k)
-        if (src[k] >= n) return CLB_EINVAL;
-    for (uint32_t k = 0; k < nsnk; ++k)
-        if (snk[k] >= n) return CLB_EINVAL;
 
     sc.indeg.assign(n + 1, 0);
     sc.order.resize(n + 1);
@@ -185,17 +124,6 @@ int flatten_side(const clb_graph_batch& g, int64_t w, int4* info, uint32_t* next
     return CLB_OK;
 }
 
-int check_side(const clb_graph_batch* g, int64_t n_windows = -1) {
-    if (!g || !g->node_off || !g->edge_off || !g->pred_off || !g->src_off || !g->snk_off) return CLB_EINVAL;
-    if (n_windows > 0) {  // the payload arrays may only be null when they are empty
-        if (g->node_off[n_windows] > 0 && !g->label) return CLB_EINVAL;
-        if (g->edge_off[n_windows] > 0 && !g->pred) return CLB_EINVAL;
-        if (g->src_off[n_windows] > 0 && !g->src) return CLB_EINVAL;
-        if (g->snk_off[n_windows] > 0 && !g->snk) return CLB_EINVAL;
-    }
-    return CLB_OK;
-}
-
 }  // namespace
 
 extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_graph_batch* g1, const clb_succ_graph_batch* g2,
@@ -203,22 +131,13 @@ extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_grap
                               int32_t* aln_pairs, uint32_t* aln_len, clb_pwfa_stats* stats) {
     if (stats) memset(stats, 0, sizeof(*stats));
     if (n_windows < 0 || !params || params->num_pw < 1 || params->num_pw > CLB_MAX_PW)
-        return host_fail(CLB_EINVAL, "bad window count or NumPW outside 1..3");
-    if (prune_limit < 0) return host_fail(CLB_EINVAL, "prune_limit must be >= 0");
-    if (n_windows > 0 && (check_side(g1, n_windows) || check_side(g2, n_windows))) return host_fail(CLB_EINVAL, "null graph arrays");
-    if (n_windows > 0 && (!score_out || !aln_off || !aln_pairs || !aln_len)) return host_fail(CLB_EINVAL, "null output arrays");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) return host_fail(CLB_ECUDA, "no CUDA device available (there is no CPU fallback)");
-    if (device < 0 || device >= ndev) return host_fail(CLB_EINVAL, "device index out of range");
-    if (getenv("CLB_COUNT_CALLS")) {  // evidence for integration tests that the GPU path really ran
-        static std::atomic<int64_t> calls(0), windows(0);
-        static std::once_flag once;
-        std::call_once(once, [] {
-            atexit([] { fprintf(stderr, "[clb] pwfa calls %lld windows %lld\n", (long long)calls.load(), (long long)windows.load()); });
-        });
-        calls += 1;
-        windows += n_windows;
-    }
+        return fail(CLB_EINVAL, "bad window count or NumPW outside 1..3");
+    if (prune_limit < 0) return fail(CLB_EINVAL, "prune_limit must be >= 0");
+    if (n_windows > 0 && (clb::check_graph_batch(g1, n_windows) || clb::check_graph_batch(g2, n_windows)))
+        return fail(CLB_EINVAL, "null graph arrays");
+    if (n_windows > 0 && (!score_out || !aln_off || !aln_pairs || !aln_len)) return fail(CLB_EINVAL, "null output arrays");
+    if (const int rc = clb::require_device(device)) return rc;
+    clb::count_call<kPwfaCalls>(n_windows);
     if (n_windows == 0) return CLB_OK;
     const int64_t nw = n_windows;
     const int P = params->num_pw;
@@ -231,11 +150,11 @@ extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_grap
         w_open[k] = 2 * params->gap_open[k];
         w_ext[k] = 2 * params->gap_extend[k] + params->match;
         if (w_open[k] == 0 || w_ext[k] == 0 || factor == 0)
-            return host_fail(CLB_EINVAL, "pwfa needs non-zero gap_open and mismatch+match (the reference's gcd divides by them)");
+            return fail(CLB_EINVAL, "pwfa needs non-zero gap_open and mismatch+match (the reference's gcd divides by them)");
         factor = gcd_u32(factor, w_open[k]);
         factor = gcd_u32(factor, w_ext[k]);
     }
-    if (factor == 0) return host_fail(CLB_EINVAL, "degenerate scoring parameters");
+    if (factor == 0) return fail(CLB_EINVAL, "degenerate scoring parameters");
     w_mismatch /= factor;
     for (int k = 0; k < P; ++k) {
         w_open[k] /= factor;
@@ -271,12 +190,12 @@ extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_grap
     for (int64_t w = 0; w < nw; ++w) {
         const int64_t n1 = g1->node_off[w + 1] - g1->node_off[w], n2 = g2->node_off[w + 1] - g2->node_off[w];
         if (n1 < 0 || n2 < 0 || n1 >= (int64_t(1) << 30) || n2 >= (int64_t(1) << 28))
-            return host_fail(CLB_EINVAL, "window size out of range");
+            return fail(CLB_EINVAL, "window size out of range");
         // WFA scores are kept in 29 bits: every step costs at most max_pen
         if ((uint64_t)(n1 + n2 + 2) * (max_pen + 1) >= (uint64_t(1) << 29))
-            return host_fail(CLB_EINVAL, "window " + std::to_string(w) + ": WFA score range exceeds 29 bits");
+            return fail(CLB_EINVAL, "window " + std::to_string(w) + ": WFA score range exceeds 29 bits");
         if (aln_off[w + 1] - aln_off[w] < n1 + n2)
-            return host_fail(CLB_EINVAL, "alignment capacity of window " + std::to_string(w) + " is below n1+n2");
+            return fail(CLB_EINVAL, "alignment capacity of window " + std::to_string(w) + " is below n1+n2");
         clb::PwfaWindow& W = win[w];
         W.n1 = (uint32_t)n1;
         W.n2 = (uint32_t)n2;
@@ -298,42 +217,24 @@ extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_grap
     }
     out_off[nw] = tot_pairs;
 
-    if (cudaSetDevice(device) != cudaSuccess) return host_fail(CLB_ECUDA, "cudaSetDevice failed");
+    if (cudaSetDevice(device) != cudaSuccess) return fail(CLB_ECUDA, "cudaSetDevice failed");
     SideOut so[2];
     for (int sd = 0; sd < 2; ++sd)
-        if (!so[sd].info.alloc(device, tot_info[sd], true) || !so[sd].next.alloc(device, tot_next[sd], true) ||
-            !so[sd].nlab.alloc(device, tot_next[sd], true))
-            return host_fail(CLB_ENOMEM, "pwfa: staging allocation failed");
+        if (so[sd].info.alloc(device, tot_info[sd], true) || so[sd].next.alloc(device, tot_next[sd], true) ||
+            so[sd].nlab.alloc(device, tot_next[sd], true))
+            return fail(CLB_ENOMEM, "pwfa: staging allocation failed");
     {
-        std::atomic<int64_t> next_w{0};
-        std::atomic<int> st{CLB_OK};
-        std::atomic<int64_t> bad{-1};
-        unsigned nthreads = std::max(1u, std::min(32u, std::thread::hardware_concurrency()));
-        if (nw < 8) nthreads = 1;
-        auto worker = [&]() {
-            Scratch sc;
-            for (;;) {
-                const int64_t w = next_w.fetch_add(1);
-                if (w >= nw || st.load() != CLB_OK) return;
-                int r = flatten_side(*g1, w, so[0].info.h + win[w].info1, so[0].next.h + win[w].next1,
-                                     so[0].nlab.h + win[w].next1, sc);
-                if (r == CLB_OK)
-                    r = flatten_side(*g2, w, so[1].info.h + win[w].info2, so[1].next.h + win[w].next2,
-                                     so[1].nlab.h + win[w].next2, sc);
-                if (r != CLB_OK) {
-                    st.store(r);
-                    bad.store(w);
-                    return;
-                }
-            }
-        };
-        std::vector<std::thread> th;
-        for (unsigned t = 1; t < nthreads; ++t) th.emplace_back(worker);
-        worker();
-        for (auto& t : th) t.join();
-        if (st.load() != CLB_OK)
-            return host_fail(st.load(), "window " + std::to_string(bad.load()) +
-                                            (st.load() == CLB_ECYCLE ? ": graph has a cycle" : ": malformed graph arrays"));
+        std::vector<Scratch> scratch(clb::pool_threads(nw, 8));
+        int64_t bad = -1;
+        const int r = clb::for_each_window(nw, 1, 8, [&](unsigned t, int64_t w) {
+            const int r1 = flatten_side(*g1, w, so[0].info.h + win[w].info1, so[0].next.h + win[w].next1,
+                                        so[0].nlab.h + win[w].next1, scratch[t]);
+            if (r1 != CLB_OK) return r1;
+            return flatten_side(*g2, w, so[1].info.h + win[w].info2, so[1].next.h + win[w].next2, so[1].nlab.h + win[w].next2,
+                                scratch[t]);
+        }, &bad);
+        if (r != CLB_OK)
+            return fail(r, "window " + std::to_string(bad) + (r == CLB_ECYCLE ? ": graph has a cycle" : ": malformed graph arrays"));
     }
 
     int rc = CLB_OK;
@@ -348,20 +249,20 @@ extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_grap
     int64_t h2d = 0;
     cudaDeviceProp prop;
 
-    PWFA_CUDA_TRY(cudaGetDeviceProperties(&prop, device));
-    PWFA_CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-    PWFA_CUDA_TRY(cudaEventCreate(&ev0));
-    PWFA_CUDA_TRY(cudaEventCreate(&ev1));
+    CUDA_TRY_CLEANUP(cudaGetDeviceProperties(&prop, device));
+    CUDA_TRY_CLEANUP(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+    CUDA_TRY_CLEANUP(cudaEventCreate(&ev0));
+    CUDA_TRY_CLEANUP(cudaEventCreate(&ev1));
     for (int sd = 0; sd < 2; ++sd) {
-        PWFA_CUDA_TRY(cudaMemcpyAsync(so[sd].info.d, so[sd].info.h, (size_t)tot_info[sd] * sizeof(int4), cudaMemcpyHostToDevice, stream));
-        PWFA_CUDA_TRY(cudaMemcpyAsync(so[sd].next.d, so[sd].next.h, (size_t)tot_next[sd] * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
-        PWFA_CUDA_TRY(cudaMemcpyAsync(so[sd].nlab.d, so[sd].nlab.h, (size_t)tot_next[sd], cudaMemcpyHostToDevice, stream));
+        CUDA_TRY_CLEANUP(cudaMemcpyAsync(so[sd].info.d, so[sd].info.h, (size_t)tot_info[sd] * sizeof(int4), cudaMemcpyHostToDevice, stream));
+        CUDA_TRY_CLEANUP(cudaMemcpyAsync(so[sd].next.d, so[sd].next.h, (size_t)tot_next[sd] * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+        CUDA_TRY_CLEANUP(cudaMemcpyAsync(so[sd].nlab.d, so[sd].nlab.h, (size_t)tot_next[sd], cudaMemcpyHostToDevice, stream));
         h2d += tot_info[sd] * (int64_t)sizeof(int4) + tot_next[sd] * 5;
     }
-    if (!s_win.alloc(device, nw, true) || !s_order.alloc(device, nw, true) || !s_queue.alloc(device, 1, false) ||
-        !s_status.alloc(device, nw, true) || !s_score.alloc(device, nw, true) || !s_wstats.alloc(device, 4 * nw, true) ||
-        !s_len.alloc(device, nw, true) || !s_aln.alloc(device, 2 * tot_pairs, true)) {
-        rc = host_fail(CLB_ENOMEM, "pwfa: result buffer allocation failed");
+    if (s_win.alloc(device, nw, true) || s_order.alloc(device, nw, true) || s_queue.alloc(device, 1, false) ||
+        s_status.alloc(device, nw, true) || s_score.alloc(device, nw, true) || s_wstats.alloc(device, 4 * nw, true) ||
+        s_len.alloc(device, nw, true) || s_aln.alloc(device, 2 * tot_pairs, true)) {
+        rc = fail(CLB_ENOMEM, "pwfa: result buffer allocation failed");
         goto cleanup;
     }
     h2d += nw * (sizeof(clb::PwfaWindow) + sizeof(int32_t));
@@ -369,7 +270,7 @@ extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_grap
     std::iota(pending.begin(), pending.end(), 0);
     for (int round = 0; !pending.empty(); ++round) {
         if (round > 10) {
-            rc = host_fail(CLB_ENOMEM, "pwfa: a window still overflows its tables after 10 enlargements");
+            rc = fail(CLB_ENOMEM, "pwfa: a window still overflows its tables after 10 enlargements");
             goto cleanup;
         }
         std::stable_sort(pending.begin(), pending.end(), [&](int32_t a, int32_t c) {
@@ -380,24 +281,24 @@ extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_grap
             slot_bytes = std::max<int64_t>(slot_bytes, ((int64_t(1) << win[w].hash_log2) +
                                                         (int64_t)prm.n_class * (int64_t(1) << win[w].fifo_log2)) * 16);
         size_t free_b = 0, total_b = 0;
-        PWFA_CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
+        CUDA_TRY_CLEANUP(cudaMemGetInfo(&free_b, &total_b));
         const int warps_per_sm = getenv("CLB_PWFA_WARPS_PER_SM") ? std::max(1, atoi(getenv("CLB_PWFA_WARPS_PER_SM"))) : 16;
         int grid = (int)std::min<int64_t>((int64_t)pending.size(), (int64_t)prop.multiProcessorCount * warps_per_sm);
         grid = (int)std::min<int64_t>(grid, (int64_t)(free_b * 0.9) / slot_bytes);
         if (grid < 1) {
-            rc = host_fail(CLB_ENOMEM, "pwfa: the tables of one window (" + std::to_string(slot_bytes) + " B) do not fit in device memory");
+            rc = fail(CLB_ENOMEM, "pwfa: the tables of one window (" + std::to_string(slot_bytes) + " B) do not fit in device memory");
             goto cleanup;
         }
         s_ws.release();
-        if (!s_ws.alloc(device, (size_t)grid * slot_bytes, false, true)) {
-            rc = host_fail(CLB_ENOMEM, "pwfa: workspace allocation failed");
+        if (s_ws.alloc(device, (size_t)grid * slot_bytes, false, true)) {
+            rc = fail(CLB_ENOMEM, "pwfa: workspace allocation failed");
             goto cleanup;
         }
         memcpy(s_win.h, win.data(), nw * sizeof(clb::PwfaWindow));
         memcpy(s_order.h, pending.data(), pending.size() * sizeof(int32_t));
-        PWFA_CUDA_TRY(cudaMemcpyAsync(s_win.d, s_win.h, nw * sizeof(clb::PwfaWindow), cudaMemcpyHostToDevice, stream));
-        PWFA_CUDA_TRY(cudaMemcpyAsync(s_order.d, s_order.h, pending.size() * sizeof(int32_t), cudaMemcpyHostToDevice, stream));
-        PWFA_CUDA_TRY(cudaMemsetAsync(s_queue.d, 0, sizeof(int32_t), stream));
+        CUDA_TRY_CLEANUP(cudaMemcpyAsync(s_win.d, s_win.h, nw * sizeof(clb::PwfaWindow), cudaMemcpyHostToDevice, stream));
+        CUDA_TRY_CLEANUP(cudaMemcpyAsync(s_order.d, s_order.h, pending.size() * sizeof(int32_t), cudaMemcpyHostToDevice, stream));
+        CUDA_TRY_CLEANUP(cudaMemsetAsync(s_queue.d, 0, sizeof(int32_t), stream));
         clb::PwfaArgs a{};
         a.info1 = so[0].info.d; a.info2 = so[1].info.d;
         a.next1 = so[0].next.d; a.next2 = so[1].next.d;
@@ -406,14 +307,14 @@ extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_grap
         a.workspace = s_ws.d; a.slot_bytes = slot_bytes;
         a.score = s_score.d; a.status = s_status.d; a.aln_len = s_len.d; a.aln = s_aln.d; a.wstats = s_wstats.d;
         a.prm = prm;
-        PWFA_CUDA_TRY(cudaEventRecord(ev0, stream));
-        PWFA_CUDA_TRY(clb::launch_pwfa(a, grid, stream));
-        PWFA_CUDA_TRY(cudaEventRecord(ev1, stream));
-        PWFA_CUDA_TRY(cudaMemcpyAsync(s_status.h, s_status.d, nw * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
-        PWFA_CUDA_TRY(cudaMemcpyAsync(s_wstats.h, s_wstats.d, 4 * nw * sizeof(int64_t), cudaMemcpyDeviceToHost, stream));
-        PWFA_CUDA_TRY(cudaStreamSynchronize(stream));
+        CUDA_TRY_CLEANUP(cudaEventRecord(ev0, stream));
+        CUDA_TRY_CLEANUP(clb::launch_pwfa(a, grid, stream));
+        CUDA_TRY_CLEANUP(cudaEventRecord(ev1, stream));
+        CUDA_TRY_CLEANUP(cudaMemcpyAsync(s_status.h, s_status.d, nw * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+        CUDA_TRY_CLEANUP(cudaMemcpyAsync(s_wstats.h, s_wstats.d, 4 * nw * sizeof(int64_t), cudaMemcpyDeviceToHost, stream));
+        CUDA_TRY_CLEANUP(cudaStreamSynchronize(stream));
         float ms = 0.f;
-        PWFA_CUDA_TRY(cudaEventElapsedTime(&ms, ev0, ev1));
+        CUDA_TRY_CLEANUP(cudaEventElapsedTime(&ms, ev0, ev1));
         if (stats) {
             stats->kernel_ms += ms;
             stats->kernel_launches += 1;
@@ -436,19 +337,19 @@ extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_grap
                 again.push_back(w);
             } else if (s == clb::kPwfaQueueDry) {
                 // the reference dereferences an empty deque here (alignment.hpp:1738): its precondition is violated
-                rc = host_fail(CLB_EINVAL, "window " + std::to_string(w) + ": no source reaches a sink within the pruning rule");
+                rc = fail(CLB_EINVAL, "window " + std::to_string(w) + ": no source reaches a sink within the pruning rule");
                 goto cleanup;
             } else {
-                rc = host_fail(CLB_ECUDA, "window " + std::to_string(w) + ": internal pwfa kernel error " + std::to_string(s));
+                rc = fail(CLB_ECUDA, "window " + std::to_string(w) + ": internal pwfa kernel error " + std::to_string(s));
                 goto cleanup;
             }
         }
         pending.swap(again);
     }
-    PWFA_CUDA_TRY(cudaMemcpyAsync(s_score.h, s_score.d, nw * sizeof(int64_t), cudaMemcpyDeviceToHost, stream));
-    PWFA_CUDA_TRY(cudaMemcpyAsync(s_len.h, s_len.d, nw * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
-    PWFA_CUDA_TRY(cudaMemcpyAsync(s_aln.h, s_aln.d, 2 * tot_pairs * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
-    PWFA_CUDA_TRY(cudaStreamSynchronize(stream));
+    CUDA_TRY_CLEANUP(cudaMemcpyAsync(s_score.h, s_score.d, nw * sizeof(int64_t), cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY_CLEANUP(cudaMemcpyAsync(s_len.h, s_len.d, nw * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY_CLEANUP(cudaMemcpyAsync(s_aln.h, s_aln.d, 2 * tot_pairs * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY_CLEANUP(cudaStreamSynchronize(stream));
     for (int64_t w = 0; w < nw; ++w) {
         const uint32_t len = s_len.h[w];
         const int64_t cap = out_off[w + 1] - out_off[w];
