@@ -82,6 +82,10 @@ def _bind(lib):
     lib.clb_chain_dp_batch.restype = ctypes.c_int
     lib.clb_chain_dp_batch.argtypes = [ctypes.c_int, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
                                        ctypes.c_void_p, ctypes.c_void_p, ctypes.POINTER(ChainStats)]
+    lib.clb_chain_dp_batch_multi.restype = ctypes.c_int
+    lib.clb_chain_dp_batch_multi.argtypes = [ctypes.c_int, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p,
+                                             ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                             ctypes.POINTER(ChainStats)]
     lib._chain_bound = True
 
 
@@ -102,6 +106,21 @@ def _c_problem(problem: ChainProblem):
 def chain_dp_batch(problems, device: int = 0, stats: Optional[ChainStats] = None):
     """``clb_chain_dp_batch``: many independent problems in one call (one launch for all that fit shared memory).
     Returns a list of (chain ranks, dp values, back-pointers, optimum), one per problem."""
+    return _chain_batch(problems, stats, lambda lib, *args: lib.clb_chain_dp_batch(device, *args))
+
+
+def chain_dp_batch_multi(problems, devices, stats: Optional[ChainStats] = None, return_parts: bool = False):
+    """``clb_chain_dp_batch_multi``: the problems dealt to several GPUs of one box by their step, insert and query counts,
+    ``clb_chain_dp_batch`` on each device's share.  ``devices`` is a list of distinct device ordinals.  Returns the list of
+    ``chain_dp_batch``, plus the index into ``devices`` each problem ran on if ``return_parts``."""
+    devs = np.ascontiguousarray(list(devices), np.int32)
+    parts = np.zeros(max(1, len(problems)), np.int32)
+    out = _chain_batch(problems, stats, lambda lib, n, *args: lib.clb_chain_dp_batch_multi(
+        len(devs), devs.ctypes.data, n, *args[:-1], parts.ctypes.data, args[-1]))
+    return (out, parts[: len(problems)]) if return_parts else out
+
+
+def _chain_batch(problems, stats, call):
     lib = load_library()
     _bind(lib)
     n = len(problems)
@@ -115,9 +134,9 @@ def chain_dp_batch(problems, device: int = 0, stats: Optional[ChainStats] = None
     PP = ctypes.POINTER(_CProblem) * max(1, n)
     VP = ctypes.c_void_p * max(1, n)
     parr = PP(*[ctypes.pointer(c[0]) for c in cps]) if n else PP()
-    _check(lib.clb_chain_dp_batch(device, n, parr, VP(*[a.ctypes.data for a in dps]), VP(*[a.ctypes.data for a in bps]),
-                                  VP(*[a.ctypes.data for a in chains]), lens.ctypes.data, opts.ctypes.data,
-                                  ctypes.byref(stats) if stats is not None else None))
+    _check(call(lib, n, parr, VP(*[a.ctypes.data for a in dps]), VP(*[a.ctypes.data for a in bps]),
+                VP(*[a.ctypes.data for a in chains]), lens.ctypes.data, opts.ctypes.data,
+                ctypes.byref(stats) if stats is not None else None))
     return [(chains[k][: int(lens[k])].copy(), dps[k][: ms[k]], bps[k][: ms[k]], float(opts[k])) for k in range(n)]
 
 
@@ -170,6 +189,36 @@ def chain_dp(problem: ChainProblem, device: int = 0, stats: Optional[ChainStats]
     _check(lib.clb_chain_dp(device, ctypes.byref(cp), dp.ctypes.data, bp.ctypes.data, chain.ctypes.data, ctypes.byref(n),
                             ctypes.byref(opt), ctypes.byref(stats) if stats is not None else None))
     return chain[: n.value].copy(), dp[:m], bp[:m], float(opt.value)
+
+
+def synth_fill_in_problems(n_problems: int, seed: int = 0, matches=(20, 60), num_pw=(0, 1, 3)):
+    """Independent random problems of the size the Anchorer's fill-in pass makes (a few dozen matches on one path per
+    graph), for tests and benchmarks of the batched calls.  Every array is in range and every DP is well defined; the
+    values mean nothing.  Problem k has ``num_pw[k % len(num_pw)]`` gap pieces."""
+    rng = np.random.default_rng(seed)
+    out = []
+    for k in range(n_problems):
+        P = num_pw[k % len(num_pw)]
+        M = int(rng.integers(matches[0], matches[1] + 1))
+        n1 = 4 * M + 8  # nodes of graph 1 = steps
+        ln = rng.integers(2, 6, M)
+        s1 = rng.integers(0, n1 - 6, M)
+        s2 = np.clip(s1 + rng.integers(-5, 6, M), 0, n1 - 6)
+        e1, e2 = s1 + ln - 1, s2 + ln - 1
+        ends = sorted(range(M), key=lambda m: (e1[m], m))
+        starts = sorted((m for m in range(M) if s1[m] > 0), key=lambda m: (s1[m], m))  # queried from the edge s1-1 -> s1
+        end_off = np.searchsorted(e1[ends], np.arange(n1 + 1), side="left").astype(np.int64)
+        qry_off = np.searchsorted(s1[starts] - 1, np.arange(n1 + 1), side="left").astype(np.int64)
+        w = ln.astype(np.float32)
+        a = dict(weight=w, dp_init=(w - 0.1 * s1).astype(np.float32), final_term=(-0.05 * (n1 - e1)).astype(np.float32),
+                 end_off=end_off, end_match=np.asarray(ends, np.uint32), qry_off=qry_off,
+                 qry_match=np.asarray(starts, np.uint32), qry_chain1=np.zeros(len(starts), np.uint32),
+                 ins_off=np.arange(M + 1, dtype=np.int64), ins_p1=np.zeros(M, np.uint32), ins_p2=np.zeros(M, np.uint32),
+                 ins_shift=(e1 - e2).astype(np.int32), ins_offset=e2.astype(np.uint32), ins_active=np.ones(M, np.uint8),
+                 qa1=(s1 - 1).astype(np.int32), qa2=(s2 - 1).astype(np.int32), qoff=s2.astype(np.uint32))
+        kp = max(1, P)
+        out.append(ChainProblem(P, (1.0, 2.0, 3.0)[:kp], (0.5, 0.2, 0.1)[:kp], 1.0, 1, 1, 0.0, a))
+    return out
 
 
 _DTYPES = {0: np.float32, 1: np.int32, 2: np.uint32, 3: np.int64, 4: np.float64}

@@ -19,7 +19,7 @@
 #include "host_common.cuh"
 
 namespace clb {
-cudaError_t launch_chain(ChainArgs args, int grid, int cluster, int prepare_grid, cudaStream_t stream, cudaEvent_t after_prepare);
+cudaError_t launch_chain(ChainArgs args, int grid, int* cluster, int prepare_grid, cudaStream_t stream, cudaEvent_t after_prepare);
 cudaError_t launch_chain_small_batch(const ChainArgs* d_args, int n, int smem_bytes, bool any_global, cudaStream_t stream);
 int chain_max_grid(int device);
 }  // namespace clb
@@ -63,8 +63,35 @@ constexpr size_t kArenaKeep = size_t(1) << 30;
 constexpr size_t kDirectCopyBytes = size_t(32) << 20;  // copy regions above this size go to the device without a pinned staging twin
 constexpr size_t kChainBatchArena = size_t(4) << 20;  // a problem up to this arena size joins a batched launch (one CTA per problem)
 constexpr int kChainClusterMax = 16;  // CTAs of the cluster a mid-sized problem runs in (non-portable size; launch_chain halves it if refused)
-std::mutex g_arena_mu;
-std::map<int, DeviceArena> g_arenas;
+
+// State kept per device ordinal, each behind its own mutex: calls on one device are serialised, calls on different devices
+// are not.  A slot is made on first use and never erased, so a reference to it stays valid while others are added.
+template <class T>
+class PerDevice {
+public:
+    struct Slot {
+        std::mutex mu;
+        T state;
+    };
+    Slot& at(int device) {
+        std::lock_guard<std::mutex> lk(mu_);
+        return slots_[device];
+    }
+    // fn(device, state) for every slot, each under its own lock
+    template <class Fn>
+    void for_each(const Fn& fn) {
+        std::lock_guard<std::mutex> lk(mu_);
+        for (auto& kv : slots_) {
+            std::lock_guard<std::mutex> ls(kv.second.mu);
+            fn(kv.first, kv.second.state);
+        }
+    }
+
+private:
+    std::mutex mu_;
+    std::map<int, Slot> slots_;
+};
+PerDevice<DeviceArena> g_arenas;
 
 // fn(begin, end) over [0, n) on up to 16 host threads (the layout of a million-match problem is tens of millions of
 // small steps; the Anchorer calls us from one thread)
@@ -517,8 +544,9 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
     std::vector<float> h_dp(M);
     std::vector<uint32_t> h_bp(M);
     int grid = 1;
-    std::lock_guard<std::mutex> arena_lock(g_arena_mu);
-    DeviceArena& ar = g_arenas[device];
+    auto& arena_slot = g_arenas.at(device);
+    std::lock_guard<std::mutex> arena_lock(arena_slot.mu);
+    DeviceArena& ar = arena_slot.state;
     bool keep = true;
     {
         ArenaPlan plan;
@@ -666,7 +694,7 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
         if (total <= (size_t)clb::kChainSmallArena && !getenv("CLB_CHAIN_NO_SMALL") && !getenv("CLB_CHAIN_GRID")) grid = 0;
         const int prepare_grid = (int)std::max<int64_t>(1, std::min<int64_t>((n_qry * C2 + 7) / 8, 8 * (int64_t)max_grid));
         CUDA_TRY_CLEANUP(cudaEventRecord(ar.ev0, ar.stream));
-        CUDA_TRY_CLEANUP(clb::launch_chain(a, grid, cluster, prepare_grid, ar.stream, ar.evp));
+        CUDA_TRY_CLEANUP(clb::launch_chain(a, grid, &cluster, prepare_grid, ar.stream, ar.evp));
         CUDA_TRY_CLEANUP(cudaEventRecord(ar.ev1, ar.stream));
         CUDA_TRY_CLEANUP(cudaMemcpyAsync(h_dp.data(), a.dp, M * sizeof(float), cudaMemcpyDeviceToHost, ar.stream));
         CUDA_TRY_CLEANUP(cudaMemcpyAsync(h_bp.data(), a.backptr, M * sizeof(uint32_t), cudaMemcpyDeviceToHost, ar.stream));
@@ -711,8 +739,8 @@ cleanup:
     return rc;
 }
 
-// Device and pinned buffers of the batched path, per device, grown on demand and kept (g_batch_mu serialises the flushes of
-// a process: a flush is one copy in, one launch, one copy out).
+// Device and pinned buffers of the batched path, per device, grown on demand and kept (the flushes of one device are
+// serialised: a flush is one copy in, one launch, one copy out).
 namespace {
 struct BatchArena {
     char* d_arena = nullptr; size_t arena_cap = 0;
@@ -724,8 +752,7 @@ struct BatchArena {
     cudaStream_t stream = nullptr;
     cudaEvent_t e0 = nullptr, e1 = nullptr;
 };
-std::mutex g_batch_mu;
-std::map<int, BatchArena> g_batch_arenas;
+PerDevice<BatchArena> g_batch_arenas;
 
 template <class T>
 cudaError_t grow_device(T*& ptr, size_t& cap, size_t want) {
@@ -762,8 +789,9 @@ int flush_contexts(int device, BatchCtx* const* ctxs, int64_t n_ctx, clb_chain_s
     }
     if (nb == 0) return CLB_OK;
     int rc = CLB_OK;
-    std::lock_guard<std::mutex> lk(g_batch_mu);
-    BatchArena& ba = g_batch_arenas[device];
+    auto& batch_slot = g_batch_arenas.at(device);
+    std::lock_guard<std::mutex> lk(batch_slot.mu);
+    BatchArena& ba = batch_slot.state;
     const double t_start = now_ms();
     CUDA_TRY(cudaSetDevice(device));
     if (!ba.stream) {
@@ -879,6 +907,62 @@ extern "C" int clb_chain_dp_batch(int device, int64_t n_problems, const clb_chai
     return CLB_OK;
 }
 
+// The batched call over several devices: the problems are dealt by a work estimate and every device runs
+// clb_chain_dp_batch on its share, from its own host thread.
+extern "C" int clb_chain_dp_batch_multi(int n_devices, const int* devices, int64_t n_problems, const clb_chain_problem* const* problems,
+                                        float* const* dp_out, int64_t* const* backptr_out, int64_t* const* chain_out, int64_t* chain_len,
+                                        float* opt_score, int32_t* part_out, clb_chain_stats* stats) {
+    const double t_start = now_ms();
+    if (stats) memset(stats, 0, sizeof(*stats));
+    if (const int rc = clb::check_devices(n_devices, devices, "clb_chain_dp_batch_multi")) return rc;
+    if (n_problems < 0 || n_problems >= (int64_t(1) << 31) || (n_problems > 0 && (!problems || !chain_out || !chain_len)))
+        return fail(CLB_EINVAL, "clb_chain_dp_batch_multi: null arguments or too many problems");
+    for (int k = 0; k < n_devices; ++k)
+        if (const int rc = clb::require_device(devices[k])) return rc;
+    // the DP costs about a step's latency times the steps (DESIGN.md section 10), and the layout grows with the events
+    std::vector<int64_t> cost((size_t)n_problems);
+    for (int64_t k = 0; k < n_problems; ++k) {
+        const clb_chain_problem* p = problems[k];
+        if (!p || !chain_out[k]) return fail(CLB_EINVAL, "clb_chain_dp_batch_multi: null problem or output");
+        cost[k] = std::max<int64_t>(0, p->n_step) + (p->ins_off && p->n_match > 0 ? p->ins_off[p->n_match] : 0) +
+                  (p->qry_off && p->n_step > 0 ? p->qry_off[p->n_step] : 0);
+    }
+    std::vector<clb_chain_stats> dev_stats(n_devices);
+    const int rc = clb::deal_to_devices(n_devices, devices, (int32_t)n_problems, cost.data(), part_out, [&](int d, const std::vector<int32_t>& sel) -> int {
+        // the share's pointers in share order; chain lengths and optima come back through local arrays
+        const size_t n = sel.size();
+        std::vector<const clb_chain_problem*> ps(n);
+        std::vector<float*> dps(n, nullptr);
+        std::vector<int64_t*> bps(n, nullptr), chains(n);
+        std::vector<int64_t> lens(n, 0);
+        std::vector<float> opts(n, 0.f);
+        for (size_t i = 0; i < n; ++i) {
+            ps[i] = problems[sel[i]];
+            if (dp_out) dps[i] = dp_out[sel[i]];
+            if (backptr_out) bps[i] = backptr_out[sel[i]];
+            chains[i] = chain_out[sel[i]];
+        }
+        const int r = clb_chain_dp_batch(devices[d], (int64_t)n, ps.data(), dps.data(), bps.data(), chains.data(), lens.data(), opts.data(),
+                                         stats ? &dev_stats[d] : nullptr);
+        if (r != CLB_OK) return r;
+        for (size_t i = 0; i < n; ++i) {
+            chain_len[sel[i]] = lens[i];
+            if (opt_score) opt_score[sel[i]] = opts[i];
+        }
+        return CLB_OK;
+    });
+    if (rc != CLB_OK) return rc;
+    if (stats) {
+        for (const clb_chain_stats& one : dev_stats) {
+            stats->build_ms += one.build_ms; stats->kernel_ms += one.kernel_ms; stats->steps += one.steps; stats->inserts += one.inserts;
+            stats->queries += one.queries; stats->tree_bytes += one.tree_bytes; stats->h2d_bytes += one.h2d_bytes;
+            stats->d2h_bytes += one.d2h_bytes; stats->kernel_launches += one.kernel_launches;
+        }
+        stats->total_ms = now_ms() - t_start;
+    }
+    return CLB_OK;
+}
+
 // The same in two halves, for callers that prepare problems on several host threads (the drop-in Anchorer runs the
 // fill-in subproblems of anchorer.hpp:657-693 on a thread pool): clb_chain_job_create lays one problem out in the CALLING
 // thread -- no device work, thread-safe -- and clb_chain_jobs_run solves the jobs of any number of threads in one launch.
@@ -932,21 +1016,18 @@ extern "C" void clb_chain_job_destroy(clb_chain_job* job) { delete job; }
 
 namespace clb {
 void chain_release_cache() {
-    std::lock_guard<std::mutex> lk(g_arena_mu);
-    for (auto& kv : g_arenas) {
-        cudaSetDevice(kv.first);
-        if (kv.second.d) cudaFree(kv.second.d);
-        if (kv.second.h) cudaFreeHost(kv.second.h);
-        if (kv.second.ev0) cudaEventDestroy(kv.second.ev0);
-        if (kv.second.ev1) cudaEventDestroy(kv.second.ev1);
-        if (kv.second.evp) cudaEventDestroy(kv.second.evp);
-        if (kv.second.stream) cudaStreamDestroy(kv.second.stream);
-    }
-    g_arenas.clear();
-    std::lock_guard<std::mutex> lb(g_batch_mu);
-    for (auto& kv : g_batch_arenas) {
-        cudaSetDevice(kv.first);
-        BatchArena& b = kv.second;
+    g_arenas.for_each([](int device, DeviceArena& a) {
+        cudaSetDevice(device);
+        if (a.d) cudaFree(a.d);
+        if (a.h) cudaFreeHost(a.h);
+        if (a.ev0) cudaEventDestroy(a.ev0);
+        if (a.ev1) cudaEventDestroy(a.ev1);
+        if (a.evp) cudaEventDestroy(a.evp);
+        if (a.stream) cudaStreamDestroy(a.stream);
+        a = DeviceArena{};
+    });
+    g_batch_arenas.for_each([](int device, BatchArena& b) {
+        cudaSetDevice(device);
         if (b.d_arena) cudaFree(b.d_arena);
         if (b.d_args) cudaFree(b.d_args);
         if (b.d_dp) cudaFree(b.d_dp);
@@ -957,7 +1038,7 @@ void chain_release_cache() {
         if (b.e0) cudaEventDestroy(b.e0);
         if (b.e1) cudaEventDestroy(b.e1);
         if (b.stream) cudaStreamDestroy(b.stream);
-    }
-    g_batch_arenas.clear();
+        b = BatchArena{};
+    });
 }
 }  // namespace clb

@@ -660,28 +660,25 @@ __global__ void __launch_bounds__(kThreads, 1) chain_small_batch_kernel(const Ch
     }
 }
 
+// Function attributes belong to the current device, so they are set at every launch (a process may chain on several
+// devices); setting one costs a few microseconds of host time.
 cudaError_t launch_chain_small_batch(const ChainArgs* d_args, int n, int smem_bytes, bool any_global, cudaStream_t stream) {
-    static bool attr_set = false;
-    if (!attr_set) {
-        cudaError_t e0 = cudaFuncSetAttribute(chain_small_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kChainSmallArena);
-        if (e0 != cudaSuccess) return e0;
-        attr_set = true;
-    }
+    const cudaError_t e0 = cudaFuncSetAttribute(chain_small_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kChainSmallArena);
+    if (e0 != cudaSuccess) return e0;
     if (any_global) chain_batch_prepare_kernel<<<n, 256, 0, stream>>>(d_args);
     chain_small_batch_kernel<<<n, kThreads, (size_t)smem_bytes, stream>>>(d_args);
     return cudaGetLastError();
 }
 
-// grid == 0: the whole problem fits into shared memory (one CTA).  Otherwise one CTA, or `cluster` > 1 CTAs of ONE
+// grid == 0: the whole problem fits into shared memory (one CTA).  Otherwise one CTA, or `*cluster` > 1 CTAs of ONE
 // thread-block cluster (hardware barrier between the phases of a step), or a cooperative grid of `grid` > 1 CTAs.
-cudaError_t launch_chain(ChainArgs args, int grid, int cluster, int prepare_grid, cudaStream_t stream, cudaEvent_t after_prepare) {
+// On return *cluster is the cluster size the kernel was launched with (1 without a cluster).
+cudaError_t launch_chain(ChainArgs args, int grid, int* cluster_io, int prepare_grid, cudaStream_t stream, cudaEvent_t after_prepare) {
+    int cluster = *cluster_io;
+    *cluster_io = 1;
     if (grid == 0) {
-        static bool attr_set = false;
-        if (!attr_set) {
-            cudaError_t e0 = cudaFuncSetAttribute(chain_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kChainSmallArena);
-            if (e0 != cudaSuccess) return e0;
-            attr_set = true;
-        }
+        const cudaError_t e0 = cudaFuncSetAttribute(chain_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kChainSmallArena);
+        if (e0 != cudaSuccess) return e0;
         if (after_prepare) cudaEventRecord(after_prepare, stream);
         chain_small_kernel<<<1, kThreads, (size_t)((args.arena_bytes + 15) / 16 * 16), stream>>>(args);
         return cudaGetLastError();
@@ -693,14 +690,9 @@ cudaError_t launch_chain(ChainArgs args, int grid, int cluster, int prepare_grid
     const ChainKernel kern = chain_kernel_for(args.num_pw);
     const int threads = args.num_pw == 0 ? kThreadsGapFree : kThreads;
     if (cluster > 1) {
-        static bool attr_set = false;
-        if (!attr_set) {  // clusters of 16; a refusal shows at launch
-            cudaFuncSetAttribute(chain_kernel<0>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-            cudaFuncSetAttribute(chain_kernel<1>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-            cudaFuncSetAttribute(chain_kernel<7>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-            cudaGetLastError();
-            attr_set = true;
-        }
+        // clusters of 16 on the current device; a refusal shows at launch
+        cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+        cudaGetLastError();
         args.sync_mode = 1;
         for (; cluster > 1; cluster /= 2) {  // a cluster size the device cannot place falls back to the next smaller one
             cudaLaunchConfig_t cfg = {};
@@ -715,7 +707,10 @@ cudaError_t launch_chain(ChainArgs args, int grid, int cluster, int prepare_grid
             cfg.attrs = at;
             cfg.numAttrs = 1;
             e = cudaLaunchKernelEx(&cfg, kern, args);
-            if (e == cudaSuccess) return e;
+            if (e == cudaSuccess) {
+                *cluster_io = cluster;
+                return e;
+            }
             cudaGetLastError();
         }
     }

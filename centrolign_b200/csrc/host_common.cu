@@ -63,6 +63,14 @@ int require_device(int device) {
     return CLB_OK;
 }
 
+int check_devices(int n_devices, const int* devices, const char* who) {
+    if (n_devices < 1 || !devices) return fail(CLB_EINVAL, std::string(who) + ": no devices");
+    for (int a = 0; a < n_devices; ++a)
+        for (int c = a + 1; c < n_devices; ++c)
+            if (devices[a] == devices[c]) return fail(CLB_EINVAL, std::string(who) + ": a device is listed twice");
+    return CLB_OK;
+}
+
 }  // namespace clb
 
 // Context creation off the critical path: a process that knows it will use `device` calls this first thing; the CUDA

@@ -220,6 +220,37 @@ int for_each_window(int64_t n, int64_t grain, int64_t serial_below, const Fn& fn
     return status.load();
 }
 
+// CLB_EINVAL unless devices[] lists n_devices >= 1 ordinals, none twice.  `who` starts the message.
+int check_devices(int n_devices, const int* devices, const char* who);
+
+// The scaffolding of the _multi entry points.  Deals n_items independent items to the devices with clb_balanced_partition
+// on cost[] (the part index per item goes to part_out if it is not null), then runs run(k, sel) -> CLB code on one host
+// thread per device that got items, where sel lists the items of devices[k] in ascending order.  Returns the first failure
+// in device order, its message prefixed with "device <ordinal>: ".
+template <class Fn>
+int deal_to_devices(int n_devices, const int* devices, int32_t n_items, const int64_t* cost, int32_t* part_out, const Fn& run) {
+    std::vector<int32_t> part(n_items);
+    const int rc = clb_balanced_partition(n_items, cost, n_devices, part.data());
+    if (rc != CLB_OK) return rc;
+    if (part_out) std::copy(part.begin(), part.end(), part_out);
+    std::vector<std::vector<int32_t>> sel(n_devices);
+    for (int32_t w = 0; w < n_items; ++w) sel[part[w]].push_back(w);
+    // each thread has its own CUDA context binding and error string; the error strings are handed to the caller's thread
+    std::vector<int> rcs(n_devices, CLB_OK);
+    std::vector<std::string> errs(n_devices);
+    std::vector<std::thread> pool;
+    for (int k = 0; k < n_devices; ++k)
+        if (!sel[k].empty())
+            pool.emplace_back([&, k] {
+                rcs[k] = run(k, sel[k]);
+                if (rcs[k] != CLB_OK) errs[k] = clb_last_error();
+            });
+    for (auto& t : pool) t.join();
+    for (int k = 0; k < n_devices; ++k)
+        if (rcs[k] != CLB_OK) return fail(rcs[k], "device " + std::to_string(devices[k]) + ": " + errs[k]);
+    return CLB_OK;
+}
+
 // CLB_COUNT_CALLS: evidence for integration tests that the GPU path really ran.  Counts the calls of an entry point and
 // their windows, and prints "<kPrefix>calls C windows W" at exit.
 template <const char* kPrefix>

@@ -694,10 +694,7 @@ int clb_balanced_partition(int32_t n_windows, const int64_t* cells, int n_parts,
 int clb_popoa_batch_multi(int n_devices, const int* devices, int32_t n_windows, const clb_graph_batch* g1,
                           const clb_graph_batch* g2, const clb_params* params, int64_t* score_out, const int64_t* aln_off,
                           int32_t* aln_pairs, uint32_t* aln_len, int32_t* part_out) {
-    if (n_devices < 1 || !devices) return fail(CLB_EINVAL, "clb_popoa_batch_multi: no devices");
-    for (int a = 0; a < n_devices; ++a)
-        for (int c = a + 1; c < n_devices; ++c)
-            if (devices[a] == devices[c]) return fail(CLB_EINVAL, "clb_popoa_batch_multi: a device is listed twice");
+    if (const int rc = clb::check_devices(n_devices, devices, "clb_popoa_batch_multi")) return rc;
     if (n_devices == 1 || n_windows <= 1) {
         if (part_out) for (int32_t w = 0; w < n_windows; ++w) part_out[w] = 0;
         return clb_popoa_batch(devices[0], n_windows, g1, g2, params, score_out, aln_off, aln_pairs, aln_len);
@@ -707,32 +704,16 @@ int clb_popoa_batch_multi(int n_devices, const int* devices, int32_t n_windows, 
     std::vector<int64_t> cells(n_windows);
     for (int32_t w = 0; w < n_windows; ++w)
         cells[w] = (g1->node_off[w + 1] - g1->node_off[w] + 1) * (g2->node_off[w + 1] - g2->node_off[w] + 1);
-    std::vector<int32_t> part(n_windows);
-    int rc = clb_balanced_partition(n_windows, cells.data(), n_devices, part.data());
-    if (rc != CLB_OK) return rc;
-    if (part_out) memcpy(part_out, part.data(), n_windows * sizeof(int32_t));
-    std::vector<std::vector<int32_t>> sel(n_devices);
-    for (int32_t w = 0; w < n_windows; ++w) sel[part[w]].push_back(w);
     // one host thread (and CUDA context) per device; each writes only its own windows' entries of the output arrays
-    std::vector<int> rcs(n_devices, CLB_OK);
-    std::vector<std::string> errs(n_devices);
-    std::vector<std::thread> pool;
-    for (int k = 0; k < n_devices; ++k)
-        pool.emplace_back([&, k] {
-            if (sel[k].empty()) return;
-            clb_batch* b = nullptr;
-            int r = create_internal(devices[k], n_windows, g1, g2, params, sel[k].data(), (int32_t)sel[k].size(), &b);
-            if (r == CLB_OK) r = clb_batch_upload(b);
-            if (r == CLB_OK) r = clb_batch_run(b);
-            if (r == CLB_OK) r = clb_batch_download(b, score_out, aln_off, aln_pairs, aln_len);
-            clb_batch_destroy(b);
-            rcs[k] = r;
-            if (r != CLB_OK) errs[k] = clb_last_error();  // thread-local: hand it to the caller's thread
-        });
-    for (auto& t : pool) t.join();
-    for (int k = 0; k < n_devices; ++k)
-        if (rcs[k] != CLB_OK) return fail(rcs[k], "device " + std::to_string(devices[k]) + ": " + errs[k]);
-    return CLB_OK;
+    return clb::deal_to_devices(n_devices, devices, n_windows, cells.data(), part_out, [&](int k, const std::vector<int32_t>& sel) {
+        clb_batch* b = nullptr;
+        int r = create_internal(devices[k], n_windows, g1, g2, params, sel.data(), (int32_t)sel.size(), &b);
+        if (r == CLB_OK) r = clb_batch_upload(b);
+        if (r == CLB_OK) r = clb_batch_run(b);
+        if (r == CLB_OK) r = clb_batch_download(b, score_out, aln_off, aln_pairs, aln_len);
+        clb_batch_destroy(b);
+        return r;
+    });
 }
 
 // Host-only diagnostic: the matrix index (1-based topological rank) flatten_side gives every node of one graph.

@@ -1,5 +1,6 @@
-// pwfa_host.cu -- host side of clb_pwfa_batch (include/centrolign_b200.h): the wavefront variant of the
-// gap fill, pwfa_po_poa (reference: include/centrolign/alignment.hpp:2299-2338).
+// pwfa_host.cu -- host side of clb_pwfa_batch and clb_pwfa_batch_multi (include/centrolign_b200.h): the wavefront
+// variant of the gap fill, pwfa_po_poa (reference: include/centrolign/alignment.hpp:2299-2338).  Both run the same code
+// on a selection of the caller's windows: clb_pwfa_batch selects all of them, the _multi call one share per device.
 //
 // Per window and side the host computes what the reference computes before its search loop --
 // minmax_distance from the sources (minmax_distance.hpp:15-73), target_reachability of the sinks
@@ -124,26 +125,11 @@ int flatten_side(const clb_succ_graph_batch& g, int64_t w, int4* info, uint32_t*
     return CLB_OK;
 }
 
-}  // namespace
-
-extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_graph_batch* g1, const clb_succ_graph_batch* g2,
-                              const clb_params* params, int64_t prune_limit, int64_t* score_out, const int64_t* aln_off,
-                              int32_t* aln_pairs, uint32_t* aln_len, clb_pwfa_stats* stats) {
-    if (stats) memset(stats, 0, sizeof(*stats));
-    if (n_windows < 0 || !params || params->num_pw < 1 || params->num_pw > CLB_MAX_PW)
-        return fail(CLB_EINVAL, "bad window count or NumPW outside 1..3");
-    if (prune_limit < 0) return fail(CLB_EINVAL, "prune_limit must be >= 0");
-    if (n_windows > 0 && (clb::check_graph_batch(g1, n_windows) || clb::check_graph_batch(g2, n_windows)))
-        return fail(CLB_EINVAL, "null graph arrays");
-    if (n_windows > 0 && (!score_out || !aln_off || !aln_pairs || !aln_len)) return fail(CLB_EINVAL, "null output arrays");
-    if (const int rc = clb::require_device(device)) return rc;
-    clb::count_call<kPwfaCalls>(n_windows);
-    if (n_windows == 0) return CLB_OK;
-    const int64_t nw = n_windows;
+// to_wfa_params (alignment.hpp:1630-1651): the penalties divided by their gcd and grouped into classes of equal value
+// (a zero gap_open makes the reference divide by zero in its gcd)
+int wfa_params(const clb_params* params, int64_t prune_limit, clb::PwfaParams& prm) {
     const int P = params->num_pw;
-
-    // to_wfa_params (alignment.hpp:1630-1651); a zero gap_open makes the reference divide by zero in its gcd
-    clb::PwfaParams prm{};
+    prm = clb::PwfaParams{};
     uint32_t w_mismatch = 2 * (params->match + params->mismatch), w_open[3] = {0, 0, 0}, w_ext[3] = {0, 0, 0};
     uint32_t factor = w_mismatch;
     for (int k = 0; k < P; ++k) {
@@ -181,13 +167,25 @@ extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_grap
         prm.factor = factor;
         prm.prune_limit = (int)std::min<int64_t>(prune_limit, int64_t(1) << 30);
     }
+    return CLB_OK;
+}
+
+// Windows sel[0..n_sel) of the batch on `device`, in one search launch plus the re-runs of windows whose tables had to be
+// enlarged.  Window w = sel[i] is flattened, checked and reported under its own index w, and its results land where
+// clb_pwfa_batch puts them; the device arrays hold the selected windows only.
+int run_windows(int device, const clb_succ_graph_batch* g1, const clb_succ_graph_batch* g2, const clb::PwfaParams& prm,
+                const int32_t* sel, int64_t n_sel, int64_t* score_out, const int64_t* aln_off, int32_t* aln_pairs,
+                uint32_t* aln_len, clb_pwfa_stats* stats) {
+    if (stats) memset(stats, 0, sizeof(*stats));
+    const int64_t nw = n_sel;
     const uint64_t max_pen = prm.pen[0];
 
     // layout
     std::vector<clb::PwfaWindow> win(nw);
     int64_t tot_info[2] = {0, 0}, tot_next[2] = {0, 0}, tot_pairs = 0;
     std::vector<int64_t> out_off(nw + 1, 0);
-    for (int64_t w = 0; w < nw; ++w) {
+    for (int64_t i = 0; i < nw; ++i) {
+        const int64_t w = sel[i];
         const int64_t n1 = g1->node_off[w + 1] - g1->node_off[w], n2 = g2->node_off[w + 1] - g2->node_off[w];
         if (n1 < 0 || n2 < 0 || n1 >= (int64_t(1) << 30) || n2 >= (int64_t(1) << 28))
             return fail(CLB_EINVAL, "window size out of range");
@@ -196,7 +194,7 @@ extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_grap
             return fail(CLB_EINVAL, "window " + std::to_string(w) + ": WFA score range exceeds 29 bits");
         if (aln_off[w + 1] - aln_off[w] < n1 + n2)
             return fail(CLB_EINVAL, "alignment capacity of window " + std::to_string(w) + " is below n1+n2");
-        clb::PwfaWindow& W = win[w];
+        clb::PwfaWindow& W = win[i];
         W.n1 = (uint32_t)n1;
         W.n2 = (uint32_t)n2;
         W.info1 = tot_info[0];
@@ -204,7 +202,7 @@ extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_grap
         W.next1 = tot_next[0];
         W.next2 = tot_next[1];
         W.out = tot_pairs;
-        out_off[w] = tot_pairs;
+        out_off[i] = tot_pairs;
         tot_info[0] += n1 + 1;
         tot_info[1] += n2 + 1;
         tot_next[0] += (g1->edge_off[w + 1] - g1->edge_off[w]) + (g1->src_off[w + 1] - g1->src_off[w]);
@@ -226,15 +224,15 @@ extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_grap
     {
         std::vector<Scratch> scratch(clb::pool_threads(nw, 8));
         int64_t bad = -1;
-        const int r = clb::for_each_window(nw, 1, 8, [&](unsigned t, int64_t w) {
-            const int r1 = flatten_side(*g1, w, so[0].info.h + win[w].info1, so[0].next.h + win[w].next1,
-                                        so[0].nlab.h + win[w].next1, scratch[t]);
+        const int r = clb::for_each_window(nw, 1, 8, [&](unsigned t, int64_t i) {
+            const int r1 = flatten_side(*g1, sel[i], so[0].info.h + win[i].info1, so[0].next.h + win[i].next1,
+                                        so[0].nlab.h + win[i].next1, scratch[t]);
             if (r1 != CLB_OK) return r1;
-            return flatten_side(*g2, w, so[1].info.h + win[w].info2, so[1].next.h + win[w].next2, so[1].nlab.h + win[w].next2,
+            return flatten_side(*g2, sel[i], so[1].info.h + win[i].info2, so[1].next.h + win[i].next2, so[1].nlab.h + win[i].next2,
                                 scratch[t]);
         }, &bad);
         if (r != CLB_OK)
-            return fail(r, "window " + std::to_string(bad) + (r == CLB_ECYCLE ? ": graph has a cycle" : ": malformed graph arrays"));
+            return fail(r, "window " + std::to_string(sel[bad]) + (r == CLB_ECYCLE ? ": graph has a cycle" : ": malformed graph arrays"));
     }
 
     int rc = CLB_OK;
@@ -322,25 +320,25 @@ extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_grap
             stats->retries = round;
         }
         std::vector<int32_t> again;
-        for (int32_t w : pending) {
-            const int s = s_status.h[w];
+        for (int32_t i : pending) {
+            const int s = s_status.h[i];
             if (s == clb::kPwfaOk) {
                 if (stats) {
-                    stats->states += s_wstats.h[4 * w];
-                    stats->dequeued += s_wstats.h[4 * w + 1];
-                    stats->steps += s_wstats.h[4 * w + 3];
+                    stats->states += s_wstats.h[4 * i];
+                    stats->dequeued += s_wstats.h[4 * i + 1];
+                    stats->steps += s_wstats.h[4 * i + 3];
                 }
             } else if (s == clb::kPwfaHashFull || s == clb::kPwfaFifoFull) {
                 // the two grow together (queue entries per settled state are bounded by the out-degrees)
-                win[w].hash_log2 += 2;
-                win[w].fifo_log2 += 2;
-                again.push_back(w);
+                win[i].hash_log2 += 2;
+                win[i].fifo_log2 += 2;
+                again.push_back(i);
             } else if (s == clb::kPwfaQueueDry) {
                 // the reference dereferences an empty deque here (alignment.hpp:1738): its precondition is violated
-                rc = fail(CLB_EINVAL, "window " + std::to_string(w) + ": no source reaches a sink within the pruning rule");
+                rc = fail(CLB_EINVAL, "window " + std::to_string(sel[i]) + ": no source reaches a sink within the pruning rule");
                 goto cleanup;
             } else {
-                rc = fail(CLB_ECUDA, "window " + std::to_string(w) + ": internal pwfa kernel error " + std::to_string(s));
+                rc = fail(CLB_ECUDA, "window " + std::to_string(sel[i]) + ": internal pwfa kernel error " + std::to_string(s));
                 goto cleanup;
             }
         }
@@ -350,12 +348,13 @@ extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_grap
     CUDA_TRY_CLEANUP(cudaMemcpyAsync(s_len.h, s_len.d, nw * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
     CUDA_TRY_CLEANUP(cudaMemcpyAsync(s_aln.h, s_aln.d, 2 * tot_pairs * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
     CUDA_TRY_CLEANUP(cudaStreamSynchronize(stream));
-    for (int64_t w = 0; w < nw; ++w) {
-        const uint32_t len = s_len.h[w];
-        const int64_t cap = out_off[w + 1] - out_off[w];
-        memcpy(aln_pairs + 2 * aln_off[w], s_aln.h + 2 * (out_off[w] + cap - len), 2 * (size_t)len * sizeof(int32_t));
+    for (int64_t i = 0; i < nw; ++i) {
+        const int32_t w = sel[i];
+        const uint32_t len = s_len.h[i];
+        const int64_t cap = out_off[i + 1] - out_off[i];
+        memcpy(aln_pairs + 2 * aln_off[w], s_aln.h + 2 * (out_off[i] + cap - len), 2 * (size_t)len * sizeof(int32_t));
         aln_len[w] = len;
-        score_out[w] = s_score.h[w];
+        score_out[w] = s_score.h[i];
     }
     if (stats) {
         stats->h2d_bytes = h2d;
@@ -367,5 +366,72 @@ cleanup:
     if (ev0) cudaEventDestroy(ev0);
     if (ev1) cudaEventDestroy(ev1);
     if (stream) cudaStreamDestroy(stream);
+    return rc;
+}
+
+// The argument checks of both entry points, in the order of clb_pwfa_batch.
+int check_pwfa_args(int32_t n_windows, const clb_succ_graph_batch* g1, const clb_succ_graph_batch* g2, const clb_params* params,
+                    int64_t prune_limit, int64_t* score_out, const int64_t* aln_off, int32_t* aln_pairs, uint32_t* aln_len) {
+    if (n_windows < 0 || !params || params->num_pw < 1 || params->num_pw > CLB_MAX_PW)
+        return fail(CLB_EINVAL, "bad window count or NumPW outside 1..3");
+    if (prune_limit < 0) return fail(CLB_EINVAL, "prune_limit must be >= 0");
+    if (n_windows > 0 && (clb::check_graph_batch(g1, n_windows) || clb::check_graph_batch(g2, n_windows)))
+        return fail(CLB_EINVAL, "null graph arrays");
+    if (n_windows > 0 && (!score_out || !aln_off || !aln_pairs || !aln_len)) return fail(CLB_EINVAL, "null output arrays");
+    return CLB_OK;
+}
+
+}  // namespace
+
+extern "C" int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_graph_batch* g1, const clb_succ_graph_batch* g2,
+                              const clb_params* params, int64_t prune_limit, int64_t* score_out, const int64_t* aln_off,
+                              int32_t* aln_pairs, uint32_t* aln_len, clb_pwfa_stats* stats) {
+    if (stats) memset(stats, 0, sizeof(*stats));
+    if (const int rc = check_pwfa_args(n_windows, g1, g2, params, prune_limit, score_out, aln_off, aln_pairs, aln_len)) return rc;
+    if (const int rc = clb::require_device(device)) return rc;
+    clb::count_call<kPwfaCalls>(n_windows);
+    if (n_windows == 0) return CLB_OK;
+    clb::PwfaParams prm;
+    if (const int rc = wfa_params(params, prune_limit, prm)) return rc;
+    std::vector<int32_t> all(n_windows);
+    std::iota(all.begin(), all.end(), 0);
+    return run_windows(device, g1, g2, prm, all.data(), n_windows, score_out, aln_off, aln_pairs, aln_len, stats);
+}
+
+// The windows dealt to the devices by (n1+1)+(n2+1): the search settles about (n1+n2)*band states (DESIGN.md section 9),
+// so a window's work grows with its side lengths, not with its cell count.
+extern "C" int clb_pwfa_batch_multi(int n_devices, const int* devices, int32_t n_windows, const clb_succ_graph_batch* g1,
+                                    const clb_succ_graph_batch* g2, const clb_params* params, int64_t prune_limit, int64_t* score_out,
+                                    const int64_t* aln_off, int32_t* aln_pairs, uint32_t* aln_len, int32_t* part_out,
+                                    clb_pwfa_stats* stats) {
+    if (stats) memset(stats, 0, sizeof(*stats));
+    if (const int rc = clb::check_devices(n_devices, devices, "clb_pwfa_batch_multi")) return rc;
+    if (const int rc = check_pwfa_args(n_windows, g1, g2, params, prune_limit, score_out, aln_off, aln_pairs, aln_len)) return rc;
+    for (int k = 0; k < n_devices; ++k)
+        if (const int rc = clb::require_device(devices[k])) return rc;
+    clb::count_call<kPwfaCalls>(n_windows);
+    if (n_windows == 0) return CLB_OK;
+    clb::PwfaParams prm;
+    if (const int rc = wfa_params(params, prune_limit, prm)) return rc;
+    std::vector<int64_t> cost(n_windows);
+    for (int32_t w = 0; w < n_windows; ++w)
+        cost[w] = (g1->node_off[w + 1] - g1->node_off[w] + 1) + (g2->node_off[w + 1] - g2->node_off[w] + 1);
+    std::vector<clb_pwfa_stats> dev_stats(n_devices);
+    const int rc = clb::deal_to_devices(n_devices, devices, n_windows, cost.data(), part_out, [&](int k, const std::vector<int32_t>& sel) {
+        return run_windows(devices[k], g1, g2, prm, sel.data(), (int64_t)sel.size(), score_out, aln_off, aln_pairs, aln_len,
+                           stats ? &dev_stats[k] : nullptr);
+    });
+    if (stats)
+        for (const clb_pwfa_stats& d : dev_stats) {  // the devices run side by side: the longest kernel time, summed counters
+            stats->kernel_ms = std::max(stats->kernel_ms, d.kernel_ms);
+            stats->kernel_launches += d.kernel_launches;
+            stats->retries += d.retries;
+            stats->states += d.states;
+            stats->dequeued += d.dequeued;
+            stats->steps += d.steps;
+            stats->h2d_bytes += d.h2d_bytes;
+            stats->d2h_bytes += d.d2h_bytes;
+            stats->workspace_bytes += d.workspace_bytes;
+        }
     return rc;
 }

@@ -86,7 +86,8 @@ struct ChainProblem {
         return p;
     }
 
-    // Runs the DP + traceback on the GPU; returns the chain as match ranks in forward order.
+    // Runs the DP + traceback on the GPU; returns the chain as match ranks in forward order.  Inside a fill-in pool
+    // (batched_parallel_for) the problem runs on the device of the calling worker's batcher, not on `device`.
     std::vector<int64_t> solve(int device = 0, float* opt_score = nullptr, clb_chain_stats* stats = nullptr,
                                std::vector<float>* dp_out = nullptr, std::vector<int64_t>* backptr_out = nullptr) const {
         const clb_chain_problem p = view();
@@ -97,7 +98,7 @@ struct ChainProblem {
         if (ChainBatcher* batcher = stats ? nullptr : ChainBatcher::current()) {
             // a worker of a fill-in pool: lay the problem out here, share the launch with the other workers (chain_batcher.hpp)
             clb_chain_job* job = nullptr;
-            const int rc = clb_chain_job_create(device, &p, dp_out ? dp_out->data() : nullptr, backptr_out ? backptr_out->data() : nullptr,
+            const int rc = clb_chain_job_create(batcher->device(), &p, dp_out ? dp_out->data() : nullptr, backptr_out ? backptr_out->data() : nullptr,
                                                 chain.data(), &len, opt_score, &job);
             if (rc != CLB_OK) throw std::runtime_error(std::string("centrolign_b200: ") + clb_last_error());
             if (job) {

@@ -8,32 +8,29 @@
 // most of its time blocked).  A worker that reaches the DP lays its problem out itself (clb_chain_job_create) and blocks in
 // ChainBatcher::solve; when every worker of the pool is blocked (or enough jobs are waiting) one of them takes all waiting
 // jobs to the device in one clb_chain_jobs_run -- a CTA per problem -- and wakes the others.  Results do not depend on
-// which jobs share a launch, so the output is the one the serial loop produces.
+// which jobs share a launch, so the output is the one the serial loop produces.  Given several devices, the pool keeps
+// one batcher per device and binds every worker to one of them: the subproblems are independent, so they spread over the
+// GPUs like the windows of a stitch.
 #ifndef CENTROLIGN_B200_CHAIN_BATCHER_HPP
 #define CENTROLIGN_B200_CHAIN_BATCHER_HPP
 
+#include <algorithm>
 #include <atomic>
 #include <condition_variable>
 #include <cstdlib>
 #include <exception>
+#include <memory>
 #include <mutex>
 #include <stdexcept>
 #include <string>
 #include <thread>
+#include <utility>
 #include <vector>
 
 #include "centrolign_b200.h"
+#include "devices.hpp"
 
 namespace centrolign_b200 {
-
-// device of the chaining calls: the first entry of CLB_DEVICES (the list the gap-fill batches are shared over), else 0
-inline int chain_device() {
-    static const int dev = [] {
-        const char* s = getenv("CLB_DEVICES");
-        return (s && *s >= '0' && *s <= '9') ? atoi(s) : 0;
-    }();
-    return dev;
-}
 
 class ChainBatcher {
 public:
@@ -41,6 +38,9 @@ public:
     typedef int (*RunJobs)(int device, int64_t n_jobs, clb_chain_job* const* jobs);
     ChainBatcher(int device, int workers, size_t max_batch, RunJobs run = clb_chain_jobs_run)
         : device_(device), active_(workers), max_batch_(max_batch), run_(run) {}
+
+    // the device every job of this batcher is created for and run on
+    int device() const { return device_; }
 
     // the batcher of the pool the calling thread works for, or nullptr: ChainProblem::solve asks
     static ChainBatcher*& current() {
@@ -106,10 +106,13 @@ private:
     bool flushing_ = false;
 };
 
-// body(i) for every i in [0, n), on a pool of workers whose ChainProblem::solve calls share launches.
+// body(i) for every i in [0, n), on a pool of workers whose ChainProblem::solve calls share launches.  With several
+// devices, worker t works for the batcher of devices[t % D] (D = the number of devices, at most the number of workers):
+// its jobs are created for that device and run there, in launches that carry that device's jobs only.
 // CLB_FILL_IN_THREADS sets the pool size (default 4 per hardware thread, 16..128); 1 = the serial loop, no batching.
 template <class Body>
-void batched_parallel_for(size_t n, int device, Body&& body, ChainBatcher::RunJobs run = clb_chain_jobs_run, int pool_size = 0) {
+void batched_parallel_for(size_t n, const std::vector<int>& devices, Body&& body, ChainBatcher::RunJobs run = clb_chain_jobs_run,
+                          int pool_size = 0) {
     static const int configured = getenv("CLB_FILL_IN_THREADS") ? atoi(getenv("CLB_FILL_IN_THREADS")) : 0;
     const unsigned hw = std::thread::hardware_concurrency();
     size_t threads = pool_size > 0 ? (size_t)pool_size
@@ -119,14 +122,20 @@ void batched_parallel_for(size_t n, int device, Body&& body, ChainBatcher::RunJo
         for (size_t i = 0; i < n; ++i) body(i);
         return;
     }
-    ChainBatcher batcher(device, (int)threads, 4 * 148, run);
+    const size_t n_dev = std::max<size_t>(1, std::min(devices.size(), threads));
+    std::vector<std::unique_ptr<ChainBatcher>> batchers;
+    for (size_t d = 0; d < n_dev; ++d) {
+        const size_t workers = threads / n_dev + (d < threads % n_dev ? 1 : 0);  // the t < threads with t % n_dev == d
+        batchers.emplace_back(new ChainBatcher(devices.empty() ? 0 : devices[d], (int)workers, 4 * 148, run));
+    }
     std::atomic<size_t> next(0);
     std::mutex err_mu;
     std::exception_ptr first_error;
     std::vector<std::thread> pool;
     pool.reserve(threads);
     for (size_t t = 0; t < threads; ++t)
-        pool.emplace_back([&] {
+        pool.emplace_back([&, t] {
+            ChainBatcher& batcher = *batchers[t % n_dev];
             ChainBatcher::current() = &batcher;
             try {
                 for (size_t i = next.fetch_add(1); i < n; i = next.fetch_add(1)) body(i);
@@ -140,6 +149,12 @@ void batched_parallel_for(size_t n, int device, Body&& body, ChainBatcher::RunJo
         });
     for (std::thread& th : pool) th.join();
     if (first_error) std::rethrow_exception(first_error);
+}
+
+// The pool on one device.
+template <class Body>
+void batched_parallel_for(size_t n, int device, Body&& body, ChainBatcher::RunJobs run = clb_chain_jobs_run, int pool_size = 0) {
+    batched_parallel_for(n, std::vector<int>(1, device), std::forward<Body>(body), run, pool_size);
 }
 
 }  // namespace centrolign_b200

@@ -30,6 +30,7 @@
 #include <vector>
 
 #include "centrolign_b200.h"
+#include "devices.hpp"
 
 namespace centrolign_b200 {
 
@@ -151,21 +152,6 @@ private:
     std::vector<uint32_t> pred_off_[2], pred_[2], src_[2], snk_[2];
 };
 
-// Device list of the process: CLB_DEVICES="0,1,..." (ordinals), else device 0.  The Stitcher recorder uses it, so a
-// reference binary built with the shadow headers spreads every stitch over the listed GPUs without a source change.
-inline std::vector<int> default_devices() {
-    std::vector<int> out;
-    if (const char* e = std::getenv("CLB_DEVICES")) {
-        int cur = -1;
-        for (const char* c = e;; ++c) {
-            if (*c >= '0' && *c <= '9') cur = (cur < 0 ? 0 : cur * 10) + (*c - '0');
-            else { if (cur >= 0) out.push_back(cur); cur = -1; if (!*c) break; }
-        }
-    }
-    if (out.empty()) out.push_back(0);
-    return out;
-}
-
 // Drop-in for the reference's po_poa: same arguments, same result.
 template <int NumPW, class Graph, class Params, class AlignmentT = Alignment>
 AlignmentT po_poa(const Graph& graph1, const Graph& graph2, const std::vector<uint64_t>& sources1,
@@ -192,13 +178,13 @@ AlignmentT po_poa(const Graph& graph1, const Graph& graph2, const std::vector<ui
 // order of the source lists decide ties, alignment.hpp:1788-1826) and calls clb_pwfa_batch.
 class PwfaBatch {
 public:
-    explicit PwfaBatch(int device = 0) : device_(device) {
-        for (int s = 0; s < 2; ++s) {
-            node_off_[s].push_back(0); edge_off_[s].push_back(0); src_off_[s].push_back(0); snk_off_[s].push_back(0);
-        }
-    }
+    explicit PwfaBatch(int device = 0) : devices_(1, device) { init(); }
+    // Several GPUs of one box: the windows are dealt to the devices by (n1+1)+(n2+1) (clb_pwfa_batch_multi) and the
+    // results come back in window order.
+    explicit PwfaBatch(const std::vector<int>& devices) : devices_(devices.empty() ? std::vector<int>(1, 0) : devices) { init(); }
 
     size_t size() const { return node_off_[0].size() - 1; }
+    const std::vector<int>& devices() const { return devices_; }
 
     template <class Graph>
     void add(const Graph& graph1, const Graph& graph2, const std::vector<uint64_t>& sources1,
@@ -232,8 +218,11 @@ public:
             aln_off[w + 1] = aln_off[w] + (node_off_[0][w + 1] - node_off_[0][w]) + (node_off_[1][w + 1] - node_off_[1][w]);
         std::vector<int32_t> pairs(2 * (size_t)aln_off[nw] + 2);
         std::vector<uint32_t> len(nw, 0);
-        const int rc = clb_pwfa_batch(device_, (int32_t)nw, &g[0], &g[1], &p, prune_limit, score.data(), aln_off.data(),
-                                      pairs.data(), len.data(), nullptr);
+        const int rc = devices_.size() == 1
+                           ? clb_pwfa_batch(devices_[0], (int32_t)nw, &g[0], &g[1], &p, prune_limit, score.data(), aln_off.data(),
+                                            pairs.data(), len.data(), nullptr)
+                           : clb_pwfa_batch_multi((int)devices_.size(), devices_.data(), (int32_t)nw, &g[0], &g[1], &p, prune_limit,
+                                                  score.data(), aln_off.data(), pairs.data(), len.data(), nullptr, nullptr);
         if (rc != CLB_OK) throw std::runtime_error(std::string("centrolign_b200: ") + clb_last_error());
         alignments.assign(nw, AlignmentT());
         for (size_t w = 0; w < nw; ++w) {
@@ -250,6 +239,11 @@ public:
     }
 
 private:
+    void init() {
+        for (int s = 0; s < 2; ++s) {
+            node_off_[s].push_back(0); edge_off_[s].push_back(0); src_off_[s].push_back(0); snk_off_[s].push_back(0);
+        }
+    }
     template <class Graph>
     void add_side(int s, const Graph& graph, const std::vector<uint64_t>& sources, const std::vector<uint64_t>& sinks) {
         const uint64_t n = graph.node_size();
@@ -271,7 +265,7 @@ private:
         snk_off_[s].push_back(snk_off_[s].back() + (int64_t)sinks.size());
     }
 
-    int device_;
+    std::vector<int> devices_;
     std::vector<int64_t> node_off_[2], edge_off_[2], src_off_[2], snk_off_[2];
     std::vector<uint8_t> label_[2];
     std::vector<uint32_t> next_off_[2], next_[2], src_[2], snk_[2];

@@ -8,7 +8,8 @@
 // the window's back-translation tables.  When the loop is done, all recorded windows go to the GPU in
 // one clb_popoa_batch per NumPW, and every marker is replaced, in order, by the translated alignment of
 // its window.  The wavefront route (pwfa_po_poa, stitcher.hpp:336-339) is recorded the same way and goes
-// out as one clb_pwfa_batch per NumPW.  Routing, gap-piece truncation, anchor copies and every other
+// out as one clb_pwfa_batch per NumPW.  Both routes use the GPUs of CLB_DEVICES (the _multi calls when it lists more
+// than one).  Routing, gap-piece truncation, anchor copies and every other
 // route are the reference's own code, executed as is.
 #ifndef CENTROLIGN_B200_STITCH_RECORDER_HPP
 #define CENTROLIGN_B200_STITCH_RECORDER_HPP
@@ -53,7 +54,7 @@ public:
         active_ = true;
         for (int k = 0; k < CLB_MAX_PW; ++k) {
             batch_[k] = PoPoaBatch(default_devices());  // CLB_DEVICES: several GPUs of the box share every stitch
-            wbatch_[k] = PwfaBatch();
+            wbatch_[k] = PwfaBatch(default_devices());
             have_params_[k] = false;
         }
         windows_.clear();

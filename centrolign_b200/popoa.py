@@ -22,7 +22,8 @@ _LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "csrc", "li
 EXPORTS = ["clb_popoa_batch", "clb_batch_create", "clb_batch_upload", "clb_batch_run", "clb_batch_download",
            "clb_batch_destroy", "clb_batch_get_stats", "clb_int32_peak_tops", "clb_last_error", "clb_device_count",
            "clb_release_cached_memory", "clb_pwfa_batch", "clb_chain_dp", "clb_topological_ranks", "clb_popoa_batch_multi",
-           "clb_balanced_partition", "clb_chain_dp_batch", "clb_chain_job_create", "clb_chain_jobs_run", "clb_chain_job_destroy", "clb_warm_up"]
+           "clb_balanced_partition", "clb_chain_dp_batch", "clb_chain_job_create", "clb_chain_jobs_run", "clb_chain_job_destroy", "clb_warm_up",
+           "clb_pwfa_batch_multi", "clb_chain_dp_batch_multi"]
 ERROR_NAMES = {0: "CLB_OK", 1: "CLB_EINVAL", 2: "CLB_ECYCLE", 3: "CLB_ECUDA", 4: "CLB_ENOMEM", 5: "CLB_ESTATE"}
 
 
@@ -96,6 +97,9 @@ def load_library() -> ctypes.CDLL:
     lib.clb_release_cached_memory.restype = None
     lib.clb_pwfa_batch.restype = ctypes.c_int
     lib.clb_pwfa_batch.argtypes = [ctypes.c_int, i32, gp, gp, pp, ctypes.c_int64, vp, vp, vp, vp, ctypes.POINTER(PwfaStats)]
+    lib.clb_pwfa_batch_multi.restype = ctypes.c_int
+    lib.clb_pwfa_batch_multi.argtypes = [ctypes.c_int, vp, i32, gp, gp, pp, ctypes.c_int64, vp, vp, vp, vp, vp,
+                                         ctypes.POINTER(PwfaStats)]
     _lib = lib
     return lib
 
@@ -266,6 +270,32 @@ def pwfa_po_poa_batch(succ_batch: WindowBatch, params: AlignmentParameters, prun
                               ctypes.byref(stats) if stats is not None else None))
     del k1, k2
     return score, [pairs[int(aln_off[w]): int(aln_off[w]) + int(aln_len[w])] for w in range(nw)]
+
+
+def pwfa_po_poa_batch_multi(succ_batch: WindowBatch, params: AlignmentParameters, prune_limit: int, devices,
+                            return_parts: bool = False, stats: Optional[PwfaStats] = None):
+    """``clb_pwfa_batch_multi``: the windows of ``pwfa_po_poa_batch`` dealt to several GPUs of one box by
+    (n1+1)+(n2+1) (one host thread per device inside the library), results in window order.  ``devices`` is a list of
+    distinct device ordinals.  Returns (scores, [alignment per window]), plus the index into ``devices`` each window ran
+    on if ``return_parts``.  ``stats``: the longest kernel time over the devices, the counters summed."""
+    lib = load_library()
+    p = _c_params(params)
+    g1, k1 = _c_side(succ_batch.g1)
+    g2, k2 = _c_side(succ_batch.g2)
+    nw = succ_batch.n_windows
+    aln_off = np.zeros(nw + 1, np.int64)
+    np.cumsum(succ_batch.aln_capacity(), out=aln_off[1:])
+    score = np.zeros(nw, np.int64)
+    aln_len = np.zeros(nw, np.uint32)
+    pairs = np.empty((max(1, int(aln_off[-1])), 2), np.int32)
+    devs = np.ascontiguousarray(list(devices), np.int32)
+    parts = np.zeros(max(1, nw), np.int32)
+    _check(lib.clb_pwfa_batch_multi(len(devs), devs.ctypes.data, nw, ctypes.byref(g1), ctypes.byref(g2), ctypes.byref(p),
+                                    int(prune_limit), score.ctypes.data, aln_off.ctypes.data, pairs.ctypes.data,
+                                    aln_len.ctypes.data, parts.ctypes.data, ctypes.byref(stats) if stats is not None else None))
+    del k1, k2
+    alns = [pairs[int(aln_off[w]): int(aln_off[w]) + int(aln_len[w])] for w in range(nw)]
+    return (score, alns, parts[:nw]) if return_parts else (score, alns)
 
 
 def topological_ranks(pred_lists) -> "np.ndarray":

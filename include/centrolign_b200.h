@@ -172,6 +172,22 @@ int clb_pwfa_batch(int device, int32_t n_windows, const clb_succ_graph_batch* g1
                    int32_t* aln_pairs, uint32_t* aln_len, clb_pwfa_stats* stats /* may be NULL */);
 
 /*
+ * The same call over several GPUs of one box, in the manner of clb_popoa_batch_multi: the windows are dealt to the
+ * devices longest-first (clb_balanced_partition) by (n1+1)+(n2+1) -- the search settles about (n1+n2)*band states, so
+ * a window's work follows its side lengths, not its cell count -- and one host thread per device runs the single-device
+ * path on its share.  Every window's result lands in the caller's arrays at the same place as with clb_pwfa_batch, and
+ * error messages name the caller's window index behind "device <ordinal>: ".  Windows whose tables must be enlarged are
+ * re-run on their own device.  devices[] lists distinct ordinals (a repeat, or one out of range, is CLB_EINVAL).
+ * part_out (may be NULL) receives, per window, the index into devices[] the window ran on.  stats (may be NULL): kernel_ms
+ * is the largest over the devices (they run side by side); kernel_launches, retries, states, dequeued, steps, h2d_bytes,
+ * d2h_bytes and workspace_bytes are sums over the devices.
+ */
+int clb_pwfa_batch_multi(int n_devices, const int* devices, int32_t n_windows, const clb_succ_graph_batch* g1,
+                         const clb_succ_graph_batch* g2, const clb_params* params, int64_t prune_limit, int64_t* score_out,
+                         const int64_t* aln_off, int32_t* aln_pairs, uint32_t* aln_len, int32_t* part_out /* may be NULL */,
+                         clb_pwfa_stats* stats /* may be NULL */);
+
+/*
  * Sparse anchor-chaining DP.  Replaces the main loops of
  *
  *     Anchorer::sparse_affine_chain_dp<...>   reference: include/centrolign/anchorer.hpp:1812-2471 (loop :2290-2417)
@@ -238,6 +254,9 @@ typedef struct clb_chain_stats {
 } clb_chain_stats;
 
 /*
+ * The chaining entry points below work on any device ordinal, and calls on different devices run side by side (each
+ * device keeps its own buffers and lock); calls on one device are serialised where they use its buffers.
+ *
  * Runs the DP on `device` and the reference's traceback.
  *   dp_out      [n_match] final DP values (may be NULL)
  *   backptr_out [n_match] back-pointer match rank, -1 = none (may be NULL)
@@ -260,6 +279,19 @@ int clb_chain_dp(int device, const clb_chain_problem* problem, float* dp_out, in
 int clb_chain_dp_batch(int device, int64_t n_problems, const clb_chain_problem* const* problems, float* const* dp_out,
                        int64_t* const* backptr_out, int64_t* const* chain_out, int64_t* chain_len, float* opt_score,
                        clb_chain_stats* stats /* may be NULL */);
+
+/*
+ * The batched call over several GPUs of one box.  The problems are dealt to the devices longest-first
+ * (clb_balanced_partition) by a work estimate -- the DP costs about a step's latency times the steps, so n_step plus the
+ * insert and query counts (ins_off[n_match] + qry_off[n_step]) -- and one host thread per device runs clb_chain_dp_batch
+ * on its share.  Per problem the outputs are exactly those of clb_chain_dp.  devices[] lists distinct ordinals (a repeat,
+ * or one out of range, is CLB_EINVAL); part_out (may be NULL) receives, per problem, the index into devices[] it ran on.
+ * stats (may be NULL) accumulates over all problems as in clb_chain_dp_batch; total_ms is the wall time of the call.
+ * One problem is never split over devices.
+ */
+int clb_chain_dp_batch_multi(int n_devices, const int* devices, int64_t n_problems, const clb_chain_problem* const* problems,
+                             float* const* dp_out, int64_t* const* backptr_out, int64_t* const* chain_out, int64_t* chain_len,
+                             float* opt_score, int32_t* part_out /* may be NULL */, clb_chain_stats* stats /* may be NULL */);
 
 /*
  * The batched call in two halves, for a caller that prepares problems on several host threads (the drop-in Anchorer runs

@@ -208,7 +208,7 @@ inline void Anchorer::fill_in_anchor_chain<BaseGraph, XM>(                      
     auto gap_matches = divvy_matches(matches, graph1, graph2, gaps, origin);                                                                \
     const auto budgets = assign_reanchor_budget(gaps);                                                                                      \
     std::vector<std::vector<anchor_t>> gap_chains(gaps.size());                                                                             \
-    centrolign_b200::batched_parallel_for(gaps.size(), centrolign_b200::chain_device(), [&](size_t g) {                                     \
+    centrolign_b200::batched_parallel_for(gaps.size(), centrolign_b200::default_devices(), [&](size_t g) {                                  \
         auto& sub1 = gaps[g].first;                                                                                                         \
         auto& sub2 = gaps[g].second;                                                                                                        \
         XM gap_merge1(sub1.subgraph), gap_merge2(sub2.subgraph);                                                                            \
