@@ -221,6 +221,41 @@ def synth_fill_in_problems(n_problems: int, seed: int = 0, matches=(20, 60), num
     return out
 
 
+def synth_chain_problem(n_match: int, n_chain1: int = 1, n_chain2: int = 1, num_pw: int = 1, seed: int = 0, shifts: int = 16,
+                        offsets: int = 64, inactive: float = 0.1, empty_pair: bool = False, n_step: Optional[int] = None):
+    """One random problem with an entry per match on every (chain1, chain2) pair, for tests and benchmarks of the search
+    structures: ``n_match * n_chain1 * n_chain2`` tree entries (one pair fewer per match with ``empty_pair``).  Shifts are
+    drawn from ``shifts`` values and offsets from ``offsets`` values, so small ranges give many equal keys; a fraction
+    ``inactive`` of the entries shape their trees without being entered.  Every match is queried on the step before its
+    start, which precedes its end, on one of ``n_step`` steps (default n_match / 2); the values mean nothing."""
+    rng = np.random.default_rng(seed)
+    M, C1, C2 = n_match, n_chain1, n_chain2
+    n1 = max(16, M // 2 if n_step is None else n_step)  # steps: several matches end on most of them
+    ln = rng.integers(2, 6, M)
+    s1 = rng.integers(1, n1 - 6, M)
+    e1 = s1 + ln - 1
+    ends = np.lexsort((np.arange(M), e1))
+    starts = np.lexsort((np.arange(M), s1))
+    pairs = [(p1, p2) for p1 in range(C1) for p2 in range(C2)]
+    if empty_pair and len(pairs) > 1:
+        pairs = pairs[:-1]
+    npm = len(pairs)
+    E = M * npm
+    a = dict(weight=ln.astype(np.float32), dp_init=(ln - 0.01 * s1).astype(np.float32),
+             final_term=(-0.001 * (n1 - e1)).astype(np.float32),
+             end_off=np.searchsorted(e1[ends], np.arange(n1 + 1), side="left").astype(np.int64), end_match=ends.astype(np.uint32),
+             qry_off=np.searchsorted(s1[starts] - 1, np.arange(n1 + 1), side="left").astype(np.int64),
+             qry_match=starts.astype(np.uint32), qry_chain1=rng.integers(0, C1, M).astype(np.uint32),
+             ins_off=(np.arange(M + 1, dtype=np.int64) * npm),
+             ins_p1=np.tile(np.array([p for p, _ in pairs], np.uint32), M), ins_p2=np.tile(np.array([q for _, q in pairs], np.uint32), M),
+             ins_shift=rng.integers(-shifts, shifts, E).astype(np.int32), ins_offset=rng.integers(0, offsets, E).astype(np.uint32),
+             ins_active=(rng.random(E) >= inactive).astype(np.uint8),
+             qa1=rng.integers(0, offsets + shifts, M * C1).astype(np.int32), qa2=rng.integers(0, offsets, M * C2).astype(np.int32),
+             qoff=rng.integers(0, offsets + 1, M * C2).astype(np.uint32))
+    k = max(1, num_pw)
+    return ChainProblem(num_pw, (1.0, 2.0, 3.0)[:k], (0.5, 0.2, 0.1)[:k], 1.0, C1, C2, 0.0, a)
+
+
 _DTYPES = {0: np.float32, 1: np.int32, 2: np.uint32, 3: np.int64, 4: np.float64}
 
 

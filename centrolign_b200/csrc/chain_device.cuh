@@ -6,7 +6,8 @@
 //   * 2*NumPW OrthogonalMaxSearchTrees keyed ((shift, match), offset on p2), all with the same keys;
 //     reference: anchorer.hpp:2084-2111, include/centrolign/orthogonal_max_search_tree.hpp
 // Both are static in SHAPE (implicit heap layout, filled in key order, max_search_tree.hpp:108-150) and only
-// their values move.  Here the same shapes are laid out once on the host (chain_host.cu) and the value side
+// their values move.  Here the same shapes are laid out once, by the host (chain_host.cu) or for large problems by the
+// device (chain_layout_kernels.cu), and the value side
 // is held in atomically-max-able words so that all updates of one DP step can run in parallel:
 //   gap-free tree node x : best[x] = max over the subtree of x of pack(value, ~insertion sequence number)
 //                          -- exactly the reference's subtree_max pointer, which moves only on a strictly
@@ -122,6 +123,119 @@ struct ChainArgs {
     uint32_t* out_backptr;
     int sync_mode;     // how the phases of a step are separated: 0 one CTA (__syncthreads), 1 one thread-block cluster
                        // (barrier.cluster), 2 cooperative grid (grid.sync)
+};
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Shapes of the implicit heaps, shared by the host layout (chain_host.cu) and the device layout (chain_layout_kernels.cu).
+// An n-node heap is a complete binary tree: levels full except the last, which is filled from the left.  Every subtree
+// of it is again such a tree.
+
+#ifdef __CUDA_ARCH__
+#define CLB_CLZ(x) __clz(x)
+#else
+#define CLB_CLZ(x) __builtin_clz(x)
+#endif
+
+// depth of heap node h (< 2^32 - 1)
+__host__ __device__ inline int heap_depth(uint32_t h) { return 31 - CLB_CLZ(h + 1); }
+
+// nodes of the left subtree of the root of an m-node heap
+__host__ __device__ inline uint32_t heap_left_size(uint32_t m) {
+    if (m <= 1) return 0;
+    const int hgt = 31 - CLB_CLZ(m);  // the root's height: levels 0..hgt
+    const uint32_t half = 1u << (hgt - 1);
+    const uint32_t last = m - ((1u << hgt) - 1);  // nodes on the last level, 1 .. 2^hgt
+    return half - 1 + (last < half ? last : half);
+}
+
+// the heap index of in-order position k of an n-node heap: the node the reference's in-order fill
+// (max_search_tree.hpp:119-150) gives the k-th smallest key; a descent from the root over the subtree sizes
+__host__ __device__ inline uint32_t heap_of_inorder(uint32_t k, uint32_t n) {
+    uint32_t h = 0, m = n;
+    for (;;) {
+        const uint32_t ls = heap_left_size(m);
+        if (k == ls) return h;
+        if (k < ls) {
+            h = 2 * h + 1;
+            m = ls;
+        } else {
+            k -= ls + 1;
+            h = 2 * h + 2;
+            m -= ls + 1;
+        }
+    }
+}
+
+// the two outer spines of an orthogonal tree carry no inner list (orthogonal_max_search_tree.hpp:175-182)
+__host__ __device__ inline bool heap_on_spine(uint32_t h) {
+    const uint64_t a = (uint64_t)h + 1, b = (uint64_t)h + 2;
+    return (a & (a - 1)) == 0 || (b & (b - 1)) == 0;
+}
+
+// nodes in the subtree of heap node h of an n-node heap (h < n)
+__host__ __device__ inline uint32_t heap_subtree_size(uint32_t h, uint32_t n) {
+    const int d = heap_depth(h), H = heap_depth(n - 1);
+    const uint64_t w = uint64_t(1) << (H - d);               // width of the subtree's last level
+    const uint64_t first = ((uint64_t)h + 1) * w - 1;        // its first heap index there
+    const uint64_t present = n > first ? (n - first < w ? n - first : w) : 0;
+    return (uint32_t)(w - 1 + present);
+}
+
+// non-spine nodes on the path from the root to h, h included: the inner lists h is an element of.  At depth d with
+// level position t, the ancestor at depth j is on the left spine iff t >> (d - j) == 0 and on the right spine iff it is
+// all ones, so the path leaves the spines min(bit length of t, bit length of its complement) levels above h.
+__host__ __device__ inline uint32_t heap_nanc(uint32_t h) {
+    const int d = heap_depth(h);
+    if (d == 0) return 0;
+    const uint32_t t = h + 1 - (1u << d), u = ((1u << d) - 1) ^ t;
+    const uint32_t bt = t ? 32 - CLB_CLZ(t) : 0, bu = u ? 32 - CLB_CLZ(u) : 0;
+    return bt < bu ? bt : bu;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Device layout (chain_layout_kernels.cu): the tables chain_host.cu's host layout builds, built by kernels straight into
+// the copy region of the call's arena.  Phase 1 (chain_layout_sort) uploads the caller's raw entry and step arrays into
+// a scratch buffer, builds the per-entry tables and sorts the entries; its one read-back is the number of gap-free trees,
+// which the arena plan needs.  Phase 2 (chain_layout_build) writes every laid-out table.
+
+struct ChainLayoutDims {
+    int64_t M, S, E, n_end, npair;
+    int C2, P;
+    int max_depth;    // depth of the deepest orthogonal node: floor(log2(largest tree))
+    bool has_active;  // the problem has an ins_active array
+};
+
+// destinations in the arena (device pointers); the orthogonal ones are unused when P == 0
+struct ChainLayoutOut {
+    int64_t* sins_live;
+    InsRec* ins;
+    int64_t* qry_live;
+    int64_t* pair_grp_off;
+    int32_t* grp_shift;
+    uint32_t* grp_base;
+    uint32_t* grp_n;
+    uint32_t* pair_base;
+    uint32_t* gf_key;
+    uint32_t* gf_match;
+    int32_t* or_shift;
+    uint32_t* or_off;
+    uint32_t* or_match;
+    uint32_t* in_base;
+    uint32_t* in_n;
+    uint32_t* in_off;
+    uint32_t* ent_rank;
+};
+
+// the caller's raw arrays the layout reads (host pointers)
+struct ChainLayoutIn {
+    const int64_t* ins_off;
+    const uint32_t *ins_p1, *ins_p2;
+    const int32_t* ins_shift;
+    const uint32_t* ins_offset;
+    const uint8_t* ins_active;  // may be null: every entry active
+    const int64_t* end_off;
+    const uint32_t* end_match;
+    const int64_t* qry_off;
 };
 
 }  // namespace clb

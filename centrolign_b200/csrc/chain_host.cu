@@ -1,6 +1,6 @@
 // chain_host.cu -- host side of clb_chain_dp (include/centrolign_b200.h): lays out the reference's search
-// structures for the device (shapes only -- see chain_device.cuh), runs the DP kernel, and performs the
-// reference's traceback (Anchorer::traceback_sparse_dp, include/centrolign/anchorer.hpp:2473-2547).
+// structures for the device (shapes only -- see chain_device.cuh; large problems are laid out by the device itself,
+// chain_layout_kernels.cu), runs the DP kernel, and performs the reference's traceback (Anchorer::traceback_sparse_dp, include/centrolign/anchorer.hpp:2473-2547).
 //
 // Shapes reproduced here:
 //   * MaxSearchTree: implicit binary heap 0..n-1 filled with the sorted keys by an in-order walk
@@ -22,6 +22,9 @@ namespace clb {
 cudaError_t launch_chain(ChainArgs args, int grid, int* cluster, int prepare_grid, cudaStream_t stream, cudaEvent_t after_prepare);
 cudaError_t launch_chain_small_batch(const ChainArgs* d_args, int n, int smem_bytes, bool any_global, cudaStream_t stream);
 int chain_max_grid(int device);
+cudaError_t chain_layout_scratch_bytes(const ChainLayoutDims& d, size_t* bytes);
+cudaError_t chain_layout_sort(const ChainLayoutIn& in, const ChainLayoutDims& d, char* scratch, cudaStream_t st, int64_t* n_groups, int64_t* h2d_bytes);
+cudaError_t chain_layout_build(const ChainLayoutDims& d, int64_t G, char* scratch, const ChainLayoutOut& o, cudaStream_t st, int64_t* n_inner);
 }  // namespace clb
 
 using clb::fail;
@@ -30,22 +33,30 @@ namespace {
 
 double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
-// heap index of every in-order position of an n-node implicit heap (max_search_tree.hpp:119-150)
-void inorder_layout(uint32_t n, std::vector<uint32_t>& heap_of_pos, std::vector<uint32_t>& stack) {
+// heap index of every in-order position of an n-node implicit heap (max_search_tree.hpp:119-150); the device layout
+// places its entries with the same function
+void inorder_layout(uint32_t n, std::vector<uint32_t>& heap_of_pos) {
     heap_of_pos.resize(n);
-    stack.clear();
-    uint32_t pos = 0;
-    uint64_t cur = 0;
-    while (cur < n || !stack.empty()) {
-        while (cur < n) {
-            stack.push_back((uint32_t)cur);
-            cur = 2 * cur + 1;
-        }
-        const uint32_t x = stack.back();
-        stack.pop_back();
-        heap_of_pos[pos++] = x;
-        cur = 2 * (uint64_t)x + 2;
+    for (uint32_t k = 0; k < n; ++k) heap_of_pos[k] = clb::heap_of_inorder(k, n);
+}
+
+// Σ over x < n of the bit length of x
+int64_t bitlen_prefix(int64_t n) {
+    int64_t s = 0;
+    for (int b = 1; b <= 33 && (int64_t(1) << (b - 1)) < n; ++b) s += n - (int64_t(1) << (b - 1));
+    return s;
+}
+// inner-list slots of an n-node orthogonal tree, Σ heap_nanc over its nodes, level by level in closed form: on level d,
+// position t has heap_nanc = min(bit length of t, bit length of 2^d - 1 - t)
+int64_t inner_slots(int64_t n) {
+    int64_t s = 0;
+    for (int d = 2; n >= 2 && d <= clb::heap_depth((uint32_t)(n - 1)); ++d) {
+        const int64_t full = int64_t(1) << d, half = full / 2;
+        const int64_t c = std::min(full, n - (full - 1));  // nodes on level d
+        s += bitlen_prefix(std::min(c, half));
+        if (c > half) s += bitlen_prefix(half) - bitlen_prefix(full - c);
     }
+    return s;
 }
 
 // All device data of one call lives in one arena: [copied segments][zero-filled segments].  The arena, its pinned
@@ -56,6 +67,8 @@ struct DeviceArena {
     size_t cap = 0;
     char* h = nullptr;  // pinned
     size_t hcap = 0;
+    char* ls = nullptr;  // scratch of the device layout, kept and released with the arena
+    size_t ls_cap = 0;
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, evp = nullptr;
 };
@@ -92,6 +105,31 @@ private:
     std::map<int, Slot> slots_;
 };
 PerDevice<DeviceArena> g_arenas;
+
+cudaError_t ensure_stream(DeviceArena& ar) {  // on the current device
+    if (ar.stream) return cudaSuccess;
+    cudaError_t e = cudaStreamCreateWithFlags(&ar.stream, cudaStreamNonBlocking);
+    if (e == cudaSuccess) e = cudaEventCreate(&ar.ev0);
+    if (e == cudaSuccess) e = cudaEventCreate(&ar.ev1);
+    if (e == cudaSuccess) e = cudaEventCreate(&ar.evp);
+    return e;
+}
+
+// Which side lays out a problem that runs on its own.  Auto: the device from kDeviceLayoutMinEntries tree entries on, if its
+// scratch fits in free device memory.  CLB_CHAIN_LAYOUT=host|device forces a side (A/B runs, tests); check builds both and
+// compares the copy regions byte for byte.  Problems the batched launch takes always keep the host layout.
+enum class LayoutSide { Auto, Host, Device, Check };
+LayoutSide layout_side_knob() {
+    const char* v = getenv("CLB_CHAIN_LAYOUT");
+    if (!v) return LayoutSide::Auto;
+    if (!strcmp(v, "host")) return LayoutSide::Host;
+    if (!strcmp(v, "device")) return LayoutSide::Device;
+    if (!strcmp(v, "check")) return LayoutSide::Check;
+    return LayoutSide::Auto;
+}
+// tools/chain_layout_bench.py on a B200 (profiles/r03_chain_layout.json, DESIGN.md section 10): the device layout is the faster
+// one at every size measured, 10^4 tree entries up; below that a call is dominated by its launches either way
+constexpr int64_t kDeviceLayoutMinEntries = 10000;
 
 // fn(begin, end) over [0, n) on up to 16 host threads (the layout of a million-match problem is tens of millions of
 // small steps; the Anchorer calls us from one thread)
@@ -162,32 +200,78 @@ struct ArenaPlan {
     }
 };
 
-// A laid-out problem: the scalar kernel arguments, and where its arrays sit in the copy region (o_*) and in the zero
+// The arrays of the copy region, in arena order.  The raw ones are the caller's arrays as they are; the others are laid
+// out by the host (chain_host.cu) or by the device (chain_layout_kernels.cu).
+enum CopySeg {
+    kSegDp, kSegBp, kSegSins, kSegIns, kSegQoff, kSegQm, kSegW, kSegQc1, kSegQa1, kSegQa2, kSegQo, kSegPg, kSegGs, kSegGb, kSegGn, kSegPb,
+    kSegGk, kSegGm, kSegOs, kSegOo, kSegOm, kSegIb, kSegIn, kSegIo, kSegEr, kSegs
+};
+constexpr const char* kSegName[kSegs] = {"dp_init", "bp0", "sins_live", "ins", "qry_live", "qry_match", "weight", "qry_chain1", "qa1",
+                                         "qa2", "qoff", "pair_grp_off", "grp_shift", "grp_base", "grp_n", "pair_base", "gf_key", "gf_match",
+                                         "or_shift", "or_off", "or_match", "in_base", "in_n", "in_off", "ent_rank"};
+constexpr size_t kSegElem[kSegs] = {4, 4, 8, sizeof(clb::InsRec), 8, 4, 4, 4, 4, 4, 4, 8, 4, 4, 4, 4, 4, 4, 4, 4, 4, 4, 4, 4, 4};
+bool seg_is_raw(int k) { return k == kSegDp || (k >= kSegQm && k <= kSegQo); }
+
+// The sizes a layout needs, known before any table exists
+struct LayoutCounts {
+    int64_t M = 0, n_qry = 0, S_live = 0, n_ins = 0, npair = 0, G = 0, E = 0, n_inner = 0, max_q = 0;
+    int C1 = 0, C2 = 0, P = 0;
+    uint32_t max_n = 0;  // largest orthogonal tree (largest pair), 0 without entries
+    int64_t pairs_used = 0;  // pairs with entries: the fewest gap-free trees there can be
+    int64_t seg_count(int k) const {
+        const int64_t Eo = P > 0 ? E : 0;
+        switch (k) {
+            case kSegDp: case kSegBp: case kSegW: return M;
+            case kSegSins: case kSegQoff: return S_live + 1;
+            case kSegIns: return n_ins;
+            case kSegQm: case kSegQc1: return n_qry;
+            case kSegQa1: return M * C1;
+            case kSegQa2: case kSegQo: return M * C2;
+            case kSegPg: case kSegPb: return npair + 1;
+            case kSegGs: case kSegGb: case kSegGn: return G;
+            case kSegGk: case kSegGm: return E;
+            case kSegIo: case kSegEr: return n_inner;
+            default: return Eo;  // or_*, in_base, in_n
+        }
+    }
+};
+
+// A laid-out problem: the scalar kernel arguments, and where its arrays sit in the copy region (o) and in the zero
 // region (z_*) of its arena.
 struct ChainLayout {
     clb::ChainArgs scalars{};  // every pointer null: bind() sets them
     size_t copy_bytes = 0, zero_bytes = 0;
     size_t arena_bytes() const { return copy_bytes + zero_bytes; }
-    size_t o_dp, o_bp, o_sins, o_ins, o_qoff, o_qm, o_w, o_qc1, o_qa1, o_qa2, o_qo, o_pg, o_gs, o_gb, o_gn, o_pb, o_gk, o_gm, o_os,
-        o_oo, o_om, o_ib, o_in, o_io, o_er;
+    size_t o[kSegs];
     size_t z_qrec, z_gford, z_gfbest, z_orord, z_bit, z_cbest, z_cbp, z_cnt, z_ranks;
 };
+
+// the copy region (sources: src[k], null where the device builds the array) and the zero region of a problem of size c
+void plan_layout(const LayoutCounts& c, const void* const* src, ChainLayout& L, ArenaPlan& plan) {
+    for (int k = 0; k < kSegs; ++k) L.o[k] = plan.copy(src ? src[k] : nullptr, (size_t)c.seg_count(k) * kSegElem[k]);
+    const int64_t T = 2 * c.P, E = c.E;
+    L.z_qrec = plan.zero((size_t)c.n_qry * c.C2 * sizeof(clb::QueryRec));
+    L.z_gford = plan.zero((size_t)E * 4); L.z_gfbest = plan.zero((size_t)E * 8);
+    L.z_orord = plan.zero((size_t)T * E * 4); L.z_bit = plan.zero((size_t)T * c.n_inner * 8);
+    L.z_cbest = plan.zero((size_t)c.M * 16); L.z_cbp = plan.zero((size_t)(c.max_q * c.C2 * (T + 1)) * 4 * 2); L.z_cnt = plan.zero(8);
+}
 
 // The kernel arguments of a laid-out problem whose copy region is at device address c and zero region at z.  The only
 // code that knows which array lives in which region.  arena_bytes covers both regions, copy_bytes the copy region.
 clb::ChainArgs bind(const ChainLayout& L, char* c, char* z) {
     clb::ChainArgs a = L.scalars;
-    a.dp = (float*)(c + L.o_dp); a.backptr = (uint32_t*)(c + L.o_bp);
-    a.sins_off = (const int64_t*)(c + L.o_sins); a.ins = (const clb::InsRec*)(c + L.o_ins);
-    a.qry_off = (const int64_t*)(c + L.o_qoff); a.qry_match = (const uint32_t*)(c + L.o_qm);
-    a.weight = (const float*)(c + L.o_w); a.qry_chain1 = (const uint32_t*)(c + L.o_qc1);
-    a.qa1 = (const int32_t*)(c + L.o_qa1); a.qa2 = (const int32_t*)(c + L.o_qa2); a.qoff = (const uint32_t*)(c + L.o_qo);
-    a.pair_grp_off = (const int64_t*)(c + L.o_pg); a.grp_shift = (const int32_t*)(c + L.o_gs);
-    a.grp_base = (const uint32_t*)(c + L.o_gb); a.grp_n = (const uint32_t*)(c + L.o_gn); a.pair_base = (const uint32_t*)(c + L.o_pb);
-    a.gf_key = (const uint32_t*)(c + L.o_gk); a.gf_match = (const uint32_t*)(c + L.o_gm);
-    a.or_shift = (const int32_t*)(c + L.o_os); a.or_off = (const uint32_t*)(c + L.o_oo); a.or_match = (const uint32_t*)(c + L.o_om);
-    a.in_base = (const uint32_t*)(c + L.o_ib); a.in_n = (const uint32_t*)(c + L.o_in); a.in_off = (const uint32_t*)(c + L.o_io);
-    a.ent_rank = (const uint32_t*)(c + L.o_er);
+    const size_t* o = L.o;
+    a.dp = (float*)(c + o[kSegDp]); a.backptr = (uint32_t*)(c + o[kSegBp]);
+    a.sins_off = (const int64_t*)(c + o[kSegSins]); a.ins = (const clb::InsRec*)(c + o[kSegIns]);
+    a.qry_off = (const int64_t*)(c + o[kSegQoff]); a.qry_match = (const uint32_t*)(c + o[kSegQm]);
+    a.weight = (const float*)(c + o[kSegW]); a.qry_chain1 = (const uint32_t*)(c + o[kSegQc1]);
+    a.qa1 = (const int32_t*)(c + o[kSegQa1]); a.qa2 = (const int32_t*)(c + o[kSegQa2]); a.qoff = (const uint32_t*)(c + o[kSegQo]);
+    a.pair_grp_off = (const int64_t*)(c + o[kSegPg]); a.grp_shift = (const int32_t*)(c + o[kSegGs]);
+    a.grp_base = (const uint32_t*)(c + o[kSegGb]); a.grp_n = (const uint32_t*)(c + o[kSegGn]); a.pair_base = (const uint32_t*)(c + o[kSegPb]);
+    a.gf_key = (const uint32_t*)(c + o[kSegGk]); a.gf_match = (const uint32_t*)(c + o[kSegGm]);
+    a.or_shift = (const int32_t*)(c + o[kSegOs]); a.or_off = (const uint32_t*)(c + o[kSegOo]); a.or_match = (const uint32_t*)(c + o[kSegOm]);
+    a.in_base = (const uint32_t*)(c + o[kSegIb]); a.in_n = (const uint32_t*)(c + o[kSegIn]); a.in_off = (const uint32_t*)(c + o[kSegIo]);
+    a.ent_rank = (const uint32_t*)(c + o[kSegEr]);
     a.qrec = (clb::QueryRec*)(z + L.z_qrec);
     a.gf_ord = (uint32_t*)(z + L.z_gford); a.gf_best = (unsigned long long*)(z + L.z_gfbest);
     a.or_ord = (uint32_t*)(z + L.z_orord); a.bit = (unsigned long long*)(z + L.z_bit);
@@ -253,6 +337,288 @@ static int chain_traceback(const clb_chain_problem* p, const float* h_dp, const 
     if (backptr_out)
         for (int64_t m = 0; m < M; ++m) backptr_out[m] = h_bp[m] == 0xffffffffu ? -1 : (int64_t)h_bp[m];
     return CLB_OK;
+}
+
+// The host layout: every table of the copy region built on up to 16 host threads.  The batched path and every problem
+// below the device-layout threshold use it; CLB_CHAIN_LAYOUT=check compares the device layout with it.
+struct HostLayout {
+    LayoutCounts c;
+    std::vector<uint32_t> bp0;
+    std::vector<int64_t> sins_live, qry_live, pair_grp_off;
+    std::vector<clb::InsRec> ins;
+    std::vector<int32_t> grp_shift, or_shift;
+    std::vector<uint32_t> grp_base32, grp_n, pair_base32, gf_key, gf_match, or_off, or_match, in_base32, in_n, in_off, ent_rank;
+    const void* src[kSegs] = {};
+};
+
+static int host_layout(const clb_chain_problem* p, HostLayout& H) {
+    const int64_t M = p->n_match, S = p->n_step, E = p->ins_off[M], n_qry = p->qry_off[S];
+    const int C1 = p->n_chain1, C2 = p->n_chain2, P = p->num_pw, T = 2 * P;
+    const int64_t npair = (int64_t)C1 * C2;
+    auto& grp_n = H.grp_n;
+    auto& gf_key = H.gf_key;
+    auto& gf_match = H.gf_match;
+    auto& pair_grp_off = H.pair_grp_off;
+    auto& grp_shift = H.grp_shift;
+    auto& or_shift = H.or_shift;
+    auto& or_off = H.or_off;
+    auto& or_match = H.or_match;
+    auto& in_n = H.in_n;
+    auto& in_off = H.in_off;
+    auto& ent_rank = H.ent_rank;
+    auto& ins = H.ins;
+    std::vector<uint32_t> ent_match(E), ent_pair(E);
+    for (int64_t m = 0; m < M; ++m)
+        for (int64_t e = p->ins_off[m]; e < p->ins_off[m + 1]; ++e) {
+            ent_match[e] = (uint32_t)m;
+            ent_pair[e] = p->ins_p1[e] * (uint32_t)C2 + p->ins_p2[e];
+        }
+    // step -> entries, in the reference's order (anchorer.hpp:2301-2310); positions double as sequence numbers
+    std::vector<int64_t> sins_off(S + 1, 0);
+    std::vector<uint32_t> sins_entry;
+    sins_entry.reserve(E);
+    int64_t max_q = 0;
+    for (int64_t s = 0; s < S; ++s) {
+        for (int64_t k = p->end_off[s]; k < p->end_off[s + 1]; ++k) {
+            const uint32_t m = p->end_match[k];
+            for (int64_t e = p->ins_off[m]; e < p->ins_off[m + 1]; ++e)
+                if (!p->ins_active || p->ins_active[e]) sins_entry.push_back((uint32_t)e);
+        }
+        sins_off[s + 1] = (int64_t)sins_entry.size();
+        max_q = std::max(max_q, p->qry_off[s + 1] - p->qry_off[s]);
+    }
+    if ((int64_t)sins_entry.size() >= (int64_t(1) << 32) - 1) return fail(CLB_EINVAL, "more than 2^32 insertions");
+    if (max_q * C2 * (T + 1) >= (int64_t(1) << 32) - 1) return fail(CLB_EINVAL, "too many queries in one step");
+
+    std::vector<uint32_t> order(E);
+    std::iota(order.begin(), order.end(), 0u);
+    std::vector<uint32_t> heap_of_pos;
+
+    // gap-free trees: one per (pair, shift), keys (offset, match)
+    std::vector<int64_t> grp_base;
+    pair_grp_off.assign(npair + 1, 0);
+    gf_key.resize(E);
+    gf_match.resize(E);
+    std::vector<uint32_t> ent_gf_grp(E), ent_gf_node(E);
+    std::vector<SortKey> keys(E);
+    parallel_for(E, 1 << 16, [&](int64_t a, int64_t b) {  // (pair, shift, offset, match)
+        for (int64_t e = a; e < b; ++e)
+            keys[e] = SortKey{((uint64_t)ent_pair[e] << 32) | ((uint32_t)p->ins_shift[e] ^ 0x80000000u),
+                              ((uint64_t)p->ins_offset[e] << 32) | ent_match[e], (uint32_t)e};
+    });
+    parallel_sort(keys);
+    for (int64_t i = 0; i < E; ++i) order[i] = keys[i].e;
+    for (int64_t i = 0; i < E;) {
+        int64_t j = i;
+        while (j < E && ent_pair[order[j]] == ent_pair[order[i]] && p->ins_shift[order[j]] == p->ins_shift[order[i]]) ++j;
+        const uint32_t g = (uint32_t)grp_base.size(), n = (uint32_t)(j - i);
+        grp_base.push_back(i);
+        grp_shift.push_back(p->ins_shift[order[i]]);
+        grp_n.push_back(n);
+        pair_grp_off[ent_pair[order[i]] + 1] += 1;
+        inorder_layout(n, heap_of_pos);
+        for (uint32_t k = 0; k < n; ++k) {
+            const uint32_t e = order[i + k], h = heap_of_pos[k];
+            gf_key[i + h] = p->ins_offset[e];
+            gf_match[i + h] = ent_match[e];
+            ent_gf_grp[e] = g;
+            ent_gf_node[e] = h;
+        }
+        i = j;
+    }
+    for (int64_t pr = 0; pr < npair; ++pr) pair_grp_off[pr + 1] += pair_grp_off[pr];
+
+    // orthogonal trees: one shape per pair, keys ((shift, match), offset)
+    std::vector<int64_t> pair_base(npair + 1, 0), in_base, ent_rank_off;
+    std::vector<uint32_t> ent_or_node;
+    int64_t n_inner = 0;
+    if (P > 0) {
+        or_shift.resize(E); or_off.resize(E); or_match.resize(E); in_n.assign(E, 0); in_base.assign(E, -1);
+        ent_or_node.resize(E); ent_rank_off.assign(E + 1, 0);
+        parallel_for(E, 1 << 16, [&](int64_t a, int64_t b) {  // (pair, shift, match)
+            for (int64_t e = a; e < b; ++e)
+                keys[e] = SortKey{((uint64_t)ent_pair[e] << 32) | ((uint32_t)p->ins_shift[e] ^ 0x80000000u), (uint64_t)ent_match[e], (uint32_t)e};
+        });
+        parallel_sort(keys);
+        for (int64_t i = 0; i < E; ++i) order[i] = keys[i].e;
+        for (int64_t e = 0; e < E; ++e) pair_base[ent_pair[e] + 1] += 1;
+        for (int64_t pr = 0; pr < npair; ++pr) pair_base[pr + 1] += pair_base[pr];
+        std::vector<uint32_t> pos_of_heap, sub_lo, sub_n, nanc;
+        std::vector<uint8_t> spine;
+        // pass 1: shapes, inner-list sizes and bases
+        for (int64_t pr = 0; pr < npair; ++pr) {
+            const int64_t ob = pair_base[pr];
+            const uint32_t n = (uint32_t)(pair_base[pr + 1] - ob);
+            if (!n) continue;
+            inorder_layout(n, heap_of_pos);
+            for (uint32_t k = 0; k < n; ++k) {
+                const uint32_t e = order[ob + k], h = heap_of_pos[k];
+                or_shift[ob + h] = p->ins_shift[e];
+                or_off[ob + h] = p->ins_offset[e];
+                or_match[ob + h] = ent_match[e];
+                ent_or_node[e] = h;
+            }
+            spine.assign(n, 0);  // orthogonal_max_search_tree.hpp:175-182: the two outer spines carry no cross tree
+            for (uint64_t c = 0; c < n; c = 2 * c + 1) spine[c] = 1;
+            for (uint64_t c = 2; c < n; c = 2 * c + 2) spine[c] = 1;
+            sub_n.assign(n, 1);
+            for (uint32_t h = n; h-- > 1;) sub_n[(h - 1) / 2] += sub_n[h];
+            nanc.assign(n, 0);
+            for (uint32_t h = 0; h < n; ++h) {
+                nanc[h] = (h ? nanc[(h - 1) / 2] : 0) + (spine[h] ? 0 : 1);
+                if (!spine[h]) {
+                    in_base[ob + h] = n_inner;
+                    in_n[ob + h] = sub_n[h];
+                    n_inner += sub_n[h];
+                }
+            }
+            for (uint32_t k = 0; k < n; ++k) ent_rank_off[order[ob + k] + 1] = nanc[heap_of_pos[k]];
+        }
+        for (int64_t e = 0; e < E; ++e) ent_rank_off[e + 1] += ent_rank_off[e];
+        if (ent_rank_off[E] != n_inner) return fail(CLB_ECUDA, "internal: inner list accounting mismatch");
+        in_off.resize(n_inner);
+        ent_rank.resize(n_inner);
+        // pass 2: inner lists by merging children lists, one tree level at a time from the leaves up (the nodes of a
+        // level are independent); a list holds outer key-order positions and is stored where the device will read it
+        std::vector<uint32_t> in_pos(n_inner);
+        for (int64_t pr = 0; pr < npair; ++pr) {
+            const int64_t ob = pair_base[pr];
+            const uint32_t n = (uint32_t)(pair_base[pr + 1] - ob);
+            if (!n) continue;
+            inorder_layout(n, heap_of_pos);
+            pos_of_heap.resize(n);
+            for (uint32_t k = 0; k < n; ++k) pos_of_heap[heap_of_pos[k]] = k;
+            auto depth_of = [](uint32_t h) { return 31 - __builtin_clz(h + 1); };  // heap index -> depth
+            for (int d = depth_of(n - 1); d >= 0; --d) {
+                const int64_t first = (int64_t(1) << d) - 1, last = std::min<int64_t>(n, (int64_t(2) << d) - 1);
+                parallel_for(last - first, std::max<int64_t>(1, 65536 / std::max<int64_t>(1, n >> d)), [&](int64_t a0, int64_t b0) {
+                    for (int64_t hh = first + a0; hh < first + b0; ++hh) {
+                        const uint32_t h = (uint32_t)hh;
+                        if (in_base[ob + h] < 0) continue;  // spine: never queried, never built
+                        const uint32_t l = 2 * h + 1, r = 2 * h + 2;
+                        uint32_t* out = in_pos.data() + in_base[ob + h];
+                        const uint32_t* L = l < n ? in_pos.data() + in_base[ob + l] : nullptr;
+                        const uint32_t* R = r < n ? in_pos.data() + in_base[ob + r] : nullptr;
+                        const uint32_t nl = l < n ? in_n[ob + l] : 0, nr = r < n ? in_n[ob + r] : 0;
+                        const uint32_t self = pos_of_heap[h];
+                        auto off_of = [&](uint32_t pos) { return or_off[ob + heap_of_pos[pos]]; };
+                        // positions of the left subtree < self < positions of the right subtree: ties in offset resolve by side
+                        const uint32_t so = off_of(self);
+                        uint32_t a = 0, b = 0, k = 0;
+                        bool self_done = false;
+                        while (a < nl || b < nr || !self_done) {
+                            // candidates in position order: L[a] < self < R[b]; pick the smallest (offset, position)
+                            int pick = -1;
+                            uint32_t bo = 0;
+                            if (a < nl) { pick = 0; bo = off_of(L[a]); }
+                            if (!self_done && (pick < 0 || so < bo)) { pick = 1; bo = so; }
+                            if (b < nr) {
+                                const uint32_t ro = off_of(R[b]);
+                                if (pick < 0 || ro < bo) pick = 2;
+                            }
+                            out[k++] = pick == 0 ? L[a++] : (pick == 1 ? self : R[b++]);
+                            if (pick == 1) self_done = true;
+                        }
+                        // offsets of the list entries and the rank of every element in this list
+                        const int64_t ib = in_base[ob + h];
+                        for (uint32_t kk = 0; kk < k; ++kk) {
+                            const uint32_t pos = out[kk], eh = heap_of_pos[pos];
+                            in_off[ib + kk] = or_off[ob + eh];
+                            ent_rank[ent_rank_off[order[ob + pos]] + (depth_of(eh) - d)] = kk;  // climbing order: the element's own node first
+                        }
+                    }
+                });
+            }
+        }
+    }
+    // insertion records in the reference's order, and the remaining per-entry tables in 32-bit form
+    if (n_inner >= (int64_t(1) << 32) - 1) return fail(CLB_EINVAL, "search structures exceed 2^32 inner slots");
+    if ((int64_t)sins_entry.size() >= (int64_t(1) << 31)) return fail(CLB_EINVAL, "more than 2^31 insertions");
+    ins.resize(sins_entry.size());
+    for (size_t i = 0; i < sins_entry.size(); ++i) {
+        const uint32_t e = sins_entry[i];
+        clb::InsRec& r = ins[i];
+        r.match = ent_match[e];
+        r.gf_base = (uint32_t)grp_base[ent_gf_grp[e]];
+        r.gf_node = ent_gf_node[e];
+        r.or_base = P > 0 ? (uint32_t)pair_base[ent_pair[e]] : 0;
+        r.or_node = P > 0 ? ent_or_node[e] : 0;
+        r.shift = p->ins_shift[e];
+        r.rank_off = P > 0 ? (uint32_t)ent_rank_off[e] : 0;
+        r.n_rank = P > 0 ? (uint32_t)(ent_rank_off[e + 1] - ent_rank_off[e]) : 0;
+    }
+    H.grp_base32.assign(grp_base.begin(), grp_base.end());
+    H.pair_base32.assign(pair_base.begin(), pair_base.end());
+    H.in_base32.resize(in_base.size());
+    for (size_t k = 0; k < in_base.size(); ++k) H.in_base32[k] = in_base[k] < 0 ? clb::kChainNone : (uint32_t)in_base[k];
+    // the device walks only the steps in which something happens (a caller may list every node of graph 1 as a step; the
+    // builders of hostcpp/chain_b200.hpp list the nodes with events): the offsets are cumulative, so dropping an empty step
+    // drops one equal entry of either list
+    H.sins_live.reserve(S + 1); H.qry_live.reserve(S + 1);
+    H.sins_live.push_back(sins_off[0]); H.qry_live.push_back(p->qry_off[0]);
+    for (int64_t s = 0; s < S; ++s)
+        if (sins_off[s + 1] != sins_off[s] || p->qry_off[s + 1] != p->qry_off[s]) {
+            H.sins_live.push_back(sins_off[s + 1]);
+            H.qry_live.push_back(p->qry_off[s + 1]);
+        }
+    H.bp0.assign(M, clb::kChainNone);
+    LayoutCounts& c = H.c;
+    c.M = M; c.n_qry = n_qry; c.S_live = (int64_t)H.sins_live.size() - 1; c.n_ins = (int64_t)ins.size(); c.npair = npair;
+    c.G = (int64_t)grp_n.size(); c.E = E; c.n_inner = n_inner; c.max_q = max_q; c.C1 = C1; c.C2 = C2; c.P = P;
+    for (int64_t pr = 0; pr < npair; ++pr) c.max_n = std::max<uint32_t>(c.max_n, H.pair_base32[pr + 1] - H.pair_base32[pr]);
+    const void* src[kSegs] = {p->dp_init, H.bp0.data(), H.sins_live.data(), ins.data(), H.qry_live.data(), p->qry_match, p->weight,
+                              p->qry_chain1, p->qa1, p->qa2, p->qoff, pair_grp_off.data(), grp_shift.data(), H.grp_base32.data(),
+                              grp_n.data(), H.pair_base32.data(), gf_key.data(), gf_match.data(), or_shift.data(), or_off.data(),
+                              or_match.data(), H.in_base32.data(), in_n.data(), in_off.data(), ent_rank.data()};
+    std::copy(src, src + kSegs, H.src);
+    (void)T;
+    return CLB_OK;
+}
+
+// The sizes of the device layout from linear passes over the caller's arrays, with the host layout's checks of them in
+// the host layout's order.  No table is built.
+static int count_layout(const clb_chain_problem* p, LayoutCounts& c) {
+    const int64_t M = p->n_match, S = p->n_step, E = p->ins_off[M];
+    const int C1 = p->n_chain1, C2 = p->n_chain2, P = p->num_pw, T = 2 * P;
+    const int64_t npair = (int64_t)C1 * C2;
+    std::vector<uint32_t> act(M);
+    for (int64_t m = 0; m < M; ++m) {
+        uint32_t n = 0;
+        for (int64_t e = p->ins_off[m]; e < p->ins_off[m + 1]; ++e) n += !p->ins_active || p->ins_active[e];
+        act[m] = n;
+    }
+    int64_t n_ins = 0, S_live = 0, max_q = 0;
+    for (int64_t s = 0; s < S; ++s) {
+        int64_t here = 0;
+        for (int64_t k = p->end_off[s]; k < p->end_off[s + 1]; ++k) here += act[p->end_match[k]];
+        n_ins += here;
+        S_live += here > 0 || p->qry_off[s + 1] != p->qry_off[s];
+        max_q = std::max(max_q, p->qry_off[s + 1] - p->qry_off[s]);
+    }
+    if (n_ins >= (int64_t(1) << 32) - 1) return fail(CLB_EINVAL, "more than 2^32 insertions");
+    if (max_q * C2 * (T + 1) >= (int64_t(1) << 32) - 1) return fail(CLB_EINVAL, "too many queries in one step");
+    std::vector<int64_t> hist(npair, 0);
+    for (int64_t e = 0; e < E; ++e) hist[p->ins_p1[e] * (int64_t)C2 + p->ins_p2[e]] += 1;
+    c = LayoutCounts{};
+    for (int64_t pr = 0; pr < npair; ++pr) {
+        c.max_n = std::max<uint32_t>(c.max_n, (uint32_t)hist[pr]);
+        c.pairs_used += hist[pr] > 0;
+        if (P > 0) c.n_inner += inner_slots(hist[pr]);
+    }
+    if (P == 0) c.max_n = 0;  // as the host layout's: no orthogonal trees
+    if (c.n_inner >= (int64_t(1) << 32) - 1) return fail(CLB_EINVAL, "search structures exceed 2^32 inner slots");
+    if (n_ins >= (int64_t(1) << 31)) return fail(CLB_EINVAL, "more than 2^31 insertions");
+    c.M = M; c.n_qry = p->qry_off[S]; c.S_live = S_live; c.n_ins = n_ins; c.npair = npair; c.E = E; c.max_q = max_q;
+    c.C1 = C1; c.C2 = C2; c.P = P;
+    return CLB_OK;
+}
+
+// whether the device layout's scratch and the problem's arena fit in the device's free memory
+static bool device_layout_fits(int device, const LayoutCounts& c, size_t arena_bytes, bool has_active, int64_t n_end, int64_t S) {
+    const clb::ChainLayoutDims dims{c.M, S, c.E, n_end, c.npair, c.C2, c.P, 0, has_active};
+    size_t scratch = 0, free_b = 0, total_b = 0;
+    if (cudaSetDevice(device) != cudaSuccess || clb::chain_layout_scratch_bytes(dims, &scratch) != cudaSuccess) return false;
+    return cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && scratch + arena_bytes < free_b;
 }
 
 static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, int64_t* backptr_out, int64_t* chain_out,
@@ -349,194 +715,41 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
         if (p->ins_p1[e] >= (uint32_t)C1 || p->ins_p2[e] >= (uint32_t)C2) return fail(CLB_EINVAL, "insert path out of range");
 
     // ------------------------------------------------------------------ layout ------------------------------------------------------------------
-    std::vector<uint32_t> ent_match(E), ent_pair(E);
-    for (int64_t m = 0; m < M; ++m)
-        for (int64_t e = p->ins_off[m]; e < p->ins_off[m + 1]; ++e) {
-            ent_match[e] = (uint32_t)m;
-            ent_pair[e] = p->ins_p1[e] * (uint32_t)C2 + p->ins_p2[e];
-        }
-    // step -> entries, in the reference's order (anchorer.hpp:2301-2310); positions double as sequence numbers
-    std::vector<int64_t> sins_off(S + 1, 0);
-    std::vector<uint32_t> sins_entry;
-    sins_entry.reserve(E);
-    int64_t max_q = 0;
-    for (int64_t s = 0; s < S; ++s) {
-        for (int64_t k = p->end_off[s]; k < p->end_off[s + 1]; ++k) {
-            const uint32_t m = p->end_match[k];
-            for (int64_t e = p->ins_off[m]; e < p->ins_off[m + 1]; ++e)
-                if (!p->ins_active || p->ins_active[e]) sins_entry.push_back((uint32_t)e);
-        }
-        sins_off[s + 1] = (int64_t)sins_entry.size();
-        max_q = std::max(max_q, p->qry_off[s + 1] - p->qry_off[s]);
+    // The host layout, or, for a problem that runs on its own and has at least kDeviceLayoutMinEntries tree entries, the
+    // device layout straight into the arena (chain_layout_kernels.cu).  CLB_CHAIN_LAYOUT=host|device|check overrides the choice.
+    const LayoutSide knob = layout_only ? LayoutSide::Host : layout_side_knob();
+    LayoutCounts cnt;
+    bool on_device = false;
+    if (knob != LayoutSide::Host && (knob != LayoutSide::Auto || E >= kDeviceLayoutMinEntries)) {
+        if (const int rc = count_layout(p, cnt)) return rc;
+        // a problem the batched launch takes keeps the host layout: its copy region is staged with the others'
+        ChainLayout L0{};
+        ArenaPlan plan0;
+        LayoutCounts lower = cnt;  // the arena with the fewest gap-free trees the problem can have
+        lower.G = cnt.pairs_used;
+        plan_layout(lower, nullptr, L0, plan0);
+        const size_t lower_total = plan0.copy_bytes + plan0.zero_bytes;
+        on_device = !(ctx && !getenv("CLB_CHAIN_NO_SMALL")) || lower_total > kChainBatchArena;
+        if (on_device && knob == LayoutSide::Auto) on_device = device_layout_fits(device, cnt, lower_total, p->ins_active != nullptr, p->end_off[S], S);
     }
-    if ((int64_t)sins_entry.size() >= (int64_t(1) << 32) - 1) return fail(CLB_EINVAL, "more than 2^32 insertions");
-    if (max_q * C2 * (T + 1) >= (int64_t(1) << 32) - 1) return fail(CLB_EINVAL, "too many queries in one step");
-
-    std::vector<uint32_t> order(E);
-    std::iota(order.begin(), order.end(), 0u);
-    std::vector<uint32_t> heap_of_pos, stack;
-
-    // gap-free trees: one per (pair, shift), keys (offset, match)
-    std::vector<int64_t> pair_grp_off(npair + 1, 0), grp_base;
-    std::vector<int32_t> grp_shift;
-    std::vector<uint32_t> grp_n, gf_key(E), gf_match(E), ent_gf_grp(E), ent_gf_node(E);
-    std::vector<SortKey> keys(E);
-    parallel_for(E, 1 << 16, [&](int64_t a, int64_t b) {  // (pair, shift, offset, match)
-        for (int64_t e = a; e < b; ++e)
-            keys[e] = SortKey{((uint64_t)ent_pair[e] << 32) | ((uint32_t)p->ins_shift[e] ^ 0x80000000u),
-                              ((uint64_t)p->ins_offset[e] << 32) | ent_match[e], (uint32_t)e};
-    });
-    parallel_sort(keys);
-    for (int64_t i = 0; i < E; ++i) order[i] = keys[i].e;
-    for (int64_t i = 0; i < E;) {
-        int64_t j = i;
-        while (j < E && ent_pair[order[j]] == ent_pair[order[i]] && p->ins_shift[order[j]] == p->ins_shift[order[i]]) ++j;
-        const uint32_t g = (uint32_t)grp_base.size(), n = (uint32_t)(j - i);
-        grp_base.push_back(i);
-        grp_shift.push_back(p->ins_shift[order[i]]);
-        grp_n.push_back(n);
-        pair_grp_off[ent_pair[order[i]] + 1] += 1;
-        inorder_layout(n, heap_of_pos, stack);
-        for (uint32_t k = 0; k < n; ++k) {
-            const uint32_t e = order[i + k], h = heap_of_pos[k];
-            gf_key[i + h] = p->ins_offset[e];
-            gf_match[i + h] = ent_match[e];
-            ent_gf_grp[e] = g;
-            ent_gf_node[e] = h;
+    const bool on_host = !on_device || knob == LayoutSide::Check;
+    HostLayout H;
+    if (on_host) {
+        if (const int rc = host_layout(p, H)) return rc;
+        if (on_device) {  // check: the linear counts of the device path against the host layout's
+            const char* what = cnt.n_ins != H.c.n_ins ? "insertion count" : cnt.S_live != H.c.S_live ? "live step count"
+                             : cnt.n_inner != H.c.n_inner ? "inner slot count" : nullptr;
+            if (what) return fail(CLB_ECUDA, std::string("CLB_CHAIN_LAYOUT=check: the device layout's ") + what + " differs from the host layout's");
         }
-        i = j;
+        cnt = H.c;
     }
-    for (int64_t pr = 0; pr < npair; ++pr) pair_grp_off[pr + 1] += pair_grp_off[pr];
-
-    // orthogonal trees: one shape per pair, keys ((shift, match), offset)
-    std::vector<int64_t> pair_base(npair + 1, 0), in_base, ent_rank_off;
-    std::vector<int32_t> or_shift;
-    std::vector<uint32_t> or_off, or_match, in_n, in_off, ent_or_node, ent_rank;
-    int64_t n_inner = 0;
-    if (P > 0) {
-        or_shift.resize(E); or_off.resize(E); or_match.resize(E); in_n.assign(E, 0); in_base.assign(E, -1);
-        ent_or_node.resize(E); ent_rank_off.assign(E + 1, 0);
-        parallel_for(E, 1 << 16, [&](int64_t a, int64_t b) {  // (pair, shift, match)
-            for (int64_t e = a; e < b; ++e)
-                keys[e] = SortKey{((uint64_t)ent_pair[e] << 32) | ((uint32_t)p->ins_shift[e] ^ 0x80000000u), (uint64_t)ent_match[e], (uint32_t)e};
-        });
-        parallel_sort(keys);
-        for (int64_t i = 0; i < E; ++i) order[i] = keys[i].e;
-        for (int64_t e = 0; e < E; ++e) pair_base[ent_pair[e] + 1] += 1;
-        for (int64_t pr = 0; pr < npair; ++pr) pair_base[pr + 1] += pair_base[pr];
-        std::vector<uint32_t> pos_of_heap, sub_lo, sub_n, nanc;
-        std::vector<uint8_t> spine;
-        // pass 1: shapes, inner-list sizes and bases
-        for (int64_t pr = 0; pr < npair; ++pr) {
-            const int64_t ob = pair_base[pr];
-            const uint32_t n = (uint32_t)(pair_base[pr + 1] - ob);
-            if (!n) continue;
-            inorder_layout(n, heap_of_pos, stack);
-            for (uint32_t k = 0; k < n; ++k) {
-                const uint32_t e = order[ob + k], h = heap_of_pos[k];
-                or_shift[ob + h] = p->ins_shift[e];
-                or_off[ob + h] = p->ins_offset[e];
-                or_match[ob + h] = ent_match[e];
-                ent_or_node[e] = h;
-            }
-            spine.assign(n, 0);  // orthogonal_max_search_tree.hpp:175-182: the two outer spines carry no cross tree
-            for (uint64_t c = 0; c < n; c = 2 * c + 1) spine[c] = 1;
-            for (uint64_t c = 2; c < n; c = 2 * c + 2) spine[c] = 1;
-            sub_n.assign(n, 1);
-            for (uint32_t h = n; h-- > 1;) sub_n[(h - 1) / 2] += sub_n[h];
-            nanc.assign(n, 0);
-            for (uint32_t h = 0; h < n; ++h) {
-                nanc[h] = (h ? nanc[(h - 1) / 2] : 0) + (spine[h] ? 0 : 1);
-                if (!spine[h]) {
-                    in_base[ob + h] = n_inner;
-                    in_n[ob + h] = sub_n[h];
-                    n_inner += sub_n[h];
-                }
-            }
-            for (uint32_t k = 0; k < n; ++k) ent_rank_off[order[ob + k] + 1] = nanc[heap_of_pos[k]];
-        }
-        for (int64_t e = 0; e < E; ++e) ent_rank_off[e + 1] += ent_rank_off[e];
-        if (ent_rank_off[E] != n_inner) return fail(CLB_ECUDA, "internal: inner list accounting mismatch");
-        in_off.resize(n_inner);
-        ent_rank.resize(n_inner);
-        // pass 2: inner lists by merging children lists, one tree level at a time from the leaves up (the nodes of a
-        // level are independent); a list holds outer key-order positions and is stored where the device will read it
-        std::vector<uint32_t> in_pos(n_inner);
-        for (int64_t pr = 0; pr < npair; ++pr) {
-            const int64_t ob = pair_base[pr];
-            const uint32_t n = (uint32_t)(pair_base[pr + 1] - ob);
-            if (!n) continue;
-            inorder_layout(n, heap_of_pos, stack);
-            pos_of_heap.resize(n);
-            for (uint32_t k = 0; k < n; ++k) pos_of_heap[heap_of_pos[k]] = k;
-            auto depth_of = [](uint32_t h) { return 31 - __builtin_clz(h + 1); };  // heap index -> depth
-            for (int d = depth_of(n - 1); d >= 0; --d) {
-                const int64_t first = (int64_t(1) << d) - 1, last = std::min<int64_t>(n, (int64_t(2) << d) - 1);
-                parallel_for(last - first, std::max<int64_t>(1, 65536 / std::max<int64_t>(1, n >> d)), [&](int64_t a0, int64_t b0) {
-                    for (int64_t hh = first + a0; hh < first + b0; ++hh) {
-                        const uint32_t h = (uint32_t)hh;
-                        if (in_base[ob + h] < 0) continue;  // spine: never queried, never built
-                        const uint32_t l = 2 * h + 1, r = 2 * h + 2;
-                        uint32_t* out = in_pos.data() + in_base[ob + h];
-                        const uint32_t* L = l < n ? in_pos.data() + in_base[ob + l] : nullptr;
-                        const uint32_t* R = r < n ? in_pos.data() + in_base[ob + r] : nullptr;
-                        const uint32_t nl = l < n ? in_n[ob + l] : 0, nr = r < n ? in_n[ob + r] : 0;
-                        const uint32_t self = pos_of_heap[h];
-                        auto off_of = [&](uint32_t pos) { return or_off[ob + heap_of_pos[pos]]; };
-                        // positions of the left subtree < self < positions of the right subtree: ties in offset resolve by side
-                        const uint32_t so = off_of(self);
-                        uint32_t a = 0, b = 0, k = 0;
-                        bool self_done = false;
-                        while (a < nl || b < nr || !self_done) {
-                            // candidates in position order: L[a] < self < R[b]; pick the smallest (offset, position)
-                            int pick = -1;
-                            uint32_t bo = 0;
-                            if (a < nl) { pick = 0; bo = off_of(L[a]); }
-                            if (!self_done && (pick < 0 || so < bo)) { pick = 1; bo = so; }
-                            if (b < nr) {
-                                const uint32_t ro = off_of(R[b]);
-                                if (pick < 0 || ro < bo) pick = 2;
-                            }
-                            out[k++] = pick == 0 ? L[a++] : (pick == 1 ? self : R[b++]);
-                            if (pick == 1) self_done = true;
-                        }
-                        // offsets of the list entries and the rank of every element in this list
-                        const int64_t ib = in_base[ob + h];
-                        for (uint32_t kk = 0; kk < k; ++kk) {
-                            const uint32_t pos = out[kk], eh = heap_of_pos[pos];
-                            in_off[ib + kk] = or_off[ob + eh];
-                            ent_rank[ent_rank_off[order[ob + pos]] + (depth_of(eh) - d)] = kk;  // climbing order: the element's own node first
-                        }
-                    }
-                });
-            }
-        }
-    }
-    // insertion records in the reference's order, and the remaining per-entry tables in 32-bit form
-    if (n_inner >= (int64_t(1) << 32) - 1) return fail(CLB_EINVAL, "search structures exceed 2^32 inner slots");
-    if ((int64_t)sins_entry.size() >= (int64_t(1) << 31)) return fail(CLB_EINVAL, "more than 2^31 insertions");
-    std::vector<clb::InsRec> ins(sins_entry.size());
-    for (size_t i = 0; i < sins_entry.size(); ++i) {
-        const uint32_t e = sins_entry[i];
-        clb::InsRec& r = ins[i];
-        r.match = ent_match[e];
-        r.gf_base = (uint32_t)grp_base[ent_gf_grp[e]];
-        r.gf_node = ent_gf_node[e];
-        r.or_base = P > 0 ? (uint32_t)pair_base[ent_pair[e]] : 0;
-        r.or_node = P > 0 ? ent_or_node[e] : 0;
-        r.shift = p->ins_shift[e];
-        r.rank_off = P > 0 ? (uint32_t)ent_rank_off[e] : 0;
-        r.n_rank = P > 0 ? (uint32_t)(ent_rank_off[e + 1] - ent_rank_off[e]) : 0;
-    }
-    std::vector<uint32_t> grp_base32(grp_base.begin(), grp_base.end()), pair_base32(pair_base.begin(), pair_base.end());
-    std::vector<uint32_t> in_base32(in_base.size());
-    for (size_t k = 0; k < in_base.size(); ++k) in_base32[k] = in_base[k] < 0 ? clb::kChainNone : (uint32_t)in_base[k];
-    const double t_built = now_ms();
+    double t_built = now_ms();
     if (layout_only) {
         fprintf(stderr, "[clb] chain layout only: %lld matches, %lld entries, %lld inner slots, %.1f ms\n", (long long)M, (long long)E,
-                (long long)n_inner, t_built - t_start);
+                (long long)cnt.n_inner, t_built - t_start);
         return fail(CLB_ECUDA, "CLB_CHAIN_LAYOUT_ONLY: layout timed, nothing computed");
     }
+    const char* layout_name = on_device ? (on_host ? "check" : "device") : "host";
 
     // ------------------------------------------------------------------ device ------------------------------------------------------------------
     int rc = CLB_OK;
@@ -551,39 +764,41 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
     {
         ArenaPlan plan;
         ChainLayout L{};
-        std::vector<uint32_t> bp0(M, clb::kChainNone);
-        L.o_dp = plan.copy(p->dp_init, M * sizeof(float));
-        L.o_bp = plan.copy(bp0);
-        // the device walks only the steps in which something happens (a caller may list every node of graph 1 as a step; the
-        // builders of hostcpp/chain_b200.hpp list the nodes with events): the offsets are cumulative, so dropping an empty step
-        // drops one equal entry of either list
-        std::vector<int64_t> sins_live, qry_live;
-        sins_live.reserve(S + 1); qry_live.reserve(S + 1);
-        sins_live.push_back(sins_off[0]); qry_live.push_back(p->qry_off[0]);
-        for (int64_t s = 0; s < S; ++s)
-            if (sins_off[s + 1] != sins_off[s] || p->qry_off[s + 1] != p->qry_off[s]) {
-                sins_live.push_back(sins_off[s + 1]);
-                qry_live.push_back(p->qry_off[s + 1]);
+        const int64_t n_inner = cnt.n_inner, max_q = cnt.max_q;
+        int64_t h2d = 0;
+        double t_staged = 0;
+        clb::ChainLayoutDims dims{M, S, E, p->end_off[S], npair, C2, P, cnt.max_n ? clb::heap_depth(cnt.max_n - 1) : 0, p->ins_active != nullptr};
+        if (on_device) {  // phase 1: per-entry tables and sorts on the device; its read-back is the number of gap-free trees
+            CUDA_TRY_CLEANUP(cudaSetDevice(device));
+            CUDA_TRY_CLEANUP(ensure_stream(ar));
+            size_t scratch = 0;
+            CUDA_TRY_CLEANUP(clb::chain_layout_scratch_bytes(dims, &scratch));
+            if (ar.ls_cap < scratch) {
+                if (ar.ls) cudaFree(ar.ls);
+                ar.ls = nullptr;
+                ar.ls_cap = 0;
+                CUDA_TRY_CLEANUP(cudaMalloc((void**)&ar.ls, scratch));
+                ar.ls_cap = scratch;
             }
-        const int64_t S_live = (int64_t)sins_live.size() - 1;
-        L.o_sins = plan.copy(sins_live); L.o_ins = plan.copy(ins);
-        L.o_qoff = plan.copy(qry_live); L.o_qm = plan.copy(p->qry_match, n_qry * sizeof(uint32_t));
-        L.o_w = plan.copy(p->weight, M * sizeof(float)); L.o_qc1 = plan.copy(p->qry_chain1, n_qry * sizeof(uint32_t));
-        L.o_qa1 = plan.copy(p->qa1, (size_t)M * C1 * sizeof(int32_t)); L.o_qa2 = plan.copy(p->qa2, (size_t)M * C2 * sizeof(int32_t));
-        L.o_qo = plan.copy(p->qoff, (size_t)M * C2 * sizeof(uint32_t));
-        L.o_pg = plan.copy(pair_grp_off); L.o_gs = plan.copy(grp_shift); L.o_gb = plan.copy(grp_base32); L.o_gn = plan.copy(grp_n);
-        L.o_pb = plan.copy(pair_base32); L.o_gk = plan.copy(gf_key); L.o_gm = plan.copy(gf_match);
-        L.o_os = plan.copy(or_shift); L.o_oo = plan.copy(or_off); L.o_om = plan.copy(or_match);
-        L.o_ib = plan.copy(in_base32); L.o_in = plan.copy(in_n); L.o_io = plan.copy(in_off); L.o_er = plan.copy(ent_rank);
-        L.z_qrec = plan.zero((size_t)n_qry * C2 * sizeof(clb::QueryRec));
-        L.z_gford = plan.zero((size_t)E * 4); L.z_gfbest = plan.zero((size_t)E * 8);
-        L.z_orord = plan.zero((size_t)T * E * 4); L.z_bit = plan.zero((size_t)T * n_inner * 8);
-        L.z_cbest = plan.zero((size_t)M * 16); L.z_cbp = plan.zero((size_t)(max_q * C2 * (T + 1)) * 4 * 2); L.z_cnt = plan.zero(8);
+            const clb::ChainLayoutIn in{p->ins_off, p->ins_p1, p->ins_p2, p->ins_shift, p->ins_offset, p->ins_active, p->end_off, p->end_match, p->qry_off};
+            int64_t G = 0;
+            CUDA_TRY_CLEANUP(clb::chain_layout_sort(in, dims, ar.ls, ar.stream, &G, &h2d));
+            if (on_host && G != cnt.G) {
+                rc = fail(CLB_ECUDA, "CLB_CHAIN_LAYOUT=check: the device layout's gap-free tree count differs from the host layout's");
+                goto cleanup;
+            }
+            cnt.G = G;
+        }
+        {
+            const void* raw[kSegs] = {};  // the device layout copies only the caller's arrays
+            raw[kSegDp] = p->dp_init; raw[kSegQm] = p->qry_match; raw[kSegW] = p->weight; raw[kSegQc1] = p->qry_chain1;
+            raw[kSegQa1] = p->qa1; raw[kSegQa2] = p->qa2; raw[kSegQo] = p->qoff;
+            plan_layout(cnt, on_device ? raw : H.src, L, plan);
+        }
         // subtree-block ranks of every orthogonal walk (2 * (depth + 1) blocks at most), if memory allows
         int rank_stride = 0;
         if (P > 0 && n_qry > 0 && !getenv("CLB_CHAIN_NO_RANKS")) {
-            uint32_t max_n = 1;
-            for (int64_t pr = 0; pr < npair; ++pr) max_n = std::max<uint32_t>(max_n, (uint32_t)(pair_base[pr + 1] - pair_base[pr]));
+            const uint32_t max_n = std::max<uint32_t>(1, cnt.max_n);
             rank_stride = 2 * (32 - __builtin_clz(max_n));
             const size_t bytes = (size_t)n_qry * C2 * 2 * rank_stride * 4;
             bool fits = bytes <= (size_t(64) << 20);  // small pools always fit; cudaMemGetInfo costs more than a small problem
@@ -604,11 +819,11 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
             b.gap_extend[k] = p->gap_extend[k];
             b.scale_ext[k] = p->scale * p->gap_extend[k];  // anchorer.hpp:2330: local_scale * gap_extend[pw / 2] (* shift on the device)
         }
-        b.n_match = M; b.n_step = S_live; b.n_entry = E; b.n_inner = n_inner; b.n_qry = n_qry; b.n_ins = (int64_t)ins.size();
+        b.n_match = M; b.n_step = cnt.S_live; b.n_entry = E; b.n_inner = n_inner; b.n_qry = n_qry; b.n_ins = cnt.n_ins;
         b.cand_bp_stride = max_q * C2 * (T + 1);
         b.rank_stride = rank_stride;
         const size_t total = plan.copy_bytes + plan.zero_bytes;
-        if (ctx && total <= kChainBatchArena && !getenv("CLB_CHAIN_NO_SMALL")) {
+        if (!on_device && ctx && total <= kChainBatchArena && !getenv("CLB_CHAIN_NO_SMALL")) {
             // batched small problem: stage the copy region and keep the layout; flush() binds it to the staged arena
             DeferredProblem d;
             d.arena_off = ctx->staging.size();
@@ -625,7 +840,7 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
             if (stats) {
                 stats->build_ms = t_built - t_start;
                 stats->steps = S;
-                stats->inserts = (int64_t)ins.size();
+                stats->inserts = cnt.n_ins;
                 stats->queries = n_qry * C2;
                 stats->tree_bytes = (int64_t)total;
                 stats->h2d_bytes = (int64_t)plan.copy_bytes;
@@ -635,12 +850,7 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
         }
         keep = total <= kArenaKeep;
         CUDA_TRY_CLEANUP(cudaSetDevice(device));
-        if (!ar.stream) {
-            CUDA_TRY_CLEANUP(cudaStreamCreateWithFlags(&ar.stream, cudaStreamNonBlocking));
-            CUDA_TRY_CLEANUP(cudaEventCreate(&ar.ev0));
-            CUDA_TRY_CLEANUP(cudaEventCreate(&ar.ev1));
-            CUDA_TRY_CLEANUP(cudaEventCreate(&ar.evp));
-        }
+        CUDA_TRY_CLEANUP(ensure_stream(ar));
         if (ar.cap < total) {
             if (ar.d) cudaFree(ar.d);
             ar.d = nullptr;
@@ -649,36 +859,78 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
             CUDA_TRY_CLEANUP(cudaMalloc((void**)&ar.d, want));
             ar.cap = want;
         }
-        // A large problem is copied segment by segment straight from the caller's arrays: pinning a staging twin of tens to
-        // hundreds of MB costs more (≈ 1 ms per MB) than the driver's own staging of a pageable copy, and a problem of that size
-        // comes a few times per alignment.  Small problems -- thousands per alignment -- share one pinned twin that stays.
-        const bool direct = plan.copy_bytes > kDirectCopyBytes && ar.hcap < plan.copy_bytes;
-        if (!direct && ar.hcap < plan.copy_bytes) {
-            if (ar.h) cudaFreeHost(ar.h);
-            ar.h = nullptr;
-            ar.hcap = 0;
-            const size_t want = std::max(plan.copy_bytes, std::min(kDirectCopyBytes, 2 * plan.copy_bytes));
-            CUDA_TRY_CLEANUP(cudaHostAlloc((void**)&ar.h, want, cudaHostAllocDefault));
-            ar.hcap = want;
-        }
-        if (!direct)
-            for (const auto& sg : plan.segs)
-                if (sg.bytes) memcpy(ar.h + sg.off, sg.src, sg.bytes);
-        const double t_staged = now_ms();
-        if (direct) {
-            for (const auto& sg : plan.segs)
-                if (sg.bytes) CUDA_TRY_CLEANUP(cudaMemcpyAsync(ar.d + sg.off, sg.src, sg.bytes, cudaMemcpyHostToDevice, ar.stream));
-        } else {
-            CUDA_TRY_CLEANUP(cudaMemcpyAsync(ar.d, ar.h, plan.copy_bytes, cudaMemcpyHostToDevice, ar.stream));
-        }
         char* zr = ar.d + plan.copy_bytes;
+        if (on_device) {
+            // phase 2: the caller's raw arrays go up as they are, every other table is written by the layout kernels
+            for (int k = 0; k < kSegs; ++k)
+                if (seg_is_raw(k) && plan.segs[k].bytes) {
+                    CUDA_TRY_CLEANUP(cudaMemcpyAsync(ar.d + plan.segs[k].off, plan.segs[k].src, plan.segs[k].bytes, cudaMemcpyHostToDevice, ar.stream));
+                    h2d += (int64_t)plan.segs[k].bytes;
+                }
+            CUDA_TRY_CLEANUP(cudaMemsetAsync(ar.d + L.o[kSegBp], 0xff, (size_t)M * 4, ar.stream));  // bp0: kChainNone
+            char* c = ar.d;
+            const clb::ChainLayoutOut out{(int64_t*)(c + L.o[kSegSins]), (clb::InsRec*)(c + L.o[kSegIns]), (int64_t*)(c + L.o[kSegQoff]),
+                                          (int64_t*)(c + L.o[kSegPg]), (int32_t*)(c + L.o[kSegGs]), (uint32_t*)(c + L.o[kSegGb]),
+                                          (uint32_t*)(c + L.o[kSegGn]), (uint32_t*)(c + L.o[kSegPb]), (uint32_t*)(c + L.o[kSegGk]),
+                                          (uint32_t*)(c + L.o[kSegGm]), (int32_t*)(c + L.o[kSegOs]), (uint32_t*)(c + L.o[kSegOo]),
+                                          (uint32_t*)(c + L.o[kSegOm]), (uint32_t*)(c + L.o[kSegIb]), (uint32_t*)(c + L.o[kSegIn]),
+                                          (uint32_t*)(c + L.o[kSegIo]), (uint32_t*)(c + L.o[kSegEr])};
+            int64_t dev_inner = 0;
+            CUDA_TRY_CLEANUP(clb::chain_layout_build(dims, cnt.G, ar.ls, out, ar.stream, &dev_inner));
+            if (P > 0 && E > 0 && dev_inner != n_inner) {
+                rc = fail(CLB_ECUDA, "internal: inner list accounting mismatch");
+                goto cleanup;
+            }
+            if (on_host) {  // check: the copy region byte for byte against the host layout's
+                std::vector<char> got;
+                for (int k = 0; k < kSegs && rc == CLB_OK; ++k) {
+                    const size_t bytes = plan.segs[k].bytes;
+                    if (!bytes) continue;
+                    got.resize(bytes);
+                    CUDA_TRY_CLEANUP(cudaMemcpy(got.data(), ar.d + plan.segs[k].off, bytes, cudaMemcpyDeviceToHost));
+                    const char* want = (const char*)H.src[k];
+                    if (memcmp(got.data(), want, bytes) == 0) continue;
+                    size_t i = 0;
+                    while (got[i] == want[i]) ++i;
+                    rc = fail(CLB_ECUDA, std::string("CLB_CHAIN_LAYOUT=check: the device layout differs from the host layout in ") + kSegName[k] + "[" +
+                                             std::to_string(i / kSegElem[k]) + "]");
+                }
+                if (rc != CLB_OK) goto cleanup;
+            }
+            t_built = t_staged = now_ms();
+        } else {
+            // A large problem is copied segment by segment straight from the caller's arrays: pinning a staging twin of tens to
+            // hundreds of MB costs more (≈ 1 ms per MB) than the driver's own staging of a pageable copy, and a problem of that size
+            // comes a few times per alignment.  Small problems -- thousands per alignment -- share one pinned twin that stays.
+            const bool direct = plan.copy_bytes > kDirectCopyBytes && ar.hcap < plan.copy_bytes;
+            if (!direct && ar.hcap < plan.copy_bytes) {
+                if (ar.h) cudaFreeHost(ar.h);
+                ar.h = nullptr;
+                ar.hcap = 0;
+                const size_t want = std::max(plan.copy_bytes, std::min(kDirectCopyBytes, 2 * plan.copy_bytes));
+                CUDA_TRY_CLEANUP(cudaHostAlloc((void**)&ar.h, want, cudaHostAllocDefault));
+                ar.hcap = want;
+            }
+            if (!direct)
+                for (const auto& sg : plan.segs)
+                    if (sg.bytes) memcpy(ar.h + sg.off, sg.src, sg.bytes);
+            t_staged = now_ms();
+            if (direct) {
+                for (const auto& sg : plan.segs)
+                    if (sg.bytes) CUDA_TRY_CLEANUP(cudaMemcpyAsync(ar.d + sg.off, sg.src, sg.bytes, cudaMemcpyHostToDevice, ar.stream));
+            } else {
+                CUDA_TRY_CLEANUP(cudaMemcpyAsync(ar.d, ar.h, plan.copy_bytes, cudaMemcpyHostToDevice, ar.stream));
+            }
+            h2d = (int64_t)plan.copy_bytes;
+        }
         CUDA_TRY_CLEANUP(cudaMemsetAsync(zr, 0, plan.zero_bytes, ar.stream));
         a = bind(L, ar.d, zr);
         a.copy_bytes = (int64_t)total;  // the single-problem path copies the zeroed region too
         // How the phases of a step are separated.  A step has `warps_per_step` independent warp-sized work items on average:
         // a handful run in one CTA (__syncthreads), up to as many as the largest cluster has warps in ONE thread-block cluster
         // (hardware cluster barrier, the items of a step spread over its SMs), more in a cooperative grid over all SMs (grid.sync).
-        const double warps_per_step = S_live ? ((double)ins.size() + (double)n_qry * C2) * (T + 1) / (double)S_live : 0.0;
+        const int64_t S_live = cnt.S_live;
+        const double warps_per_step = S_live ? ((double)cnt.n_ins + (double)n_qry * C2) * (T + 1) / (double)S_live : 0.0;
         const int max_grid = clb::chain_max_grid(device);
         const int warps_per_cta = P == 0 ? 28 : 16;  // chain_kernels.cu: the gap-free kernel runs with 896 threads
         int cluster = 1;
@@ -709,19 +961,20 @@ static int chain_dp_impl(int device, const clb_chain_problem* p, float* dp_out, 
         if (getenv("CLB_TIMING")) {
             float pms = 0.f;
             cudaEventElapsedTime(&pms, ar.ev0, ar.evp);
-            fprintf(stderr, "[clb] chain: build %.1f ms, alloc+stage %.1f ms (%.0f MB arena, %.0f MB copied), prepare kernel %.2f ms, DP kernel %.2f ms, "
-                            "enqueue..sync %.1f ms (grid %d, cluster %d, %lld of %lld steps with events, %.0f warp items per step, rank pool %s)\n",
-                    t_built - t_start, t_staged - t_built, total / 1e6, plan.copy_bytes / 1e6, pms, ms - pms, now_ms() - t_staged, grid, cluster,
+            fprintf(stderr, "[clb] chain: build %.1f ms (%s layout), alloc+stage %.1f ms (%.0f MB arena, %.0f MB copied), prepare kernel %.2f ms, "
+                            "DP kernel %.2f ms, enqueue..sync %.1f ms (grid %d, cluster %d, %lld of %lld steps with events, %.0f warp items per step, "
+                            "rank pool %s)\n",
+                    t_built - t_start, layout_name, t_staged - t_built, total / 1e6, h2d / 1e6, pms, ms - pms, now_ms() - t_staged, grid, cluster,
                     (long long)S_live, (long long)S, warps_per_step, rank_stride ? "on" : "off");
         }
         if (stats) {
             stats->build_ms = t_built - t_start;
             stats->kernel_ms = ms;
             stats->steps = S;
-            stats->inserts = (int64_t)ins.size();
+            stats->inserts = cnt.n_ins;
             stats->queries = n_qry * C2;
             stats->tree_bytes = (int64_t)total;
-            stats->h2d_bytes = (int64_t)plan.copy_bytes;
+            stats->h2d_bytes = h2d;
             stats->d2h_bytes = M * 8;
             stats->kernel_launches = (grid == 0 || n_qry == 0) ? 1 : 2;
         }
@@ -735,6 +988,11 @@ cleanup:
         if (ar.h) cudaFreeHost(ar.h);
         ar.d = ar.h = nullptr;
         ar.cap = ar.hcap = 0;
+    }
+    if ((!keep || rc != CLB_OK || ar.ls_cap > kArenaKeep) && ar.ls) {  // the layout scratch: the same rule, and never kept above kArenaKeep
+        cudaFree(ar.ls);
+        ar.ls = nullptr;
+        ar.ls_cap = 0;
     }
     return rc;
 }
@@ -1020,6 +1278,7 @@ void chain_release_cache() {
         cudaSetDevice(device);
         if (a.d) cudaFree(a.d);
         if (a.h) cudaFreeHost(a.h);
+        if (a.ls) cudaFree(a.ls);
         if (a.ev0) cudaEventDestroy(a.ev0);
         if (a.ev1) cudaEventDestroy(a.ev1);
         if (a.evp) cudaEventDestroy(a.evp);
